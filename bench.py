@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --gpus N --steps K ...  # the reference's CPU algorithm (oracle port) on host cores
+    python bench.py ... --dump-outputs DIR                   # + state after the last timed step, seeded sample of targets, DIR/*.npy
 
 One "step" = one tick of the hot path over every target of the pool: TargetManager::update(id, dt, meas) for
 each target (predict + update + t / n_meas bookkeeping; a Philox-free 5 % of the targets miss their measurement
@@ -67,6 +68,9 @@ def parse():
     ap.add_argument("--no-c5", action="store_true", help="skip BASELINE configs[4] (mixed models sharded by id, all-gather at N>1)")
     ap.add_argument("--c5-targets", type=int, default=8 << 20, help="C5 targets per GPU (64 Mi over 8 GPUs)")
     ap.add_argument("--cpu-seconds", type=float, default=12.0)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the state of a fixed, seeded sample of the benchmarked targets as DIR/<name>.npy "
+                         "(with --gpus N > 1: a sample of rank 0's shard)")
     return ap.parse_args()
 
 
@@ -314,6 +318,29 @@ def make_inputs(torch, p0, n_sets, stride, miss_prob, seed):
     return meas, act
 
 
+DUMP_BYTES = 48 << 20   # float64 payload of --dump-outputs whatever the model: small enough to keep beside a result and compare
+
+
+DUMP_FIELDS = ("x", "P", "t", "n_meas")
+
+
+def dump_ids(n, world, rank, N):
+    """ids of the targets --dump-outputs writes: a fixed, seeded sample of this process's n targets (owner(id) = id mod world),
+    ascending.  It depends on the model, the target count and the number of GPUs only, so two builds run with the same arguments
+    are compared target for target.  With --gpus N > 1 only rank 0 writes, so the sample comes from rank 0's shard."""
+    k = min(n, DUMP_BYTES // ((N + N * N + 3) * 8))
+    sample = np.sort(np.random.default_rng(20261020).choice(n, k, replace=False))
+    return (sample.astype(np.int64) * world + rank).astype(np.uint32)
+
+
+def write_outputs(out_dir, ids, state):
+    """What a caller of the timed path reads back after its last step (te_pool_read_state: x, P, t, n_meas) for the targets
+    `ids`, as float64 DIR/<name>.npy files."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in [("ids", ids)] + [(f, state[f]) for f in DUMP_FIELDS]:
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a, dtype=np.float64))
+
+
 def main():
     args = parse()
     rank = int(os.environ.get("RANK", "0"))
@@ -346,6 +373,7 @@ def main():
     n_upd = [int((a == 2).sum().item()) for a in act]
     B_upd = te.bytes_per_step(mtype)
     B_pred = B_upd - 8 * (7 if M == 6 else 3) - 16          # no measurement read, n_meas untouched
+    d_ids = dump_ids(n, world, rank, N) if args.dump_outputs and rank == 0 else None
     torch.cuda.synchronize()
 
     def barrier():
@@ -377,7 +405,10 @@ def main():
     ev1.record(stream)
     barrier()
     burst_note = None
+    dumped = None
     if not sampler.sm:
+        if d_ids is not None:
+            dumped = pool.read_state(d_ids, want=DUMP_FIELDS)   # the burst below moves the state on
         # the timed region was shorter than NVML start-up + one 20 ms sample: keep sampling under an untimed burst of the same ticks
         t_end = time.perf_counter() + 0.5
         while time.perf_counter() < t_end:
@@ -388,6 +419,8 @@ def main():
     clocks = sampler.result()
     if burst_note:
         clocks["note"] = burst_note
+    if d_ids is not None:   # written after the clock sampling; the burst decision above is taken before any read
+        write_outputs(args.dump_outputs, d_ids, dumped if dumped is not None else pool.read_state(d_ids, want=DUMP_FIELDS))
     ms = ev0.elapsed_time(ev1)
     t_ms = torch.tensor([ms], dtype=torch.float64, device="cuda")
     if world > 1:

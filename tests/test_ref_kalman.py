@@ -32,7 +32,8 @@ def _golden():
 def _lib():
     subprocess.check_call(["make", "-C", os.path.join(ROOT, "oracle"), "-s"])
     if not os.path.exists(LIB):
-        pytest.skip("oracle/_ref/libref_kalman.so not built (no /root/reference here)")
+        pytest.skip("needs oracle/_ref/libref_kalman.so, which `make -C oracle REF=<checkout of the original target_estimation project>` "
+                    "builds from the original's own sources; they are not part of this repository, and this comparison has no stored form")
     L = C.CDLL(LIB)
     p, i = C.c_void_p, C.c_int
     L.ref_lkf_new.restype = p; L.ref_lkf_new.argtypes = [p, p, p, p, p, i, i]

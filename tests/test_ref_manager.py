@@ -21,7 +21,8 @@ DT = 1.0 / 250.0
 def _lib():
     subprocess.check_call(["make", "-C", os.path.join(ROOT, "oracle"), "-s"])
     if not os.path.exists(LIB):
-        pytest.skip("oracle/_ref/libref_manager.so not built (no /root/reference here)")
+        pytest.skip("needs oracle/_ref/libref_manager.so, which `make -C oracle REF=<checkout of the original target_estimation project>` "
+                    "builds from the original's own sources; they are not part of this repository, and this comparison has no stored form")
     orc.lib()   # libte_oracle.so first: the stand-in polynomial solver resolves orc_poly_roots from it
     L = C.CDLL(LIB, mode=C.RTLD_GLOBAL)
     p, i, d, u, ll = C.c_void_p, C.c_int, C.c_double, C.c_uint, C.c_longlong

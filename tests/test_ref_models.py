@@ -24,7 +24,8 @@ DT = 1.0 / 250.0
 def _lib():
     subprocess.check_call(["make", "-C", os.path.join(ROOT, "oracle"), "-s"])
     if not os.path.exists(LIB):
-        pytest.skip("oracle/_ref/libref_models.so not built (no /root/reference here)")
+        pytest.skip("needs oracle/_ref/libref_models.so, which `make -C oracle REF=<checkout of the original target_estimation project>` "
+                    "builds from the original's own sources; they are not part of this repository, and this comparison has no stored form")
     L = C.CDLL(LIB)
     p, i, d, u = C.c_void_p, C.c_int, C.c_double, C.c_uint
     L.ref_target_new.restype = p; L.ref_target_new.argtypes = [i, u, d, d, p, i, p, i, p, p, p, p]

@@ -22,7 +22,8 @@ DT = 1.0 / 250.0
 def _lib():
     subprocess.check_call(["make", "-C", os.path.join(ROOT, "oracle"), "-s"])
     if not os.path.exists(LIB):
-        pytest.skip("oracle/_ref/libref_manager.so not built (no /root/reference here)")
+        pytest.skip("needs oracle/_ref/libref_manager.so, which `make -C oracle REF=<checkout of the original target_estimation project>` "
+                    "builds from the original's own sources; they are not part of this repository, and this comparison has no stored form")
     orc.lib()
     L = C.CDLL(LIB, mode=C.RTLD_GLOBAL)
     if not hasattr(L, "refr_new"):
