@@ -14,7 +14,7 @@
 
 namespace target_estimation_b200 {
 
-class TickTargetManager;
+class TickFrontEnd;
 
 struct TfRecord {
   uint32_t rec_sec = 0, rec_nsec = 0;   // receive time of the message record (what `rosbag play --clock` publishes as now)
@@ -34,6 +34,6 @@ struct ReplayStats {
 // target_node's loop on the recording: tick k runs at now_k = (first record time) + k / frequency (integer nanoseconds);
 // after each tick the messages received up to now_k are delivered, one measurementCallBack per message.  Ends
 // `extra_ticks` ticks after the last message was delivered.
-ReplayStats replayBag(TickTargetManager& mgr, const std::vector<TfRecord>& records, double frequency, long long extra_ticks = 0);
+ReplayStats replayBag(TickFrontEnd& mgr, const std::vector<TfRecord>& records, double frequency, long long extra_ticks = 0);
 
 }  // namespace target_estimation_b200

@@ -296,27 +296,60 @@ class Measurement {   // target_manager_ros.hpp:74-134
   bool stamp_dirty_ = false;
 };
 
-class TickTargetManager : public TargetManager {
+// The node loop of RosTargetManager (target_manager_ros.hpp:136-183): what replayBag and the C-ABI's target_tick_manager_* calls
+// drive, on one device (TickTargetManager) or on every GPU of the box (ShardedTickTargetManager).
+class TickFrontEnd {
+ public:
+  virtual ~TickFrontEnd() {}
+  // /tf callback (src/target_manager_ros.cpp:26-39): frame "<token>_<id>"; a frame that contains the token but does
+  // not parse BREAKS the loop (the rest of the message is dropped), like the reference
+  virtual void measurementCallBack(long long n, const char* const* child_frame_ids, const uint32_t* sec, const uint32_t* nsec,
+                                   const double* poses) = 0;
+  virtual void measurementCallBackIds(long long n, const unsigned* ids, const uint32_t* sec, const uint32_t* nsec, const double* poses) = 0;
+  // RosTargetManager::update(dt) (:41-92) with ros::Time::now() = (now_sec, now_nsec).  erased (optional) receives
+  // the ids removed by the expiry rule in ascending order.
+  virtual void tick(const double& dt, uint32_t now_sec, uint32_t now_nsec, std::vector<unsigned>* erased = nullptr) = 0;
+  // the poses the node would broadcast after the last tick: ids + [n][7]
+  virtual const std::vector<unsigned>& publishedIds() const = 0;
+  virtual const std::vector<double>& publishedPoses() const = 0;
+  virtual void setTargetTokenName(const std::string& token_name) = 0;
+  virtual void setExpirationTime(double t) = 0;
+  virtual double time() const = 0;
+  virtual size_t mailboxCount() = 0;   // measurements_.size() of the reference
+  bool publish = true;   // gather the filtered poses every tick (the TF broadcast of :78-87)
+ protected:
+  // the frames of one message -> (id, stamp, pose) records, the reference's loop (:26-39): frames without the token are skipped,
+  // the first frame that carries it but does not parse ends the message
+  static void parseFrames(const std::string& token, long long n, const char* const* frames, const uint32_t* sec, const uint32_t* nsec,
+                          const double* poses, std::vector<unsigned>& ids, std::vector<uint32_t>& s, std::vector<uint32_t>& ns,
+                          std::vector<double>& p);
+};
+
+class TickTargetManager : public TargetManager, public TickFrontEnd {
  public:
   TickTargetManager(target_t type, const MatrixXd& Q, const MatrixXd& R, const MatrixXd& P, int device = 0);
   explicit TickTargetManager(const std::string& yaml_file, int device = 0);
   ~TickTargetManager() override;
-  // /tf callback (src/target_manager_ros.cpp:26-39): frame "<token>_<id>"; a frame that contains the token but does
-  // not parse BREAKS the loop (the rest of the message is dropped), like the reference
-  void measurementCallBack(long long n, const char* const* child_frame_ids, const uint32_t* sec, const uint32_t* nsec, const double* poses);
-  void measurementCallBackIds(long long n, const unsigned* ids, const uint32_t* sec, const uint32_t* nsec, const double* poses);
-  // RosTargetManager::update(dt) (:41-92) with ros::Time::now() = (now_sec, now_nsec).  erased (optional) receives
-  // the ids removed by the expiry rule in ascending order.
-  void tick(const double& dt, uint32_t now_sec, uint32_t now_nsec, std::vector<unsigned>* erased = nullptr);
-  // the poses the node would broadcast after the last tick: ascending ids + [n][7]
-  const std::vector<unsigned>& publishedIds() const { return pub_ids_; }
-  const std::vector<double>& publishedPoses() const { return pub_poses_; }
-  void setTargetTokenName(const std::string& token_name) { token_name_ = token_name; }
-  void setExpirationTime(double t);
-  double time() const { return t_; }
-  size_t mailboxCount();   // measurements_.size() of the reference: device mailboxes + target-less ones + host ones
-  bool publish = true;   // gather the filtered poses every tick (the TF broadcast of :78-87)
+  void measurementCallBack(long long n, const char* const* child_frame_ids, const uint32_t* sec, const uint32_t* nsec,
+                           const double* poses) override;
+  void measurementCallBackIds(long long n, const unsigned* ids, const uint32_t* sec, const uint32_t* nsec, const double* poses) override;
+  void tick(const double& dt, uint32_t now_sec, uint32_t now_nsec, std::vector<unsigned>* erased = nullptr) override;
+  // ascending ids + [n][7]
+  const std::vector<unsigned>& publishedIds() const override { return pub_ids_; }
+  const std::vector<double>& publishedPoses() const override { return pub_poses_; }
+  void setTargetTokenName(const std::string& token_name) override { token_name_ = token_name; }
+  void setExpirationTime(double t) override;
+  double time() const override { return t_; }
+  size_t mailboxCount() override;   // device mailboxes + target-less ones + host ones
  private:
+  friend class ShardedTickTargetManager;
+  // the pieces of the sharded node loop, each under the manager's lock
+  te_pool* devicePool();   // flushes the queued by-hand calls; the tick's pool, or NULL while some id needs a host mailbox
+  void ingestDev(long long n, const uint32_t* dev_ids, const uint32_t* dev_sec, const uint32_t* dev_nsec, const double* dev_poses);
+  void advance(const double& dt, uint32_t now_sec, uint32_t now_nsec, std::vector<unsigned>* erased);   // tick() without the broadcast
+  long long publishCount();                                  // poses the broadcast covers (every target)
+  void publishInto(unsigned* ids, double* poses, long long n);   // their ascending ids and [n][7] poses
+  bool foreignPossible(te_pool* pool);
   te_pool* tickPool();
   void tickForeign(const double& dt, uint32_t now_sec, uint32_t now_nsec, std::vector<unsigned>& gone_out);
   int cls_ = -1;   // model class of (Q_, R_, P_) in the pool of type_
@@ -343,12 +376,30 @@ class TickTargetManager : public TargetManager {
 // The optional exchange of estimates (SURVEY.md 8(e)) is gatherEstimates(): [pose7 | twist6] records of every target, all shards,
 // gathered on every device over NCCL (te_group_*), then read back from the publishing shard's device.
 // ---------------------------------------------------------------------------------------------------
+// id mod G without a division per record (the routing passes look at every id of a batch; a hardware divide per id cost more than
+// the tick it feeds): a mask for powers of two, else Lemire's multiply-shift remainder, exact for 32-bit operands
+struct FastMod {
+  explicit FastMod(unsigned d) : d_(d), pow2_((d & (d - 1)) == 0), m_(~(unsigned long long)0 / d + 1) {}
+  unsigned operator()(unsigned a) const {
+    if (pow2_) return a & (d_ - 1);
+    const unsigned long long low = m_ * a;
+    return (unsigned)(((unsigned __int128)low * d_) >> 64);
+  }
+  unsigned d_;
+  bool pow2_;
+  unsigned long long m_;
+};
+
 class ShardWorkers;
 class ShardedTargetManager : public TargetManager {
  public:
   // devices NULL = devices 0 .. n_shards-1; a device may repeat (several shards on one GPU: a one-GPU box still runs the
   // sharded host logic -- the estimate exchange then uses device copies, NCCL needs distinct devices)
   ShardedTargetManager(const std::string& file, int n_shards, const int* devices = nullptr);
+ protected:
+  // the same with shards made by make_shard(device) (a derived manager's shards are derived managers)
+  ShardedTargetManager(const std::string& file, int n_shards, const int* devices, const std::function<TargetManager*(int)>& make_shard);
+ public:
   ~ShardedTargetManager() override;
   int shards() const { return (int)shard_.size(); }
   int owner(unsigned id) const { return (int)(id % (unsigned)shard_.size()); }
@@ -393,8 +444,14 @@ class ShardedTargetManager : public TargetManager {
   double lastGatherMs() const { return gather_ms_; }
   bool gatherUsesNccl();
 
- private:
-  template <class F> void forEachShard(F&& f);   // f(r) on shard r's worker thread, all shards at once; rethrows the first error
+ protected:
+  void forEachShard(const std::function<void(int)>& f);   // f(r) on shard r's worker thread, all shards at once; rethrows the first error
+  // The routing of a batch on the host (a parallel stable partition by owner, see updateBatch): reserve(r, m) sizes shard r's
+  // staging for its m records (on r's worker thread); scatter(t, lo, hi, at) runs on router thread t for the records [lo, hi) of
+  // the batch and puts record k of owner r at place at[r]++ of r's staging.  Returns the records of every shard.
+  std::vector<size_t> routeOnHost(long long n, const unsigned* ids, const std::function<void(int, size_t)>& reserve,
+                                  const std::function<void(int, long long, long long, size_t*)>& scatter);
+  te_group* group();   // created on first use
   std::vector<std::unique_ptr<TargetManager>> shard_;
   std::vector<int> devices_;
   std::unique_ptr<ShardWorkers> workers_;   // one thread per shard: the shards' batched calls
@@ -409,6 +466,50 @@ class ShardedTargetManager : public TargetManager {
     size_t cap = 0;
   };
   std::vector<Stage> stage_;
+};
+
+// ---------------------------------------------------------------------------------------------------
+// The node loop over every GPU of the box: one TickTargetManager per shard (owner(id) = id mod G, shard r on devices[r]).  A /tf
+// message is parsed on the host as a whole, then routed ON THE DEVICES (te_group_route_records: G chunk uploads in parallel, a
+// stable partition by owner on every device, NCCL send / receive between them) and every shard's worker ingests its run in place
+// (te_pool_mailbox_ingest_dev): host work per message is O(G) copies, not a pass over the records.  Arrival order per id is kept, so
+// Measurement::update sees the records of an id in the order the single-device loop sees them.  While some shard keeps host
+// mailboxes (an id lives there under another model type, created by hand) the message takes the host route instead: the router
+// threads of the batched calls, then that shard's measurementCallBackIds.  TE_SHARD_HOST_ROUTE in the environment of the process
+// (read when the manager is made) forces the host route -- a debugging switch.
+// A tick runs every shard's tick on its worker thread at once; the erased ids of all shards come back as one ascending list, and
+// the broadcast is shard-major (shard 0's targets in ascending id, then shard 1's, ...: denseIds() order), every shard writing its
+// slice straight into one page-locked output.  By-hand calls, batched calls and gatherEstimates work as in ShardedTargetManager.
+// ---------------------------------------------------------------------------------------------------
+class ShardedTickTargetManager : public ShardedTargetManager, public TickFrontEnd {
+ public:
+  ShardedTickTargetManager(const std::string& yaml_file, int n_shards, const int* devices = nullptr);
+  ~ShardedTickTargetManager() override;
+  TickTargetManager& tickShard(int r) { return static_cast<TickTargetManager&>(*shard_[(size_t)r]); }
+  void measurementCallBack(long long n, const char* const* child_frame_ids, const uint32_t* sec, const uint32_t* nsec,
+                           const double* poses) override;
+  void measurementCallBackIds(long long n, const unsigned* ids, const uint32_t* sec, const uint32_t* nsec, const double* poses) override;
+  void tick(const double& dt, uint32_t now_sec, uint32_t now_nsec, std::vector<unsigned>* erased = nullptr) override;
+  // shard-major ids + [n][7]
+  const std::vector<unsigned>& publishedIds() const override { return pub_ids_; }
+  const std::vector<double>& publishedPoses() const override { return pub_poses_; }
+  void setTargetTokenName(const std::string& token_name) override { token_name_ = token_name; }
+  void setExpirationTime(double t) override;
+  double time() const override;
+  size_t mailboxCount() override;   // sum over the shards
+
+ private:
+  std::string token_name_ = "target";
+  bool force_host_route_ = false;
+  std::vector<unsigned> pub_ids_;
+  std::vector<double> pub_poses_;
+  void* pub_pinned_[2] = {nullptr, nullptr};   // storage of pub_ids_ / pub_poses_ while it is page-locked
+  struct HostStage {   // per shard: its records of a message on the host route
+    std::vector<unsigned> ids;
+    std::vector<uint32_t> sec, nsec;
+    std::vector<double> poses;
+  };
+  std::vector<HostStage> host_stage_;
 };
 
 // utils.hpp:273-313

@@ -96,6 +96,13 @@ int target_manager_gather_uses_nccl(const target_manager_c* self);
 /* ---- tick front-end: RosTargetManager semantics without ROS (src/target_manager_ros.cpp:26-92) ----
  * The handle is also a valid target_manager_c* for every function above. */
 target_manager_c* target_tick_manager_new(const char* file, int device);
+/* The same node loop over n_shards devices (devices[r], NULL = 0 .. n_shards-1; a device may repeat), owner(id) = id mod n_shards:
+ * every /tf message is routed to the owners on the devices (te_group_route_records), every shard ticks on its own device at once.
+ * The handle is valid for every target_tick_manager_* and every target_manager_* call above (target_manager_shards,
+ * target_manager_gather_estimates included).  Differences from a one-device handle: target_tick_manager_published lists the poses
+ * shard-major (shard 0's targets in ascending id, then shard 1's, ...: target_manager_get_dense_ids order); erased ids stay one
+ * ascending list. */
+target_manager_c* target_tick_manager_new_sharded(const char* file, int n_shards, const int* devices);
 void target_tick_manager_set_expiration(const target_manager_c* self, double timeout_s);
 void target_tick_manager_set_token(const target_manager_c* self, const char* token);
 /* gather the filtered poses after every tick (the TF broadcast of src/target_manager_ros.cpp:78-87; default on) or leave them on the
@@ -110,7 +117,7 @@ void target_tick_manager_callback_ids(const target_manager_c* self, long long n,
  * rule (their ids, ascending, into erased_out up to cap), or -1 on error */
 long long target_tick_manager_update(const target_manager_c* self, double dt, unsigned int now_sec, unsigned int now_nsec,
                                      unsigned int* erased_out, long long cap);
-/* the filtered poses broadcast by the last tick: ascending ids + [n][7]; returns n */
+/* the filtered poses broadcast by the last tick: ascending ids (shard-major on a sharded handle) + [n][7]; returns n */
 long long target_tick_manager_published(const target_manager_c* self, unsigned int* ids_out, double* poses_out, long long cap);
 double target_tick_manager_time(const target_manager_c* self);
 long long target_tick_manager_mailboxes(const target_manager_c* self);

@@ -261,6 +261,19 @@ const uint32_t* te_group_dev_ids(te_group* g, int r);
 long long te_group_fetch(te_group* g, int root, double* records_out, uint32_t* ids_out, long long cap);
 /* device time of the last gather (ms, max over the devices; CUDA events around the collective on every device's stream) */
 double te_group_last_gather_ms(te_group* g);
+/* Route one /tf message (host arrays, arrival order; should be page-locked) to the shards' devices: record k belongs to shard
+ * ids[k] mod G.  The message is cut into G contiguous chunks by position; chunk c is copied to shard c's device (the G links copy at
+ * once) and partitioned there by owner, stably (te_route_partition_kernel); then every shard receives its runs, [from chunk 0 | from
+ * chunk 1 | ...], over grouped NCCL send / receive between distinct devices, by device copies otherwise.  Arrival order per id is
+ * kept.  pools[r] = the pool of shard r (its device and stream; none may be NULL).  Asynchronous, ordered on each pool's stream like
+ * te_group_allgather_estimates (the host waits only for the G x G owner counts).  Afterwards te_group_routed() gives shard r's
+ * records on its own device, in arrival order: four SoA arrays that te_pool_mailbox_ingest_dev takes as they are (valid until the
+ * next routed message).  counts_out[r] (optional) = records of shard r.  The buffers grow with the largest message seen and are
+ * reused.  Returns n, -1 on error. */
+long long te_group_route_records(te_group* g, te_pool* const* pools, long long n, const uint32_t* ids, const uint32_t* sec,
+                                 const uint32_t* nsec, const double* poses /*[n][7]*/, long long* counts_out);
+int te_group_routed(te_group* g, int r, long long* n, const uint32_t** dev_ids, const uint32_t** dev_sec,
+                    const uint32_t** dev_nsec, const double** dev_poses);
 
 /* ---- device micro-benchmarks behind the roofline statements (csrc/te_diag.cu; not on any product path) ---------------------- */
 /* FP64 FMA rate of `device` in TFLOP/s (dependent-chain kernel, 8 chains per thread, best of 5) and the rate of a plain streaming

@@ -95,6 +95,8 @@ SIGNATURES = {
     "te_group_dev_ids": (_p, [_p, _i]),
     "te_group_fetch": (_ll, [_p, _i, _p, _p, _ll]),
     "te_group_last_gather_ms": (_d, [_p]),
+    "te_group_route_records": (_ll, [_p, _p, _ll, _p, _p, _p, _p, _p]),
+    "te_group_routed": (_i, [_p, _i, _p, _p, _p, _p, _p]),
 }
 
 for _name, (_res, _args) in SIGNATURES.items():

@@ -111,18 +111,20 @@ int mailbox_ingest_impl(te_pool* p, long long n, const uint32_t* ids, const uint
                           tw[1] - tw[0], tw[2] - tw[1], tw[3] - tw[2], tw[4] - tw[3], n_unknown);
     return 0;
   }
-  // device source: pack the unknown records (device order) into one block [pose 7 | index | id | sec | nsec] x n_unknown, read it
-  // back in one copy to pinned memory, queue the records in arrival order
+  // device source: pack the unknown records into one block [pose 7 | index | id | sec | nsec] x n_unknown, read it back in one copy
+  // to pinned memory, queue the records in arrival order.  With targets in the pool the stable sort has left the unknown records at
+  // the end of rec_out in arrival order already; otherwise the lookup's list is in completion order and is sorted here
   const size_t nu = (size_t)n_unknown;
+  const int* list = p->n > 0 ? rec_out + (nr - n_unknown) : unknown;
   char* d_blk = (char*)p->arena.get(nu * 72);
   double* o_pose = (double*)d_blk;
   int* o_idx = (int*)(o_pose + 7 * nu);
   uint32_t* o_ids = (uint32_t*)(o_idx + nu);
   uint32_t* o_sec = o_ids + nu;
   uint32_t* o_nsec = o_sec + nu;
-  te::mb_pack_unknown_kernel<<<cdiv(n_unknown, 256), 256, 0, p->stream>>>(n_unknown, unknown, d_ids, d_sec, d_nsec, d_pose, o_ids, o_sec, o_nsec, o_pose);
+  te::mb_pack_unknown_kernel<<<cdiv(n_unknown, 256), 256, 0, p->stream>>>(n_unknown, list, d_ids, d_sec, d_nsec, d_pose, o_ids, o_sec, o_nsec, o_pose);
   CK(cudaGetLastError());
-  CK(cudaMemcpyAsync(o_idx, unknown, nu * sizeof(int), cudaMemcpyDeviceToDevice, p->stream));
+  CK(cudaMemcpyAsync(o_idx, list, nu * sizeof(int), cudaMemcpyDeviceToDevice, p->stream));
   char* h_blk = pinned_stage(p, nu * 72);
   CK(cudaMemcpyAsync(h_blk, d_blk, nu * 72, cudaMemcpyDeviceToHost, p->stream));
   CK(cudaStreamSynchronize(p->stream));

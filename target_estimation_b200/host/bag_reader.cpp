@@ -159,7 +159,7 @@ std::vector<TfRecord> readBagTf(const std::string& path, const std::string& topi
   return std::move(p.out);
 }
 
-ReplayStats replayBag(TickTargetManager& mgr, const std::vector<TfRecord>& rec, double frequency, long long extra_ticks) {
+ReplayStats replayBag(TickFrontEnd& mgr, const std::vector<TfRecord>& rec, double frequency, long long extra_ticks) {
   if (!(frequency > 0.0)) throw std::invalid_argument("frequency must be > 0");
   ReplayStats st;
   if (rec.empty()) return st;

@@ -86,19 +86,6 @@ class ShardWorkers {
 };
 
 namespace {
-// id mod G without a division per record (the routing passes look at every id of a batch; a hardware divide per id cost more than
-// the tick it feeds): a mask for powers of two, else Lemire's multiply-shift remainder, exact for 32-bit operands
-struct FastMod {
-  explicit FastMod(unsigned d) : d_(d), pow2_((d & (d - 1)) == 0), m_(~(unsigned long long)0 / d + 1) {}
-  unsigned operator()(unsigned a) const {
-    if (pow2_) return a & (d_ - 1);
-    const unsigned long long low = m_ * a;
-    return (unsigned)(((unsigned __int128)low * d_) >> 64);
-  }
-  unsigned d_;
-  bool pow2_;
-  unsigned long long m_;
-};
 // page-locked staging of one shard (the shard's batched calls copy from it at PCIe speed)
 void stageReserve(double*& meas, unsigned char*& action, size_t& cap, size_t n) {
   if (n <= cap) return;
@@ -114,7 +101,12 @@ void stageReserve(double*& meas, unsigned char*& action, size_t& cap, size_t n) 
 }
 }  // namespace
 
-ShardedTargetManager::ShardedTargetManager(const std::string& file, int n_shards, const int* devices) : TargetManager(file, devices ? devices[0] : 0) {
+ShardedTargetManager::ShardedTargetManager(const std::string& file, int n_shards, const int* devices)
+    : ShardedTargetManager(file, n_shards, devices, [&file](int d) { return new TargetManager(file, d); }) {}
+
+ShardedTargetManager::ShardedTargetManager(const std::string& file, int n_shards, const int* devices,
+                                           const std::function<TargetManager*(int)>& make_shard)
+    : TargetManager(file, devices ? devices[0] : 0) {
   if (n_shards <= 0) throw std::invalid_argument("a sharded manager needs at least one shard");
   const int n_dev = te_device_count();
   if (n_dev <= 0) throw std::runtime_error("no CUDA device available");
@@ -122,7 +114,7 @@ ShardedTargetManager::ShardedTargetManager(const std::string& file, int n_shards
     const int d = devices ? devices[r] : r;
     if (d < 0 || d >= n_dev) throw std::invalid_argument("no such CUDA device: " + std::to_string(d));
     devices_.push_back(d);
-    shard_.emplace_back(new TargetManager(file, d));
+    shard_.emplace_back(make_shard(d));
     shard_.back()->quiet = true;
   }
   stage_.resize((size_t)n_shards);
@@ -143,10 +135,9 @@ ShardedTargetManager::~ShardedTargetManager() {
   }
 }
 
-template <class F> void ShardedTargetManager::forEachShard(F&& f) {
+void ShardedTargetManager::forEachShard(const std::function<void(int)>& f) {
   if (shard_.size() == 1) { f(0); return; }
-  const std::function<void(int)> fn = std::forward<F>(f);
-  workers_->run(fn);
+  workers_->run(f);
 }
 
 // ---- per-id calls: the owner's ------------------------------------------------------------------------------------------
@@ -222,12 +213,42 @@ long long ShardedTargetManager::updateBatch(long long n, const unsigned* ids, do
   const unsigned G = (unsigned)shard_.size();
   const FastMod owner_of(G);
   if (G == 1) return shard_[0]->updateBatch(n, ids, dt, meas, action);
-  // Routing = a parallel stable partition of the batch by owner, every access sequential.  Routing thread t (there are as many as
-  // the host offers, at most 16, at least G) takes the t-th contiguous chunk of the records: (1) it counts the owners in its chunk; the prefix sums give chunk t a place in every shard's staging behind the
-  // chunks before it; (2) it streams its chunk once more and appends every record to its owner's staging (G write streams per
-  // worker).  Inside a shard the records keep the caller's order (chunks are ordered, and so is each chunk), so the records of one
-  // id stay in sequence.  (3) every shard runs its batched call on its own staging.  (A pass per shard over the whole batch, each
-  // picking its own records out, gathered 56-byte records at a stride of G records: 300 ms for 33 M records on 8 shards.)
+  const std::vector<size_t> total = routeOnHost(
+      n, ids,
+      [&](int r, size_t m) {   // (each worker sizes its own shard's staging: page-locking is the slow part and runs in parallel)
+        Stage& st = stage_[(size_t)r];
+        st.ids.resize(m);
+        stageReserve(st.meas, st.action, st.cap, m);
+      },
+      [&](int, long long lo, long long hi, size_t* at) {
+        for (long long k = lo; k < hi; ++k) {
+          const unsigned r = owner_of(ids[k]);
+          Stage& st = stage_[r];
+          const size_t j = at[r]++;
+          st.ids[j] = ids[k];
+          if (meas) std::memcpy(st.meas + 7 * j, meas + 7 * (size_t)k, 56);
+          st.action[j] = action ? action[k] : (unsigned char)TE_ACT_UPDATE;
+        }
+      });
+  std::atomic<long long> applied{0};
+  forEachShard([&](int r) {
+    Stage& st = stage_[(size_t)r];
+    if (total[(size_t)r] == 0) return;
+    applied += shard_[(size_t)r]->updateBatch((long long)total[(size_t)r], st.ids.data(), dt, meas ? st.meas : nullptr, st.action);
+  });
+  return applied.load();
+}
+
+// Routing = a parallel stable partition of the batch by owner, every access sequential.  Routing thread t (there are as many as
+// the host offers, at most 16, at least G) takes the t-th contiguous chunk of the records: (1) it counts the owners in its chunk; the
+// prefix sums give chunk t a place in every shard's staging behind the chunks before it; (2) it streams its chunk once more and
+// appends every record to its owner's staging (G write streams per worker).  Inside a shard the records keep the caller's order
+// (chunks are ordered, and so is each chunk), so the records of one id stay in sequence.  (A pass per shard over the whole batch,
+// each picking its own records out, gathered 56-byte records at a stride of G records: 300 ms for 33 M records on 8 shards.)
+std::vector<size_t> ShardedTargetManager::routeOnHost(long long n, const unsigned* ids, const std::function<void(int, size_t)>& reserve,
+                                                      const std::function<void(int, long long, long long, size_t*)>& scatter) {
+  const unsigned G = (unsigned)shard_.size();
+  const FastMod owner_of(G);
   const unsigned T = (unsigned)routers_->size();   // routing threads (>= G)
   std::vector<size_t> count((size_t)T * G, 0);     // [chunk t][owner r]
   auto chunk_lo = [&](unsigned t) { return (long long)((__int128)n * t / T); };
@@ -243,30 +264,13 @@ long long ShardedTargetManager::updateBatch(long long n, const unsigned* ids, do
       offset[(size_t)t * G + r] = total[r];
       total[r] += count[(size_t)t * G + r];
     }
-  forEachShard([&](int r) {   // (each worker sizes its own shard's staging: page-locking is the slow part and runs in parallel)
-    Stage& st = stage_[(size_t)r];
-    st.ids.resize(total[(size_t)r]);
-    stageReserve(st.meas, st.action, st.cap, total[(size_t)r]);
-  });
+  forEachShard([&](int r) { reserve(r, total[(size_t)r]); });
   const std::function<void(int)> scatter_pass = [&](int t) {
     std::vector<size_t> at(offset.begin() + (long)t * G, offset.begin() + (long)(t + 1) * G);
-    for (long long k = chunk_lo((unsigned)t), e = chunk_lo((unsigned)t + 1); k < e; ++k) {
-      const unsigned r = owner_of(ids[k]);
-      Stage& st = stage_[r];
-      const size_t j = at[r]++;
-      st.ids[j] = ids[k];
-      if (meas) std::memcpy(st.meas + 7 * j, meas + 7 * (size_t)k, 56);
-      st.action[j] = action ? action[k] : (unsigned char)TE_ACT_UPDATE;
-    }
+    scatter(t, chunk_lo((unsigned)t), chunk_lo((unsigned)t + 1), at.data());
   };
   routers_->run(scatter_pass);
-  std::atomic<long long> applied{0};
-  forEachShard([&](int r) {
-    Stage& st = stage_[(size_t)r];
-    if (total[(size_t)r] == 0) return;
-    applied += shard_[(size_t)r]->updateBatch((long long)total[(size_t)r], st.ids.data(), dt, meas ? st.meas : nullptr, st.action);
-  });
-  return applied.load();
+  return total;
 }
 
 long long ShardedTargetManager::eraseBatch(long long n, const unsigned* ids) {
@@ -353,13 +357,15 @@ void ShardedTargetManager::updateDenseWait(int lag) {
 }
 
 // ---- the optional exchange of estimates ----------------------------------------------------------------------------------------
-bool ShardedTargetManager::gatherUsesNccl() {
+te_group* ShardedTargetManager::group() {
   if (!group_) {
     group_ = te_group_create((int)devices_.size(), devices_.data());
     if (!group_) throw std::runtime_error(te_last_error());
   }
-  return te_group_uses_nccl(group_) == 1;
+  return group_;
 }
+
+bool ShardedTargetManager::gatherUsesNccl() { return te_group_uses_nccl(group()) == 1; }
 
 long long ShardedTargetManager::gatherEstimates(std::vector<unsigned>* ids, std::vector<double>* records13, int publisher) {
   if (publisher < 0 || publisher >= (int)shard_.size()) throw std::invalid_argument("no such shard");

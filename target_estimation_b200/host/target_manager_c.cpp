@@ -237,8 +237,8 @@ int target_manager_gather_uses_nccl(const target_manager_c* self) {
 }
 
 // ---- tick front-end ---------------------------------------------------------------------------------
-static TickTargetManager* T(const target_manager_c* self) {
-  TickTargetManager* t = dynamic_cast<TickTargetManager*>(M(self));
+static TickFrontEnd* T(const target_manager_c* self) {
+  TickFrontEnd* t = dynamic_cast<TickFrontEnd*>(M(self));
   if (!t) throw std::invalid_argument("handle is not a tick manager");
   return t;
 }
@@ -247,6 +247,13 @@ target_manager_c* target_tick_manager_new(const char* file, int device) {
     if (!file || !file[0]) throw std::invalid_argument("a model file is required");
     TargetManager* m = new TickTargetManager(std::string(file), device);
     m->quiet = true;
+    return (target_manager_c*)m;
+  });
+}
+target_manager_c* target_tick_manager_new_sharded(const char* file, int n_shards, const int* devices) {
+  return guard((target_manager_c*)nullptr, [&]() -> target_manager_c* {
+    if (!file || !file[0]) throw std::invalid_argument("a model file is required");
+    TargetManager* m = new ShardedTickTargetManager(std::string(file), n_shards, devices);
     return (target_manager_c*)m;
   });
 }

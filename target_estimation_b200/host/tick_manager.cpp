@@ -57,18 +57,16 @@ te_pool* TickTargetManager::tickPool() {
   return pool;
 }
 
-void TickTargetManager::measurementCallBack(long long n, const char* const* frames, const uint32_t* sec, const uint32_t* nsec,
-                                            const double* poses) {   // :26-39
-  std::lock_guard<std::recursive_mutex> lg(target_lock_);
+void TickFrontEnd::parseFrames(const std::string& token, long long n, const char* const* frames, const uint32_t* sec, const uint32_t* nsec,
+                               const double* poses, std::vector<unsigned>& ids, std::vector<uint32_t>& s, std::vector<uint32_t>& ns,
+                               std::vector<double>& p) {   // :26-39
   // frame names -> ids; the loop ends at the first frame that carries the token but does not parse (e.g. the node's own
   // "<token>_filt_<id>" output frames, SURVEY.md H10); frames without the token are skipped
-  std::vector<unsigned> ids;
-  std::vector<uint32_t> s, ns;
-  std::vector<double> p;
+  ids.clear(); s.clear(); ns.clear(); p.clear();
   ids.reserve((size_t)n); s.reserve((size_t)n); ns.reserve((size_t)n); p.reserve((size_t)n * 7);
   for (long long i = 0; i < n; ++i) {
     const std::string name(frames[i]);
-    if (name.find(token_name_) != std::string::npos) {
+    if (name.find(token) != std::string::npos) {
       unsigned id;
       if (!getId(name, id)) break;
       ids.push_back(id);
@@ -77,7 +75,32 @@ void TickTargetManager::measurementCallBack(long long n, const char* const* fram
       p.insert(p.end(), poses + 7 * i, poses + 7 * i + 7);
     }
   }
+}
+
+void TickTargetManager::measurementCallBack(long long n, const char* const* frames, const uint32_t* sec, const uint32_t* nsec,
+                                            const double* poses) {
+  std::lock_guard<std::recursive_mutex> lg(target_lock_);
+  std::vector<unsigned> ids;
+  std::vector<uint32_t> s, ns;
+  std::vector<double> p;
+  parseFrames(token_name_, n, frames, sec, nsec, poses, ids, s, ns, p);
   measurementCallBackIds((long long)ids.size(), ids.data(), s.data(), ns.data(), p.data());
+}
+
+// an id the manager knows under another model type, or a host mailbox, may be named: the records must be split per id
+bool TickTargetManager::foreignPossible(te_pool* pool) { return !measurements_.empty() || targets_.size() != (size_t)te_pool_size(pool); }
+
+te_pool* TickTargetManager::devicePool() {
+  std::lock_guard<std::recursive_mutex> lg(target_lock_);
+  flushLocked();
+  te_pool* pool = tickPool();
+  return foreignPossible(pool) ? nullptr : pool;
+}
+
+void TickTargetManager::ingestDev(long long n, const uint32_t* dev_ids, const uint32_t* dev_sec, const uint32_t* dev_nsec, const double* dev_poses) {
+  std::lock_guard<std::recursive_mutex> lg(target_lock_);
+  if (n <= 0) return;
+  if (te_pool_mailbox_ingest_dev(tickPool(), n, dev_ids, dev_sec, dev_nsec, dev_poses) < 0) throw std::runtime_error(te_last_error());
 }
 
 void TickTargetManager::measurementCallBackIds(long long n, const unsigned* ids, const uint32_t* sec, const uint32_t* nsec,
@@ -86,8 +109,7 @@ void TickTargetManager::measurementCallBackIds(long long n, const unsigned* ids,
   if (n <= 0) return;
   flushLocked();
   te_pool* pool = tickPool();
-  const bool foreign_possible = !measurements_.empty() || targets_.size() != (size_t)te_pool_size(pool);
-  if (!foreign_possible) {   // the whole message in one call: lookup, stable sort by slot, per-slot Measurement::update on the device
+  if (!foreignPossible(pool)) {   // the whole message in one call: lookup, stable sort by slot, per-slot Measurement::update on the device
     if (te_pool_mailbox_ingest(pool, n, ids, sec, nsec, poses) < 0) throw std::runtime_error(te_last_error());
     return;
   }
@@ -168,6 +190,31 @@ void TickTargetManager::tickForeign(const double& dt, uint32_t now_sec, uint32_t
 
 void TickTargetManager::tick(const double& dt, uint32_t now_sec, uint32_t now_nsec, std::vector<unsigned>* erased) {   // :41-92
   std::lock_guard<std::recursive_mutex> lg(target_lock_);
+  advance(dt, now_sec, now_nsec, erased);
+  // 3. the filtered poses the node broadcasts (:76-87)
+  if (!publish) {
+    pub_ids_.clear();
+    pub_poses_.clear();
+    return;
+  }
+  const long long n = publishCount();
+  // The output vectors keep their storage across ticks (no re-zeroing) and that storage is page-locked while it lasts, so the
+  // read-back of 56 B per target runs at PCIe speed instead of through the driver's pageable staging
+  if (pub_poses_.capacity() < (size_t)n * 7) {
+    if (pub_pinned_) te_host_unregister(pub_pinned_);
+    pub_pinned_ = nullptr;
+    pub_poses_.clear();
+    pub_poses_.reserve((size_t)(n + n / 4) * 7);
+    if (pub_poses_.capacity() * sizeof(double) >= (1u << 20) && te_host_register(pub_poses_.data(), pub_poses_.capacity() * sizeof(double)) == 0)
+      pub_pinned_ = pub_poses_.data();
+  }
+  pub_ids_.resize((size_t)n);
+  pub_poses_.resize((size_t)n * 7);
+  publishInto(pub_ids_.data(), pub_poses_.data(), n);
+}
+
+void TickTargetManager::advance(const double& dt, uint32_t now_sec, uint32_t now_nsec, std::vector<unsigned>* erased) {
+  std::lock_guard<std::recursive_mutex> lg(target_lock_);
   if (!(dt >= 0.0)) throw std::invalid_argument("dt must be >= 0");
   flushLocked();
   te_pool* pool = tickPool();
@@ -198,42 +245,28 @@ void TickTargetManager::tick(const double& dt, uint32_t now_sec, uint32_t now_ns
     }
   }
   if (erased) erased->assign(gone.begin(), gone.end());
-  // 3. the filtered poses the node broadcasts (:76-87)
-  if (!publish) {
-    pub_ids_.clear();
-    pub_poses_.clear();
-  } else {
-    const long long n_pool = te_pool_size(pool);
-    if (measurements_.empty() && targets_.size() == (size_t)n_pool) {
-      // every target lives in the tick's pool: ids and poses of all slots in slot order = ascending ids, no per-id lookups.
-      // The output vectors keep their storage across ticks (no re-zeroing) and that storage is page-locked while it lasts, so the
-      // read-back of 56 B per target runs at PCIe speed instead of through the driver's pageable staging
-      if (pub_poses_.capacity() < (size_t)n_pool * 7) {
-        if (pub_pinned_) te_host_unregister(pub_pinned_);
-        pub_pinned_ = nullptr;
-        pub_poses_.clear();
-        pub_poses_.reserve((size_t)(n_pool + n_pool / 4) * 7);
-        if (pub_poses_.capacity() * sizeof(double) >= (1u << 20) && te_host_register(pub_poses_.data(), pub_poses_.capacity() * sizeof(double)) == 0)
-          pub_pinned_ = pub_poses_.data();
-      }
-      pub_ids_.resize((size_t)n_pool);
-      pub_poses_.resize((size_t)n_pool * 7);
-      if (n_pool > 0) {
-        if (te_pool_ids(pool, pub_ids_.data(), n_pool) < 0 ||
-            te_pool_read_estimates(pool, n_pool, nullptr, nullptr, pub_poses_.data(), nullptr, nullptr, nullptr, nullptr) < 0)
-          throw std::runtime_error(te_last_error());
-      }
-    } else {
-      pub_ids_ = getAvailableTargets();
-      if (pub_poses_.capacity() < pub_ids_.size() * 7 && pub_pinned_) {   // the vector is about to move: unlock the old storage
-        te_host_unregister(pub_pinned_);
-        pub_pinned_ = nullptr;
-      }
-      pub_poses_.resize(pub_ids_.size() * 7);
-      if (!pub_ids_.empty()) getEstimatesBatch((long long)pub_ids_.size(), pub_ids_.data(), nullptr, pub_poses_.data(), nullptr, nullptr, nullptr);
-    }
-  }
   t_ = t_ + dt;   // :89
+}
+
+long long TickTargetManager::publishCount() {
+  std::lock_guard<std::recursive_mutex> lg(target_lock_);
+  return (long long)targets_.size();
+}
+
+void TickTargetManager::publishInto(unsigned* ids, double* poses, long long n) {
+  std::lock_guard<std::recursive_mutex> lg(target_lock_);
+  if (n != (long long)targets_.size()) throw std::logic_error("publishInto: the output does not fit the targets");
+  if (n == 0) return;
+  te_pool* pool = tickPool();
+  if (measurements_.empty() && targets_.size() == (size_t)te_pool_size(pool)) {
+    // every target lives in the tick's pool: ids and poses of all slots in slot order = ascending ids, no per-id lookups
+    if (te_pool_ids(pool, ids, n) < 0 || te_pool_read_estimates(pool, n, nullptr, nullptr, poses, nullptr, nullptr, nullptr, nullptr) < 0)
+      throw std::runtime_error(te_last_error());
+  } else {
+    const std::vector<unsigned> all = getAvailableTargets();
+    std::copy(all.begin(), all.end(), ids);
+    getEstimatesBatch(n, ids, nullptr, poses, nullptr, nullptr, nullptr);
+  }
 }
 
 size_t TickTargetManager::mailboxCount() {

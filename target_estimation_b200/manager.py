@@ -48,6 +48,7 @@ _SIG = {
     "target_manager_last_gather_ms": (_d, [_p]),
     "target_manager_gather_uses_nccl": (_i, [_p]),
     "target_tick_manager_new": (_p, [C.c_char_p, _i]),
+    "target_tick_manager_new_sharded": (_p, [C.c_char_p, _i, _p]),
     "target_tick_manager_set_expiration": (None, [_p, _d]),
     "target_tick_manager_set_token": (None, [_p, C.c_char_p]),
     "target_tick_manager_set_publish": (None, [_p, _i]),
@@ -308,3 +309,14 @@ class TickManagerC(TargetManagerC):
 
     def mailboxes(self):
         return int(clib.target_tick_manager_mailboxes(self.h))
+
+
+class ShardedTickManagerC(TickManagerC, ShardedManagerC):
+    """target_tick_manager_new_sharded: the node loop over n_shards devices (owner(id) = id mod n_shards), /tf messages routed to the
+    owners on the devices; published() is shard-major (dense_ids() order)"""
+
+    def __init__(self, yaml_file, n_shards, devices=None):
+        dev = np.ascontiguousarray(devices, dtype=np.int32) if devices is not None else None
+        self.h = clib.target_tick_manager_new_sharded(yaml_file.encode(), int(n_shards), _ptr(dev))
+        if not self.h:
+            raise RuntimeError("target_tick_manager_new_sharded failed: %s" % clib.target_manager_last_error().decode())
