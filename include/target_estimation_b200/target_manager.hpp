@@ -241,23 +241,70 @@ class MovingAvgFilter {
   bool complete_;
 };
 
-// intersection_solver.hpp:55-125.  One object = one reference solver (one pair of moving-average
-// filters + previous intersection pose shared by every id queried through it, SURVEY.md H9).
+// intersection_solver.hpp:55-125.  One solver STREAM = one reference solver (one pair of moving-average filters + previous
+// intersection pose shared by every id queried through it, SURVEY.md H9); every query through a stream updates it in call order.
+// The reference's per-id methods use stream 0.  query() is the batched form: query k goes through stream[k] (NULL = k).
+// A manager holding several model types keeps one state per stream and model type (the filters live beside the pool they are
+// used with; a reference solver used across model types would share them).
+// Any handle works: on a ShardedTargetManager (and so a ShardedTickTargetManager) the solver keeps one te_isolver per (shard, model
+// type) and the shard home[stream] that holds each stream's current state.  A call routes its queries to the owners of their ids
+// (in call order), moves the state of every stream whose home is another shard to the shard that now queries it
+// (te_isolver_move_streams, bit-exact), then queries all shards at once.  So the results are those of the same solver on one
+// plain manager, whichever shards the ids of a stream live on.  Memory: a shard allocates its stream arrays (n_streams x
+// (2 filters_length + 9) doubles + 5 bytes per model type) on its first query, so each device then holds what a single-device
+// solver of the same n_streams holds.
+class ShardedTargetManager;
 class IntersectionSolver {
  public:
   typedef std::shared_ptr<IntersectionSolver> Ptr;
-  IntersectionSolver(TargetManager::Ptr target_manager, const unsigned int filters_length = 250);
+  IntersectionSolver(TargetManager::Ptr target_manager, const unsigned int filters_length = 250, long long n_streams = 1);
   ~IntersectionSolver();
   double getIntersectionTimeWithSphere(const unsigned int& id, const double& t1, const Vector3d& origin, const double& radius);
   bool getIntersectionPoseWithSphere(const unsigned int& id, const double& t1, const double& pos_th, const double& ang_th,
                                      const Vector3d& origin, const double& radius, Vector7d& intersection_pose);
+  // n queries at once: delta[k] as getIntersectionTimeWithSphere, pose7[k] / converged[k] as getIntersectionPoseWithSphere through
+  // stream[k] (stream NULL = k, then n <= streams() for pose queries); pose7 NULL = times only (no stream is touched, pos_th / ang_th may be NULL);
+  // delta / converged may be NULL.  A stream may appear more than once: the batch is then cut in front of each repeat and the
+  // pieces run in order, so a batch always equals the same queries issued one by one.  An unknown id gives -1 / initPose / false
+  // and leaves its stream untouched.  Returns the number of queries whose id exists.
+  long long query(long long n, const unsigned* ids, const int* stream, const double* t1, const double* origin /*[n][3]*/,
+                  const double* radius, const double* pos_th, const double* ang_th, double* delta, double* pose7,
+                  unsigned char* converged);
+  long long streams() const { return n_streams_; }
+  // host wall time of the last query() by phase, ms: [0] routing by owner (and model type), [1] moves of stream state between
+  // shards, [2] the shards' te_isolver_query calls (uploads, kernels, read-backs; all shards at once), [3] results into call order
+  const double* lastPhaseMs() const { return phase_ms_; }
+
  private:
-  te_isolver* solverFor(int type);
+  struct Part {   // the queries of one shard in one call (a routed copy of the caller's rows)
+    std::vector<unsigned> ids;
+    std::vector<long long> where;   // caller's row
+    std::vector<int> stream;
+    std::vector<double> t1, origin, radius, pos_th, ang_th, delta, pose;
+    std::vector<unsigned char> conv;
+    int only = -1;                       // model type of the shard's targets, -1 = no target, -2 = several types (see type)
+    std::vector<signed char> type;       // several types: model type per query, -1 = unknown id
+    std::vector<std::vector<int>> moves;   // [type * G + source shard]: streams whose state comes from that shard
+    long long found = 0;
+  };
+  long long queryRun(long long n, const unsigned* ids, const int* stream, const double* t1, const double* origin, const double* radius,
+                     const double* pos_th, const double* ang_th, double* delta, double* pose7, unsigned char* converged);   // no stream twice
+  void classify(int r, long long m, const unsigned* ids);
+  void collectMoves(int r, long long m, const int* stream);
+  long long queryShard(int r, long long m, const unsigned* ids, const int* stream, const double* t1, const double* origin,
+                       const double* radius, const double* pos_th, const double* ang_th, double* delta, double* pose7, unsigned char* conv);
+  TargetManager& shardOf(int r);
+  te_isolver* solverFor(int r, int type);
   TargetManager::Ptr target_manager_;
+  ShardedTargetManager* sharded_ = nullptr;   // the manager as a sharded one, else NULL
   unsigned filters_length_;
-  // the filters live on the device with the pool they were last used with; a reference solver used
-  // across model types would share them -- documented limitation: one solver state per model type
-  te_isolver* solvers_[4] = {nullptr, nullptr, nullptr, nullptr};
+  long long n_streams_;
+  std::vector<std::array<te_isolver*, 4>> solvers_;   // [shard][model type], created on first use
+  std::vector<int> home_;                             // sharded: [type * n_streams + stream] shard of the state, -1 = fresh everywhere
+  std::vector<Part> part_;
+  std::vector<unsigned> seen_;                        // repeat detection: seen_[stream] == gen_ within the current piece
+  unsigned gen_ = 0;
+  double phase_ms_[4] = {0, 0, 0, 0};
 };
 
 // ---------------------------------------------------------------------------------------------------
@@ -452,6 +499,7 @@ class ShardedTargetManager : public TargetManager {
   std::vector<size_t> routeOnHost(long long n, const unsigned* ids, const std::function<void(int, size_t)>& reserve,
                                   const std::function<void(int, long long, long long, size_t*)>& scatter);
   te_group* group();   // created on first use
+  friend class IntersectionSolver;   // routes its queries with routeOnHost and runs them with forEachShard
   std::vector<std::unique_ptr<TargetManager>> shard_;
   std::vector<int> devices_;
   std::unique_ptr<ShardWorkers> workers_;   // one thread per shard: the shards' batched calls

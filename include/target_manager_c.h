@@ -81,7 +81,7 @@ void target_manager_flush(const target_manager_c* self);
 /* ---- all GPUs of the box behind one handle (BASELINE.json north_star: targets shard by id, no collective on the hot path) ----
  * n_shards TargetManagers, shard r on CUDA device devices[r] (NULL = devices 0 .. n_shards-1), owner(id) = id mod n_shards.  The
  * handle is a valid target_manager_c* for every function above: per-id calls go to the owner, the *_batch calls route their records
- * to the owners on the host and run on all devices at once.  (IntersectionSolver objects attach to one shard's manager.) */
+ * to the owners on the host and run on all devices at once.  target_isolver_* (below) works on it as on a plain manager. */
 target_manager_c* target_manager_new_sharded(const char* file, int n_shards, const int* devices);
 /* number of shards behind the handle (1 for a plain manager) */
 int target_manager_shards(const target_manager_c* self);
@@ -151,6 +151,33 @@ int target_manager_write_log(const target_manager_c* self, const char* folder);
 /* writeTxtFile itself (utils.hpp:78-120): cols == 1 writes the vector form */
 int target_write_txt_file(const char* filename, const double* values, long long rows, long long cols);
 const char* target_manager_last_error(void);
+
+/* ---- IntersectionSolver (src/intersection_solver.cpp:42-124) on any handle: plain, on-device, sharded, tick, sharded tick ----
+ * One solver holds n_streams solver streams; one stream = one reference IntersectionSolver object (previous intercept pose + two
+ * moving-average windows of filters_length samples), updated by every pose query through it, in call order.  The per-id calls use
+ * stream 0.  On a sharded handle every stream's state follows its queries from shard to shard (moved between the devices,
+ * bit-exact), so the results equal those of the same solver on a plain manager.  A manager holding several model types keeps one
+ * state per stream and model type.  The solver does not own the manager: delete it before the manager.  Errors: NULL / -1 / false
+ * with target_manager_last_error(). */
+typedef void target_isolver_c;
+target_isolver_c* target_isolver_new(const target_manager_c* m, long long n_streams, unsigned filters_length);
+void target_isolver_delete(target_isolver_c* s);
+/* getIntersectionTimeWithSphere: time to the first contact with the sphere, -1 = none or unknown id */
+double target_isolver_get_time(const target_isolver_c* s, unsigned id, double t1, const double origin[3], double radius);
+/* getIntersectionPoseWithSphere: pose[7] = intercept pose (initPose 0 0 0 0 0 0 1 if none); true once both filtered errors are
+ * below the thresholds.  t1, pos_th and ang_th must be >= 0. */
+bool target_isolver_get_pose(const target_isolver_c* s, unsigned id, double t1, double pos_th, double ang_th, const double origin[3],
+                             double radius, double pose[7]);
+/* n queries at once: query k = ids[k] through stream[k] (NULL = k, then n <= n_streams for pose queries) at t1[k], sphere origin[k][3] / radius[k],
+ * thresholds pos_th[k] / ang_th[k].  delta_out[k] = the time, pose7_out[k][7] / converged_out[k] = the pose query (pose7_out NULL =
+ * times only: no stream is touched and the thresholds may be NULL); any output may be NULL.  A stream named more than once is
+ * updated in call order, as by the same queries one by one.  Returns the number of queries whose id exists, -1 on error. */
+long long target_isolver_query_batch(const target_isolver_c* s, long long n, const unsigned int* ids, const int* stream, const double* t1,
+                                     const double* origin, const double* radius, const double* pos_th, const double* ang_th,
+                                     double* delta_out, double* pose7_out, unsigned char* converged_out);
+/* host wall time of the last query by phase, ms: routing, stream moves between shards, the shards' device queries, results into
+ * call order; returns 0, -1 on error */
+int target_isolver_last_timing(const target_isolver_c* s, double ms_out[4]);
 
 #ifdef __cplusplus
 }

@@ -226,10 +226,17 @@ te_isolver* te_isolver_create(te_pool* p, long long n_streams, unsigned filters_
 void te_isolver_destroy(te_isolver* s);
 /* query k: target ids[k] through solver stream stream[k] (NULL = k).  Each stream may appear at most
  * once per call.  delta_t[k] = getIntersectionTimeWithSphere (-1 = none); pose7/converged as
- * getIntersectionPoseWithSphere (pass pose7 NULL to only compute delta_t without touching filters). */
+ * getIntersectionPoseWithSphere (pass pose7 NULL to only compute delta_t without touching filters).
+ * Returns the number of queries whose id exists. */
 int te_isolver_query(te_isolver* s, long long n, const uint32_t* ids, const int32_t* stream, const double* t1,
                      const double* origin /*[n][3]*/, const double* radius, const double* pos_th, const double* ang_th,
                      double* delta_t, double* pose7, uint8_t* converged);
+/* Move the complete state of the listed streams (previous pose, both windows, both sums, window index, complete flag) from src to
+ * dst: two solvers of the same model type and filters_length, usually of pools on two devices.  Afterwards stream streams[k] of dst
+ * holds, byte for byte, what stream streams[k] of src held; src keeps its copy.  The streams are gathered into one block on src's
+ * device (isolver_pack_streams_kernel), copied once (peer copy between devices, device copy on one), and scattered on dst's device
+ * (isolver_unpack_streams_kernel).  Each solver's staging grows only when a move is larger than any before.  Synchronous. */
+int te_isolver_move_streams(te_isolver* src, te_isolver* dst, long long n, const int32_t* streams);
 
 /* Dense device-resident form: one query per slot (query k = slot k = solver stream k; needs n_streams >= pool size).
  * dev_t1 NULL = each target's own time; dev_delta / dev_pose7 / dev_converged may be NULL.  Asynchronous. */

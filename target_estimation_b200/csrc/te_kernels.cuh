@@ -916,4 +916,49 @@ __global__ void isolver_kernel(const double* __restrict__ tiles, const int* __re
   if (conv_out) conv_out[k] = converged ? 1 : 0;
 }
 
+// queries whose id exists (slot >= 0), added to *count
+static __global__ void isolver_count_found_kernel(const int* __restrict__ slots, long long n, unsigned long long* count) {
+  const long long k = blockIdx.x * (long long)blockDim.x + threadIdx.x;
+  const unsigned found = __ballot_sync(0xffffffffu, k < n && slots[k] >= 0);
+  if ((threadIdx.x & 31) == 0 && found) atomicAdd(count, (unsigned long long)__popc(found));
+}
+
+// The complete state of n solver streams as one block of ISOLVER_ROWS(L) rows of n doubles, row-major, column j = streams[j]:
+// prev_pose (7 rows) | pos_win (L) | ang_win (L) | pos_sum | ang_sum | idx | complete.  idx and complete are small integers,
+// exact in a double, so pack + unpack moves every byte of the state unchanged.  Thread i handles row i / n, column i % n: the block
+// is written (pack) and read (unpack) coalesced; the window rows are [L][n_streams] on both sides, so consecutive listed streams
+// are coalesced there too.
+__host__ __device__ inline long long isolver_rows(unsigned L) { return 2 * (long long)L + 11; }
+
+static __global__ void isolver_pack_streams_kernel(IsolverState st, const int* __restrict__ streams, long long n, double* __restrict__ block) {
+  const long long L = st.L, total = isolver_rows(st.L) * n;
+  for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
+    const long long row = i / n, s = streams[i - row * n];
+    double v;
+    if (row < 7) v = st.prev_pose[s * 7 + row];
+    else if (row < 7 + L) v = st.pos_win[(row - 7) * st.n_streams + s];
+    else if (row < 7 + 2 * L) v = st.ang_win[(row - 7 - L) * st.n_streams + s];
+    else if (row == 7 + 2 * L) v = st.pos_sum[s];
+    else if (row == 8 + 2 * L) v = st.ang_sum[s];
+    else if (row == 9 + 2 * L) v = (double)st.idx[s];
+    else v = (double)st.complete[s];
+    block[i] = v;
+  }
+}
+
+static __global__ void isolver_unpack_streams_kernel(IsolverState st, const int* __restrict__ streams, long long n, const double* __restrict__ block) {
+  const long long L = st.L, total = isolver_rows(st.L) * n;
+  for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
+    const long long row = i / n, s = streams[i - row * n];
+    const double v = block[i];
+    if (row < 7) st.prev_pose[s * 7 + row] = v;
+    else if (row < 7 + L) st.pos_win[(row - 7) * st.n_streams + s] = v;
+    else if (row < 7 + 2 * L) st.ang_win[(row - 7 - L) * st.n_streams + s] = v;
+    else if (row == 7 + 2 * L) st.pos_sum[s] = v;
+    else if (row == 8 + 2 * L) st.ang_sum[s] = v;
+    else if (row == 9 + 2 * L) st.idx[s] = (unsigned)v;
+    else st.complete[s] = (uint8_t)v;
+  }
+}
+
 }  // namespace te

@@ -219,6 +219,11 @@ struct te_pool {
 struct te_isolver {
   te_pool* pool = nullptr;
   te::IsolverState st{};
+  // te_isolver_move_streams: the packed streams and their indices on this solver's device (grow-only)
+  double* move_block = nullptr;
+  int* move_streams = nullptr;
+  size_t move_cap = 0;   // streams
+  unsigned long long* d_found = nullptr;   // te_isolver_query's count of existing ids
 };
 
 namespace tehost {

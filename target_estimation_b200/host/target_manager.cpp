@@ -5,6 +5,7 @@
 #include "target_estimation_b200/target_manager.hpp"
 
 #include <algorithm>
+#include <chrono>
 #include <cmath>
 #include <cstring>
 #include <fstream>
@@ -876,48 +877,273 @@ double MovingAvgFilter::update(double value) {
 // ----------------------------------------------------------------------------------------------
 // IntersectionSolver (src/intersection_solver.cpp:19-124)
 // ----------------------------------------------------------------------------------------------
-IntersectionSolver::IntersectionSolver(TargetManager::Ptr tm, const unsigned int filters_length)
-    : target_manager_(tm), filters_length_(filters_length) {
+IntersectionSolver::IntersectionSolver(TargetManager::Ptr tm, const unsigned int filters_length, long long n_streams)
+    : target_manager_(tm), filters_length_(filters_length), n_streams_(n_streams) {
   if (!tm) throw std::invalid_argument("IntersectionSolver needs a target manager (assert of src/intersection_solver.cpp:21)");
+  if (n_streams <= 0 || n_streams > 0x7fffffffLL) throw std::invalid_argument("n_streams must be in [1, 2^31)");
+  sharded_ = dynamic_cast<ShardedTargetManager*>(tm.get());
+  const int G = sharded_ ? sharded_->shards() : 1;
+  solvers_.assign((size_t)G, std::array<te_isolver*, 4>{nullptr, nullptr, nullptr, nullptr});
+  part_.resize((size_t)G);
+  for (Part& P : part_) P.moves.resize(4 * (size_t)G);
 }
 IntersectionSolver::~IntersectionSolver() {
-  for (te_isolver*& s : solvers_) {
-    if (s) te_isolver_destroy(s);
-    s = nullptr;
-  }
+  for (auto& per_shard : solvers_)
+    for (te_isolver*& s : per_shard) {
+      if (s) te_isolver_destroy(s);
+      s = nullptr;
+    }
 }
-te_isolver* IntersectionSolver::solverFor(int type) {
-  if (!solvers_[type]) {
-    solvers_[type] = te_isolver_create(target_manager_->poolOf(type, false), 1, filters_length_);
-    if (!solvers_[type]) throw PoolError(te_last_error());
+TargetManager& IntersectionSolver::shardOf(int r) { return sharded_ ? sharded_->shard(r) : *target_manager_; }
+te_isolver* IntersectionSolver::solverFor(int r, int type) {
+  te_isolver*& s = solvers_[(size_t)r][(size_t)type];
+  if (!s) {
+    s = te_isolver_create(shardOf(r).poolOf(type, false), n_streams_, filters_length_);
+    if (!s) throw PoolError(te_last_error());
   }
-  return solvers_[type];
+  return s;
 }
 double IntersectionSolver::getIntersectionTimeWithSphere(const unsigned int& id, const double& t1, const Vector3d& origin,
-                                                         const double& radius) {
-  std::lock_guard<std::recursive_mutex> lg(target_manager_->lock());
-  int type;
-  if (!target_manager_->typeOf(id, type)) return -1;   // :44,:87-88
-  target_manager_->flush();
-  const uint32_t uid = id;
+                                                         const double& radius) {   // :44-90
+  const int s0 = 0;
   double delta = -1.0;
-  ck(te_isolver_query(solverFor(type), 1, &uid, nullptr, &t1, origin.data(), &radius, nullptr, nullptr, &delta, nullptr, nullptr));
+  query(1, &id, &s0, &t1, origin.data(), &radius, nullptr, nullptr, &delta, nullptr, nullptr);
   return delta;
 }
 bool IntersectionSolver::getIntersectionPoseWithSphere(const unsigned int& id, const double& t1, const double& pos_th, const double& ang_th,
-                                                       const Vector3d& origin, const double& radius, Vector7d& intersection_pose) {
+                                                       const Vector3d& origin, const double& radius, Vector7d& intersection_pose) {   // :92-124
   if (!(t1 >= 0.0) || !(pos_th >= 0.0) || !(ang_th >= 0.0)) throw std::invalid_argument("t1, pos_th, ang_th must be >= 0 (:94-96)");
   intersection_pose = Vector7d{0, 0, 0, 0, 0, 0, 1};   // initPose (:99)
-  std::lock_guard<std::recursive_mutex> lg(target_manager_->lock());
-  int type;
-  if (!target_manager_->typeOf(id, type)) return false;
-  target_manager_->flush();
-  const uint32_t uid = id;
+  const int s0 = 0;
   double delta = -1.0;
   uint8_t conv = 0;
-  ck(te_isolver_query(solverFor(type), 1, &uid, nullptr, &t1, origin.data(), &radius, &pos_th, &ang_th, &delta, intersection_pose.data(),
-                      &conv));
+  query(1, &id, &s0, &t1, origin.data(), &radius, &pos_th, &ang_th, &delta, intersection_pose.data(), &conv);
   return conv != 0;
+}
+
+long long IntersectionSolver::query(long long n, const unsigned* ids, const int* stream, const double* t1, const double* origin,
+                                    const double* radius, const double* pos_th, const double* ang_th, double* delta, double* pose7,
+                                    unsigned char* converged) {
+  if (n < 0) throw std::invalid_argument("negative query count");
+  if (n > 0 && (!ids || !t1 || !origin || !radius)) throw std::invalid_argument("ids, t1, origin and radius are required");
+  if (pose7 && n > 0 && (!pos_th || !ang_th)) throw std::invalid_argument("thresholds are required with pose7");
+  if (!stream && pose7 && n > n_streams_) throw std::invalid_argument("more queries than solver streams (stream NULL = query index)");
+  if (stream)
+    for (long long k = 0; k < n; ++k)
+      if (stream[k] < 0 || stream[k] >= n_streams_) throw std::invalid_argument("bad stream index");
+  if (pose7)
+    for (long long k = 0; k < n; ++k)
+      if (!(t1[k] >= 0.0) || !(pos_th[k] >= 0.0) || !(ang_th[k] >= 0.0)) throw std::invalid_argument("t1, pos_th, ang_th must be >= 0 (:94-96)");
+  std::lock_guard<std::recursive_mutex> lg(target_manager_->lock());
+  std::fill(phase_ms_, phase_ms_ + 4, 0.0);
+  if (n == 0) return 0;
+  target_manager_->flush();
+  auto run = [&](long long lo, long long hi) {
+    return queryRun(hi - lo, ids + lo, stream ? stream + lo : nullptr, t1 + lo, origin + 3 * lo, radius + lo, pos_th ? pos_th + lo : nullptr,
+                    ang_th ? ang_th + lo : nullptr, delta ? delta + lo : nullptr, pose7 ? pose7 + 7 * lo : nullptr,
+                    converged ? converged + lo : nullptr);
+  };
+  // only queries with pose7 touch a stream: those are cut in front of every repeated stream, as TargetManager::updateBatch cuts
+  // in front of a repeated id
+  if (!stream || !pose7) return run(0, n);
+  if (seen_.empty()) seen_.assign((size_t)n_streams_, 0);
+  auto next_gen = [&] {
+    if (++gen_ == 0) {
+      std::fill(seen_.begin(), seen_.end(), 0u);
+      gen_ = 1;
+    }
+  };
+  next_gen();
+  long long found = 0, start = 0;
+  for (long long k = 0; k < n; ++k) {
+    unsigned& mark = seen_[(size_t)stream[k]];
+    if (mark == gen_) {
+      found += run(start, k);
+      start = k;
+      next_gen();
+    }
+    seen_[(size_t)stream[k]] = gen_;
+  }
+  return found + run(start, n);
+}
+
+// the model type(s) of shard r's targets: one pool in use -> every query goes to it (the kernel finds unknown ids itself); several
+// -> a host lookup per query
+void IntersectionSolver::classify(int r, long long m, const unsigned* ids) {
+  Part& P = part_[(size_t)r];
+  TargetManager& M = shardOf(r);
+  std::lock_guard<std::recursive_mutex> lg(M.lock());
+  int n_pools = 0;
+  P.only = -1;
+  for (int t = 0; t < 4; ++t) {
+    te_pool* p = M.poolOf(t, false);
+    if (p && te_pool_size(p) > 0) { ++n_pools; P.only = t; }
+  }
+  if (n_pools <= 1) return;
+  P.only = -2;
+  P.type.resize((size_t)m);
+  for (long long j = 0; j < m; ++j) {
+    int ty;
+    P.type[(size_t)j] = M.typeOf(ids[j], ty) ? (signed char)ty : (signed char)-1;
+  }
+}
+
+// the streams shard r queries whose state lives on another shard, grouped by (model type, source); home_ then names r.  (A stream
+// appears once per piece, so the shards' workers touch disjoint entries of home_.)
+void IntersectionSolver::collectMoves(int r, long long m, const int* stream) {
+  Part& P = part_[(size_t)r];
+  const int G = (int)part_.size();
+  for (auto& v : P.moves) v.clear();
+  for (long long j = 0; j < m; ++j) {
+    const int t = P.only >= 0 ? P.only : (P.only == -2 ? P.type[(size_t)j] : -1);
+    if (t < 0) continue;
+    int& h = home_[(size_t)t * (size_t)n_streams_ + (size_t)stream[j]];
+    if (h >= 0 && h != r) P.moves[(size_t)t * G + (size_t)h].push_back(stream[j]);
+    h = r;
+  }
+}
+
+long long IntersectionSolver::queryShard(int r, long long m, const unsigned* ids, const int* stream, const double* t1, const double* origin,
+                                         const double* radius, const double* pos_th, const double* ang_th, double* delta, double* pose7,
+                                         unsigned char* conv) {
+  Part& P = part_[(size_t)r];
+  std::lock_guard<std::recursive_mutex> lg(shardOf(r).lock());
+  if (!pose7) stream = nullptr;   // times only: no stream is read (and stream NULL = k may exceed the streams then)
+  if (P.only >= 0) {
+    const long long rc = te_isolver_query(solverFor(r, P.only), m, ids, stream, t1, origin, radius, pos_th, ang_th, delta, pose7, conv);
+    ck(rc);
+    return rc;
+  }
+  static const double init_pose[7] = {0, 0, 0, 0, 0, 0, 1};
+  for (long long j = 0; j < m; ++j) {   // unknown ids (all of them on a shard without targets)
+    if (delta) delta[j] = -1.0;
+    if (pose7) std::memcpy(pose7 + 7 * j, init_pose, sizeof(init_pose));
+    if (conv) conv[j] = 0;
+  }
+  if (P.only == -1) return 0;
+  long long found = 0;
+  std::vector<long long> rows;
+  std::vector<unsigned> s_ids;
+  std::vector<int> s_stream;
+  std::vector<double> s_t1, s_origin, s_radius, s_pth, s_ath, s_delta, s_pose;
+  std::vector<unsigned char> s_conv;
+  for (int t = 0; t < 4; ++t) {   // one sub-batch per model type
+    rows.clear();
+    for (long long j = 0; j < m; ++j)
+      if (P.type[(size_t)j] == t) rows.push_back(j);
+    const long long q = (long long)rows.size();
+    if (q == 0) continue;
+    s_ids.resize((size_t)q); s_stream.resize((size_t)q); s_t1.resize((size_t)q); s_origin.resize(3 * (size_t)q); s_radius.resize((size_t)q);
+    s_pth.resize(pos_th ? (size_t)q : 0); s_ath.resize(ang_th ? (size_t)q : 0);
+    s_delta.resize((size_t)q); s_pose.resize(pose7 ? 7 * (size_t)q : 0); s_conv.resize((size_t)q);
+    for (long long i = 0; i < q; ++i) {
+      const long long j = rows[(size_t)i];
+      s_ids[(size_t)i] = ids[j];
+      s_stream[(size_t)i] = stream ? stream[j] : (int)j;
+      s_t1[(size_t)i] = t1[j];
+      std::memcpy(&s_origin[3 * (size_t)i], origin + 3 * j, 24);
+      s_radius[(size_t)i] = radius[j];
+      if (pos_th) s_pth[(size_t)i] = pos_th[j];
+      if (ang_th) s_ath[(size_t)i] = ang_th[j];
+    }
+    const long long rc = te_isolver_query(solverFor(r, t), q, s_ids.data(), pose7 ? s_stream.data() : nullptr, s_t1.data(), s_origin.data(), s_radius.data(),
+                                          pos_th ? s_pth.data() : nullptr, ang_th ? s_ath.data() : nullptr, s_delta.data(),
+                                          pose7 ? s_pose.data() : nullptr, s_conv.data());
+    ck(rc);
+    found += rc;
+    for (long long i = 0; i < q; ++i) {
+      const long long j = rows[(size_t)i];
+      if (delta) delta[j] = s_delta[(size_t)i];
+      if (pose7) std::memcpy(pose7 + 7 * j, &s_pose[7 * (size_t)i], 56);
+      if (conv) conv[j] = pose7 ? s_conv[(size_t)i] : 0;
+    }
+  }
+  return found;
+}
+
+long long IntersectionSolver::queryRun(long long n, const unsigned* ids, const int* stream, const double* t1, const double* origin,
+                                       const double* radius, const double* pos_th, const double* ang_th, double* delta, double* pose7,
+                                       unsigned char* converged) {
+  typedef std::chrono::steady_clock clk;
+  auto ms_since = [](clk::time_point a) { return std::chrono::duration<double, std::milli>(clk::now() - a).count(); };
+  const int G = (int)part_.size();
+  clk::time_point t0 = clk::now();
+  if (G == 1 && !sharded_) {   // a plain manager: the caller's arrays as they are
+    classify(0, n, ids);
+    phase_ms_[0] += ms_since(t0);
+    t0 = clk::now();
+    const long long found = queryShard(0, n, ids, stream, t1, origin, radius, pos_th, ang_th, delta, pose7, converged);
+    phase_ms_[2] += ms_since(t0);
+    return found;
+  }
+  // 1. route: every shard's queries in call order
+  const FastMod owner_of((unsigned)G);
+  const bool with_pose = pose7 != nullptr;
+  const std::vector<size_t> total = sharded_->routeOnHost(
+      n, ids,
+      [&](int r, size_t m) {
+        Part& P = part_[(size_t)r];
+        P.ids.resize(m); P.where.resize(m); P.stream.resize(m); P.t1.resize(m); P.origin.resize(3 * m); P.radius.resize(m);
+        P.pos_th.resize(with_pose ? m : 0); P.ang_th.resize(with_pose ? m : 0);
+        P.delta.resize(m); P.pose.resize(with_pose ? 7 * m : 0); P.conv.resize(m);
+      },
+      [&](int, long long lo, long long hi, size_t* at) {
+        for (long long k = lo; k < hi; ++k) {
+          const unsigned r = owner_of(ids[k]);
+          Part& P = part_[r];
+          const size_t j = at[r]++;
+          P.ids[j] = ids[k];
+          P.where[j] = k;
+          P.stream[j] = stream ? stream[k] : (int)k;
+          P.t1[j] = t1[k];
+          std::memcpy(&P.origin[3 * j], origin + 3 * k, 24);
+          P.radius[j] = radius[k];
+          if (with_pose) { P.pos_th[j] = pos_th[k]; P.ang_th[j] = ang_th[k]; }
+        }
+      });
+  if (with_pose && home_.empty()) home_.assign(4 * (size_t)n_streams_, -1);
+  sharded_->forEachShard([&](int r) {
+    const long long m = (long long)total[(size_t)r];
+    classify(r, m, part_[(size_t)r].ids.data());
+    if (with_pose) collectMoves(r, m, part_[(size_t)r].stream.data());
+  });
+  phase_ms_[0] += ms_since(t0);
+  // 2. move the state of every stream that changes shard, one group per (model type, source, destination), before any query
+  t0 = clk::now();
+  if (with_pose)
+    for (int r = 0; r < G; ++r)
+      for (int t = 0; t < 4; ++t)
+        for (int h = 0; h < G; ++h) {
+          const std::vector<int>& v = part_[(size_t)r].moves[(size_t)t * G + (size_t)h];
+          if (!v.empty()) ck(te_isolver_move_streams(solverFor(h, t), solverFor(r, t), (long long)v.size(), v.data()));
+        }
+  phase_ms_[1] += ms_since(t0);
+  // 3. every shard queries at once
+  t0 = clk::now();
+  sharded_->forEachShard([&](int r) {
+    Part& P = part_[(size_t)r];
+    const long long m = (long long)total[(size_t)r];
+    P.found = m == 0 ? 0
+                     : queryShard(r, m, P.ids.data(), P.stream.data(), P.t1.data(), P.origin.data(), P.radius.data(),
+                                  with_pose ? P.pos_th.data() : nullptr, with_pose ? P.ang_th.data() : nullptr, P.delta.data(),
+                                  with_pose ? P.pose.data() : nullptr, with_pose ? P.conv.data() : nullptr);
+  });
+  phase_ms_[2] += ms_since(t0);
+  // 4. results into call order (rows of different shards are disjoint)
+  t0 = clk::now();
+  long long found = 0;
+  for (const Part& P : part_) found += P.found;
+  sharded_->forEachShard([&](int r) {
+    const Part& P = part_[(size_t)r];
+    for (size_t j = 0; j < total[(size_t)r]; ++j) {
+      const long long k = P.where[j];
+      if (delta) delta[k] = P.delta[j];
+      if (pose7) std::memcpy(pose7 + 7 * k, &P.pose[7 * j], 56);
+      if (converged) converged[k] = with_pose ? P.conv[j] : 0;
+    }
+  });
+  phase_ms_[3] += ms_since(t0);
+  return found;
 }
 
 // ----------------------------------------------------------------------------------------------

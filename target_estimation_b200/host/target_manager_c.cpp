@@ -33,6 +33,10 @@ template <class F, class R> R guard(R fallback, F&& f) {
   return fallback;
 }
 inline TargetManager* M(const target_manager_c* self) { return (TargetManager*)self; }
+inline IntersectionSolver* S(const target_isolver_c* s) {
+  if (!s) throw std::invalid_argument("null solver");
+  return (IntersectionSolver*)s;
+}
 }  // namespace
 
 extern "C" {
@@ -180,6 +184,46 @@ void target_manager_flush(const target_manager_c* self) {
   guard(0, [&] { M(self)->flush(); return 0; });
 }
 const char* target_manager_last_error(void) { return g_err.c_str(); }
+
+// ---- IntersectionSolver -------------------------------------------------------------------------------------------
+target_isolver_c* target_isolver_new(const target_manager_c* m, long long n_streams, unsigned filters_length) {
+  return guard((target_isolver_c*)nullptr, [&]() -> target_isolver_c* {
+    if (!m) throw std::invalid_argument("null manager");
+    if (n_streams <= 0) throw std::invalid_argument("n_streams must be > 0");
+    if (filters_length == 0) throw std::invalid_argument("filters_length must be > 0");
+    TargetManager::Ptr mp(M(m), [](TargetManager*) {});   // the caller owns the manager
+    return (target_isolver_c*)new IntersectionSolver(mp, filters_length, n_streams);
+  });
+}
+void target_isolver_delete(target_isolver_c* s) { delete (IntersectionSolver*)s; }
+double target_isolver_get_time(const target_isolver_c* s, unsigned id, double t1, const double origin[3], double radius) {
+  return guard(-1.0, [&] {
+    if (!origin) throw std::invalid_argument("origin is required");
+    return S(s)->getIntersectionTimeWithSphere(id, t1, Vector3d{origin[0], origin[1], origin[2]}, radius);
+  });
+}
+bool target_isolver_get_pose(const target_isolver_c* s, unsigned id, double t1, double pos_th, double ang_th, const double origin[3],
+                             double radius, double pose[7]) {
+  return guard(false, [&] {
+    if (!origin || !pose) throw std::invalid_argument("origin and pose are required");
+    Vector7d p;
+    const bool ok = S(s)->getIntersectionPoseWithSphere(id, t1, pos_th, ang_th, Vector3d{origin[0], origin[1], origin[2]}, radius, p);
+    std::memcpy(pose, p.data(), sizeof(double) * 7);
+    return ok;
+  });
+}
+long long target_isolver_query_batch(const target_isolver_c* s, long long n, const unsigned int* ids, const int* stream, const double* t1,
+                                     const double* origin, const double* radius, const double* pos_th, const double* ang_th,
+                                     double* delta_out, double* pose7_out, unsigned char* converged_out) {
+  return guard(-1LL, [&] { return S(s)->query(n, ids, stream, t1, origin, radius, pos_th, ang_th, delta_out, pose7_out, converged_out); });
+}
+int target_isolver_last_timing(const target_isolver_c* s, double ms_out[4]) {
+  return guard(-1, [&] {
+    if (!ms_out) throw std::invalid_argument("ms_out is required");
+    std::memcpy(ms_out, S(s)->lastPhaseMs(), sizeof(double) * 4);
+    return 0;
+  });
+}
 
 // ---- all GPUs of the box behind one handle --------------------------------------------------------------
 target_manager_c* target_manager_new_sharded(const char* file, int n_shards, const int* devices) {

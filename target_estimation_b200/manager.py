@@ -60,6 +60,12 @@ _SIG = {
     "target_tick_manager_mailboxes": (_ll, [_p]),
     "target_bag_read_tf": (_ll, [C.c_char_p, C.c_char_p, _p, _ll]),
     "target_tick_manager_replay_bag": (_ll, [_p, C.c_char_p, C.c_char_p, _d, _ll, _p]),
+    "target_isolver_new": (_p, [_p, _ll, _u]),
+    "target_isolver_delete": (None, [_p]),
+    "target_isolver_get_time": (_d, [_p, _u, _d, _p, _d]),
+    "target_isolver_get_pose": (C.c_bool, [_p, _u, _d, _d, _d, _p, _d, _p]),
+    "target_isolver_query_batch": (_ll, [_p, _ll, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p]),
+    "target_isolver_last_timing": (_i, [_p, _p]),
 }
 for _n, (_r, _a) in _SIG.items():
     _f = getattr(clib, _n)
@@ -320,3 +326,61 @@ class ShardedTickManagerC(TickManagerC, ShardedManagerC):
         self.h = clib.target_tick_manager_new_sharded(yaml_file.encode(), int(n_shards), _ptr(dev))
         if not self.h:
             raise RuntimeError("target_tick_manager_new_sharded failed: %s" % clib.target_manager_last_error().decode())
+
+
+class IntersectionSolverC:
+    """target_isolver_* on any manager handle above: n_streams reference IntersectionSolver objects (the per-id calls use stream 0)"""
+
+    def __init__(self, mgr, n_streams=1, filters_length=250):
+        self.mgr = mgr   # (the solver must go before its manager)
+        self.h = clib.target_isolver_new(mgr.h, int(n_streams), int(filters_length))
+        if not self.h:
+            raise RuntimeError("target_isolver_new failed: %s" % clib.target_manager_last_error().decode())
+
+    def close(self):
+        if getattr(self, "h", None):
+            clib.target_isolver_delete(self.h)
+            self.h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def time(self, id_, t1, origin, radius):
+        origin = np.ascontiguousarray(origin, dtype=np.float64)
+        return float(clib.target_isolver_get_time(self.h, int(id_), float(t1), _ptr(origin), float(radius)))
+
+    def pose(self, id_, t1, pos_th, ang_th, origin, radius):
+        """(converged, pose7)"""
+        origin = np.ascontiguousarray(origin, dtype=np.float64)
+        out = np.zeros(7)
+        ok = bool(clib.target_isolver_get_pose(self.h, int(id_), float(t1), float(pos_th), float(ang_th), _ptr(origin), float(radius), _ptr(out)))
+        return ok, out
+
+    def query_batch(self, ids, t1, origin, radius, pos_th=None, ang_th=None, stream=None, with_pose=True):
+        """(found, delta [n], pose [n][7] or None, converged [n] or None); t1 / origin / radius / thresholds broadcast to n"""
+        ids = np.ascontiguousarray(ids, dtype=np.uint32)
+        n = ids.size
+        t1 = np.ascontiguousarray(np.broadcast_to(t1, (n,)), dtype=np.float64)
+        origin = np.ascontiguousarray(np.broadcast_to(origin, (n, 3)), dtype=np.float64)
+        radius = np.ascontiguousarray(np.broadcast_to(radius, (n,)), dtype=np.float64)
+        pos_th = np.ascontiguousarray(np.broadcast_to(pos_th, (n,)), dtype=np.float64) if pos_th is not None else None
+        ang_th = np.ascontiguousarray(np.broadcast_to(ang_th, (n,)), dtype=np.float64) if ang_th is not None else None
+        stream = np.ascontiguousarray(stream, dtype=np.int32) if stream is not None else None
+        delta = np.zeros(n)
+        pose = np.zeros((n, 7)) if with_pose else None
+        conv = np.zeros(n, dtype=np.uint8) if with_pose else None
+        found = int(clib.target_isolver_query_batch(self.h, n, _ptr(ids), _ptr(stream), _ptr(t1), _ptr(origin), _ptr(radius), _ptr(pos_th),
+                                                    _ptr(ang_th), _ptr(delta), _ptr(pose), _ptr(conv)))
+        if found < 0:
+            raise RuntimeError(clib.target_manager_last_error().decode())
+        return found, delta, pose, conv
+
+    def last_timing(self):
+        """ms of the last query by phase: routing, moves, device, results into call order"""
+        ms = np.zeros(4)
+        if clib.target_isolver_last_timing(self.h, _ptr(ms)) < 0:
+            raise RuntimeError(clib.target_manager_last_error().decode())
+        return dict(zip(("route_ms", "move_ms", "device_ms", "writeback_ms"), (float(v) for v in ms)))
