@@ -270,6 +270,16 @@ class IntersectionSolver {
   long long query(long long n, const unsigned* ids, const int* stream, const double* t1, const double* origin /*[n][3]*/,
                   const double* radius, const double* pos_th, const double* ang_th, double* delta, double* pose7,
                   unsigned char* converged);
+  // The k earliest sphere intercepts over every target of the manager (te_pool_earliest_intersections on every (shard, model type)
+  // pool that holds targets; the shards of a sharded manager run at once).  Sphere j = (t1[j], origin[j][3], radius[j]); delta of
+  // target i is bit for bit query()'s time for (i, t1[j], origin[j], radius[j]), a hit is delta >= 0 (-0.0 ranks as 0).  hits_out[j] =
+  // the number of hits; rows 0 .. min(k, hits) - 1 of ids_out[j][.] / delta_out[j][.] are those hits by (delta, id), the pools' sorted
+  // lists merged on the host; the other rows are id 0xFFFFFFFF and delta -1.  The result does not depend on the shard count or on
+  // which pool holds a target.  Read-only: no solver stream is created or touched; queued per-id calls are flushed first.
+  // 0 <= k <= 65536 (k == 0: counts only, ids_out / delta_out may be NULL).  The intercept pose of a returned target is
+  // getEstimatesBatch(ids, t1 + delta).  Returns the total number of hits.
+  long long earliestIntersections(long long q, const double* t1, const double* origin /*[q][3]*/, const double* radius, long long k,
+                                  unsigned* ids_out /*[q][k]*/, double* delta_out /*[q][k]*/, long long* hits_out /*[q]*/);
   long long streams() const { return n_streams_; }
   // host wall time of the last query() by phase, ms: [0] routing by owner (and model type), [1] moves of stream state between
   // shards, [2] the shards' te_isolver_query calls (uploads, kernels, read-backs; all shards at once), [3] results into call order
@@ -304,6 +314,13 @@ class IntersectionSolver {
   std::vector<Part> part_;
   std::vector<unsigned> seen_;                        // repeat detection: seen_[stream] == gen_ within the current piece
   unsigned gen_ = 0;
+  struct SweepList {   // earliestIntersections: the sorted rows of one (shard, model type) pool (grow-only)
+    std::vector<unsigned> ids;
+    std::vector<double> delta;
+    std::vector<long long> hits;
+    bool used = false;
+  };
+  std::vector<SweepList> sweep_;                      // [shard * 4 + model type]
   double phase_ms_[4] = {0, 0, 0, 0};
 };
 

@@ -175,6 +175,14 @@ bool target_isolver_get_pose(const target_isolver_c* s, unsigned id, double t1, 
 long long target_isolver_query_batch(const target_isolver_c* s, long long n, const unsigned int* ids, const int* stream, const double* t1,
                                      const double* origin, const double* radius, const double* pos_th, const double* ang_th,
                                      double* delta_out, double* pose7_out, unsigned char* converged_out);
+/* The k earliest sphere intercepts over every target of the manager (IntersectionSolver::earliestIntersections): sphere j = t1[j],
+ * origin[j][3], radius[j].  hits_out[j] = the number of targets whose time (target_isolver_query_batch's delta, bit for bit) is >= 0;
+ * rows 0 .. min(k, hits_out[j]) - 1 of ids_out[j][k] / delta_out[j][k] are those targets by (delta, id), the other rows id 0xFFFFFFFF
+ * and delta -1.  Read-only: no solver stream is touched.  0 <= k <= 65536 (k == 0: counts only, ids_out / delta_out may be NULL); the
+ * arrays may be NULL only when q == 0.  The intercept pose of a returned target is target_manager_get_estimates_batch(ids, t1 + delta).
+ * Returns the total number of hits, -1 on error. */
+long long target_isolver_earliest(const target_isolver_c* s, long long q, const double* t1, const double* origin, const double* radius, long long k,
+                                  unsigned int* ids_out, double* delta_out, long long* hits_out);
 /* host wall time of the last query by phase, ms: routing, stream moves between shards, the shards' device queries, results into
  * call order; returns 0, -1 on error */
 int target_isolver_last_timing(const target_isolver_c* s, double ms_out[4]);

@@ -238,6 +238,17 @@ int te_isolver_query(te_isolver* s, long long n, const uint32_t* ids, const int3
  * (isolver_unpack_streams_kernel).  Each solver's staging grows only when a move is larger than any before.  Synchronous. */
 int te_isolver_move_streams(te_isolver* src, te_isolver* dst, long long n, const int32_t* streams);
 
+/* The k earliest sphere intercepts over every target of the pool (read-only: no solver stream, filter or target state is touched).
+ * Sphere j = (t1[j], origin[j][3], radius[j]), host arrays.  For target i, delta_ij is bit for bit te_isolver_query's delta_t for
+ * (i, t1[j], origin[j], radius[j]); a hit is delta >= 0 (-0.0 is a hit and ranks as 0; -1 and NaN are not).  hits_out[j] = the
+ * number of hits; rows 0 .. min(k, hits_out[j]) - 1 of ids_out[j][.] / delta_out[j][.] are those hits ordered by (delta, id), delta
+ * as te_isolver_query returns it; the remaining rows are id 0xFFFFFFFF and delta -1.  0 <= k <= 65536; k == 0 gives the counts
+ * only (ids_out / delta_out may then be NULL).  The targets are swept on the device in chunks of spheres sized from the pool, the
+ * k-th key of every sphere is found by radix select, and only q x k rows cross to the host.  Uniform-velocity and angular-velocity
+ * pools never intercept (zero t^4 coefficient) and run no kernel.  Synchronous.  Returns the total number of hits. */
+long long te_pool_earliest_intersections(te_pool* p, long long q, const double* t1, const double* origin /*[q][3]*/, const double* radius,
+                                         long long k, uint32_t* ids_out /*[q][k]*/, double* delta_out /*[q][k]*/, long long* hits_out /*[q]*/);
+
 /* Dense device-resident form: one query per slot (query k = slot k = solver stream k; needs n_streams >= pool size).
  * dev_t1 NULL = each target's own time; dev_delta / dev_pose7 / dev_converged may be NULL.  Asynchronous. */
 int te_isolver_query_dense(te_isolver* s, const double* dev_t1, const double* dev_origin /*[size][3]*/, const double* dev_radius,

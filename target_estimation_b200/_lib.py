@@ -77,6 +77,7 @@ SIGNATURES = {
     "te_isolver_destroy": (None, [_p]),
     "te_isolver_query": (_i, [_p, _ll, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p]),
     "te_isolver_query_dense": (_i, [_p, _p, _p, _p, _d, _d, _p, _p, _p]),
+    "te_pool_earliest_intersections": (_ll, [_p, _ll, _p, _p, _p, _ll, _p, _p, _p]),
     "te_isolver_move_streams": (_i, [_p, _p, _ll, _p]),
     "te_pool_tick_host_async": (_i, [_p, _d, _p, _i, _p, _i, _p]),
     "te_pool_tick_host_wait": (_i, [_p, _i]),

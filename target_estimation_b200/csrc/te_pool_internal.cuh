@@ -4,6 +4,7 @@
 //   te_step.cu     step-kernel launch policy and the stepping entry points (dense / replay / host / by id / fused expiry)
 //   te_mailbox.cu  device-resident mailboxes (the node loop)
 //   te_isolver.cu  batched IntersectionSolver
+//   te_sweep.cu    the k earliest sphere intercepts over every target of a pool (te_pool_earliest_intersections)
 //   te_group.cu    several pools on several devices: the NCCL all-gather of estimate records
 #pragma once
 #include <algorithm>

@@ -1,0 +1,122 @@
+// te_sweep.cu -- te_pool_earliest_intersections of include/te_pool.h: the k earliest sphere intercepts over every target of a pool,
+// selected on the device (kernels in te_sweep.cuh).  Only q x k rows and q hit counts cross PCIe.
+#include <cub/device/device_segmented_sort.cuh>
+
+#include "te_pool_internal.cuh"
+#include "te_sweep.cuh"
+
+using namespace tehost;
+
+namespace {
+// keys of one chunk: at most this many (sphere, target) pairs, 256 MB
+constexpr long long SWEEP_PAIRS = 1LL << 25;
+
+// delta of every slot for one sphere into keys (as doubles): the kernel and arguments of te_isolver_query_dense, so every bit is
+// te_isolver_query's
+template <int TYPE>
+void launch_deltas(te_pool* p, int n, const double* t1, const double* origin, const double* radius, unsigned long long* keys) {
+  te::isolver_kernel<TYPE><<<cdiv(n, 128), 128, 0, p->stream>>>(p->buf[p->cur].tiles, nullptr, nullptr, n, t1, origin, radius, nullptr, nullptr,
+                                                                 te::IsolverState{}, reinterpret_cast<double*>(keys), nullptr, nullptr);
+}
+}  // namespace
+
+extern "C" long long te_pool_earliest_intersections(te_pool* p, long long q, const double* t1, const double* origin, const double* radius,
+                                                    long long k, uint32_t* ids_out, double* delta_out, long long* hits_out) {
+  return guarded_ll(p, [&]() -> long long {
+    if (q < 0) throw std::invalid_argument("q must be >= 0");
+    if (k < 0 || k > 65536) throw std::invalid_argument("k must be in [0, 65536]");
+    if (q == 0) return 0;
+    if (!t1 || !origin || !radius || !hits_out) throw std::invalid_argument("t1, origin, radius and hits_out are required");
+    if (k > 0 && (!ids_out || !delta_out)) throw std::invalid_argument("ids_out and delta_out are required when k > 0");
+    const long long n = p->n;
+    // uniform-velocity and angular-velocity targets carry no acceleration: the t^4 coefficient is 0 and no target intercepts
+    if (n == 0 || p->model == te::UNIFORM_VELOCITY || p->model == te::ANGULAR_VELOCITIES) {
+      std::fill(hits_out, hits_out + q, 0LL);
+      if (k > 0) {
+        std::fill(ids_out, ids_out + q * k, 0xFFFFFFFFu);
+        std::fill(delta_out, delta_out + q * k, -1.0);
+      }
+      return 0;
+    }
+    const int C = (int)std::max(1LL, std::min({q, (long long)te::SWEEP_MAX_CHUNK, SWEEP_PAIRS / n}));
+    const unsigned cap = (unsigned)k + te::SWEEP_SLACK;
+    std::vector<double> sph((size_t)q * 5);   // t1, origin, radius of sphere j as one record
+    for (long long j = 0; j < q; ++j) {
+      sph[5 * j] = t1[j];
+      std::memcpy(&sph[5 * j + 1], origin + 3 * j, 24);
+      sph[5 * j + 4] = radius[j];
+    }
+    const double* d_sph = to_dev(p, sph.data(), sph.size());
+    double* b_t1 = p->arena.get_n<double>((size_t)n * 5);   // one sphere broadcast to every slot: isolver_kernel's inputs
+    double* b_origin = b_t1 + n;
+    double* b_radius = b_t1 + 4 * n;
+    auto* keys = p->arena.get_n<unsigned long long>((size_t)C * n);
+    auto* hits = p->arena.get_n<unsigned long long>(C);
+    auto* sel = p->arena.get_n<te::SweepSel>(C);
+    auto* hist = p->arena.get_n<unsigned>((size_t)C * te::SWEEP_BINS);
+    auto* count = p->arena.get_n<unsigned>(C);
+    int* seg = p->arena.get_n<int>(2 * (size_t)C + 1);   // begin offsets | end offsets | overflow flag
+    int* overflow = seg + 2 * C;
+    unsigned long long *rank_a = nullptr, *rank_b = nullptr;
+    unsigned *slot_a = nullptr, *slot_b = nullptr;
+    uint32_t* d_ids = nullptr;
+    double* d_delta = nullptr;
+    void* sort_tmp = nullptr;
+    size_t sort_bytes = 0;
+    const int items = C * (int)cap;
+    if (k > 0) {
+      rank_a = p->arena.get_n<unsigned long long>(items);
+      rank_b = p->arena.get_n<unsigned long long>(items);
+      slot_a = p->arena.get_n<unsigned>(items);
+      slot_b = p->arena.get_n<unsigned>(items);
+      d_ids = p->arena.get_n<uint32_t>((size_t)C * k);
+      d_delta = p->arena.get_n<double>((size_t)C * k);
+      size_t by_slot = 0, by_rank = 0;
+      CK(cub::DeviceSegmentedSort::StableSortPairs(nullptr, by_slot, slot_a, slot_b, rank_a, rank_b, items, C, seg, seg + C, p->stream));
+      CK(cub::DeviceSegmentedSort::StableSortPairs(nullptr, by_rank, rank_a, rank_b, slot_a, slot_b, items, C, seg, seg + C, p->stream));
+      sort_bytes = std::max(by_slot, by_rank);
+      sort_tmp = p->arena.get(sort_bytes);
+    }
+    CK(cudaMemsetAsync(hist, 0, (size_t)C * te::SWEEP_BINS * sizeof(unsigned), p->stream));
+    CK(cudaMemsetAsync(overflow, 0, sizeof(int), p->stream));
+    const int bx = std::max(1, std::min(cdiv(n, 256 * 4), (p->n_sm * 8 + C - 1) / C));
+    for (long long j0 = 0; j0 < q; j0 += C) {
+      const int nq = (int)std::min<long long>(C, q - j0);
+      CK(cudaMemsetAsync(hits, 0, (size_t)nq * sizeof(unsigned long long), p->stream));
+      for (int c = 0; c < nq; ++c) {
+        unsigned long long* kc = keys + (size_t)c * n;
+        te::sweep_broadcast_kernel<<<cdiv(n, 256), 256, 0, p->stream>>>((int)n, d_sph + 5 * (j0 + c), b_t1, b_origin, b_radius);
+        if (p->model == te::UNIFORM_ACCELERATION) launch_deltas<te::UNIFORM_ACCELERATION>(p, (int)n, b_t1, b_origin, b_radius, kc);
+        else launch_deltas<te::ANGULAR_RATES>(p, (int)n, b_t1, b_origin, b_radius, kc);
+        te::sweep_key_kernel<<<cdiv(n, 256), 256, 0, p->stream>>>((int)n, kc, hits + c);
+      }
+      CK(cudaGetLastError());
+      if (k > 0) {
+        te::sweep_init_kernel<<<1, te::SWEEP_MAX_CHUNK, 0, p->stream>>>(nq, (unsigned)k, hits, sel, count);
+        for (int pass = 0; pass < te::SWEEP_PASSES; ++pass) {
+          te::sweep_hist_kernel<<<dim3(bx, nq), 256, 0, p->stream>>>(keys, (int)n, sel, te::sweep_shift(pass), hist);
+          te::sweep_select_kernel<<<nq, 1024, 0, p->stream>>>(hist, sel, te::sweep_shift(pass));
+        }
+        te::sweep_collect_kernel<<<dim3(bx, nq), 256, 0, p->stream>>>(keys, (int)n, sel, cap, count, rank_a, slot_a);
+        te::sweep_segments_kernel<<<1, te::SWEEP_MAX_CHUNK, 0, p->stream>>>(nq, cap, count, seg, seg + C, overflow);
+        CK(cudaGetLastError());
+        // (slot, then stable by rank: ties of delta come out in ascending slot = ascending id)
+        CK(cub::DeviceSegmentedSort::StableSortPairs(sort_tmp, sort_bytes, slot_a, slot_b, rank_a, rank_b, nq * (int)cap, nq, seg, seg + C, p->stream));
+        CK(cub::DeviceSegmentedSort::StableSortPairs(sort_tmp, sort_bytes, rank_b, rank_a, slot_b, slot_a, nq * (int)cap, nq, seg, seg + C, p->stream));
+        te::sweep_output_kernel<<<dim3(cdiv(k, 256), nq), 256, 0, p->stream>>>((int)k, sel, slot_a, cap, keys, (int)n, p->buf[p->cur].cold.ids,
+                                                                                d_ids, d_delta);
+        CK(cudaGetLastError());
+        CK(cudaMemcpyAsync(ids_out + j0 * k, d_ids, (size_t)nq * k * sizeof(uint32_t), cudaMemcpyDeviceToHost, p->stream));
+        CK(cudaMemcpyAsync(delta_out + j0 * k, d_delta, (size_t)nq * k * sizeof(double), cudaMemcpyDeviceToHost, p->stream));
+      }
+      CK(cudaMemcpyAsync(hits_out + j0, hits, (size_t)nq * sizeof(long long), cudaMemcpyDeviceToHost, p->stream));
+    }
+    int h_overflow = 0;
+    CK(cudaMemcpyAsync(&h_overflow, overflow, sizeof(int), cudaMemcpyDeviceToHost, p->stream));
+    CK(cudaStreamSynchronize(p->stream));
+    if (h_overflow) throw std::logic_error("te_pool_earliest_intersections: candidate overflow (selection invariant broken)");
+    long long total = 0;
+    for (long long j = 0; j < q; ++j) total += hits_out[j];
+    return total;
+  });
+}

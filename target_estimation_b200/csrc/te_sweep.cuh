@@ -1,0 +1,218 @@
+// te_sweep.cuh -- sm_100a kernels of te_pool_earliest_intersections (te_sweep.cu): for each of a chunk of spheres, the k targets of
+// the pool with the smallest intercept time, selected on the device without sorting the pool.
+//   keys            per sphere, isolver_kernel's delta of every slot (see sweep_broadcast_kernel) becomes a 64-bit key: the bits
+//                   of delta for a hit, ~0 otherwise; hits are counted
+//   hist / select   radix select over the 96-bit composite (rank(key), slot) in eight 12-bit digits: one histogram of the keys that
+//                   still match the selected prefix, then the digit bucket that holds the k-th; refinement stops as soon as that
+//                   bucket is small (usually after the second digit)
+//   collect         every key at or below the boundary bucket: at most k - 1 + SWEEP_SLACK candidates per sphere
+//   output          after a stable sort of the candidates by slot, then by rank (cub::DeviceSegmentedSort): rows of (id, delta)
+// A hit's key orders like its delta (a non-negative double's bits order like the value); rank() maps -0.0 to 0, so -0.0 ranks as 0
+// while the key keeps the bits that query() returns.  Slots are in ascending-id order, so (rank, slot) order is (delta, id) order.
+#pragma once
+#include <cub/block/block_scan.cuh>
+
+#include "te_kernels.cuh"
+
+namespace te {
+
+constexpr int SWEEP_MAX_CHUNK = 32;     // spheres per chunk (the y dimension of the selection kernels' grids)
+constexpr int SWEEP_BINS = 4096;        // 12-bit digits
+constexpr int SWEEP_PASSES = 8;         // 96 bits = 64-bit key + 32-bit slot: (rank, slot) is unique, so 8 digits always resolve
+constexpr unsigned SWEEP_SLACK = 2048;  // a boundary bucket of at most this many keys is collected whole
+constexpr unsigned long long SWEEP_MISS = ~0ull;
+
+__host__ __device__ inline int sweep_shift(int pass) { return 84 - 12 * pass; }   // lowest bit of digit `pass` in the 96-bit composite
+__device__ __forceinline__ unsigned long long sweep_rank(unsigned long long key) { return key == 0x8000000000000000ull ? 0ull : key; }
+
+// the selected prefix of the composite (rank, slot): a composite matches when (rank & mk) == pk and (slot & ms) == ps
+struct SweepSel {
+  unsigned long long pk, mk;
+  unsigned ps, ms;
+  unsigned kk;     // rank still to place inside the boundary bucket (1-based)
+  unsigned take;   // rows to return: min(k, hits)
+  int done;
+};
+
+__device__ __forceinline__ unsigned sweep_digit(unsigned long long r, unsigned s, int sh) {
+  if (sh >= 32) return (unsigned)(r >> (sh - 32)) & (SWEEP_BINS - 1);
+  if (sh + 12 <= 32) return (s >> sh) & (SWEEP_BINS - 1);
+  return (unsigned)((r << (32 - sh)) | (unsigned long long)(s >> sh)) & (SWEEP_BINS - 1);
+}
+
+__device__ __forceinline__ void sweep_set_digit(SweepSel& S, unsigned b, int sh) {
+  if (sh >= 32) {
+    S.pk |= (unsigned long long)b << (sh - 32);
+    S.mk |= (unsigned long long)(SWEEP_BINS - 1) << (sh - 32);
+  } else if (sh + 12 <= 32) {
+    S.ps |= b << sh;
+    S.ms |= (unsigned)(SWEEP_BINS - 1) << sh;
+  } else {   // the digit straddles the key's low bits and the slot's high bits
+    const int lo = 32 - sh;
+    S.pk |= b >> lo;
+    S.mk |= (1ull << (12 - lo)) - 1;
+    S.ps |= (b & ((1u << lo) - 1)) << sh;
+    S.ms |= ((1u << lo) - 1) << sh;
+  }
+}
+
+// isolver_kernel (dense form: query = slot) computes every target's delta for one sphere; these two kernels feed it and read it.
+// The sweep runs the very kernel te_isolver_query runs rather than a second copy of derive_outputs + the quartic: nvcc leaves most FP64
+// multiplies and adds unrounded in PTX and ptxas contracts them into FMAs according to the surrounding code, so a copy inlined into
+// another kernel gives other bits (measured on angular-rates pools: about half of the deltas differed in the last bits).
+static __global__ void sweep_broadcast_kernel(int n, const double* __restrict__ sphere /*t1, x, y, z, radius*/, double* __restrict__ t1,
+                                              double* __restrict__ origin, double* __restrict__ radius) {
+  const int s = blockIdx.x * blockDim.x + threadIdx.x;
+  if (s >= n) return;
+  t1[s] = sphere[0];
+  origin[3 * s] = sphere[1];
+  origin[3 * s + 1] = sphere[2];
+  origin[3 * s + 2] = sphere[3];
+  radius[s] = sphere[4];
+}
+
+// delta (written by isolver_kernel in place) -> key: the bits of delta for a hit (delta >= 0), SWEEP_MISS otherwise; hits counted
+static __global__ void sweep_key_kernel(int n, unsigned long long* __restrict__ keys, unsigned long long* __restrict__ hits) {
+  const int s = blockIdx.x * blockDim.x + threadIdx.x;
+  bool hit = false;
+  if (s < n) {
+    const double d = __longlong_as_double((long long)keys[s]);
+    hit = d >= 0.0;
+    if (!hit) keys[s] = SWEEP_MISS;
+  }
+  const unsigned b = __ballot_sync(0xffffffffu, hit);
+  if ((threadIdx.x & 31) == 0 && b) atomicAdd(hits, (unsigned long long)__popc(b));
+}
+
+// per sphere: rows to return and the state of the selection.  Nothing to select when every hit is returned (hits <= k: the empty
+// prefix matches them all) or none is.
+static __global__ void sweep_init_kernel(int nq, unsigned k, const unsigned long long* __restrict__ hits, SweepSel* __restrict__ sel,
+                                         unsigned* __restrict__ count) {
+  const int c = blockIdx.x * blockDim.x + threadIdx.x;
+  if (c >= nq) return;
+  const unsigned long long h = hits[c];
+  const unsigned take = h < k ? (unsigned)h : k;
+  sel[c] = SweepSel{0ull, 0ull, 0u, 0u, take, take, (take == 0 || h <= k) ? 1 : 0};
+  count[c] = 0;
+}
+
+// histogram of digit `sh` over the hits of sphere blockIdx.y that match the selected prefix
+static __global__ void __launch_bounds__(256) sweep_hist_kernel(const unsigned long long* __restrict__ keys, int n,
+                                                                const SweepSel* __restrict__ sel, int sh, unsigned* __restrict__ hist) {
+  const int c = blockIdx.y;
+  const SweepSel S = sel[c];
+  if (S.done) return;
+  __shared__ unsigned h[SWEEP_BINS];
+  for (int i = threadIdx.x; i < SWEEP_BINS; i += blockDim.x) h[i] = 0;
+  __syncthreads();
+  const unsigned long long* kc = keys + (size_t)c * n;
+  const int lane = threadIdx.x & 31;
+  for (long long base = (long long)blockIdx.x * blockDim.x; base < n; base += (long long)gridDim.x * blockDim.x) {   // uniform trip count
+    const int s = (int)base + threadIdx.x;
+    const unsigned long long key = s < n ? kc[s] : SWEEP_MISS;
+    const unsigned long long r = sweep_rank(key);
+    const bool m = key != SWEEP_MISS && (r & S.mk) == S.pk && ((unsigned)s & S.ms) == S.ps;
+    const unsigned act = __ballot_sync(0xffffffffu, m);
+    if (m) {   // one shared atomic per distinct digit of the warp: the first digits of the keys are few
+      const unsigned dg = sweep_digit(r, (unsigned)s, sh);
+      const unsigned peers = __match_any_sync(act, dg);
+      if (lane == __ffs(peers) - 1) atomicAdd(&h[dg], (unsigned)__popc(peers));
+    }
+  }
+  __syncthreads();
+  unsigned* hc = hist + (size_t)c * SWEEP_BINS;
+  for (int i = threadIdx.x; i < SWEEP_BINS; i += blockDim.x)
+    if (h[i]) atomicAdd(&hc[i], h[i]);
+}
+
+// the digit bucket of sphere blockIdx.x that holds its kk-th matching key; the histogram is left zeroed for the next digit
+static __global__ void __launch_bounds__(1024) sweep_select_kernel(unsigned* __restrict__ hist, SweepSel* __restrict__ sel, int sh) {
+  const int c = blockIdx.x;
+  if (sel[c].done) return;
+  const unsigned kk = sel[c].kk;
+  unsigned* hc = hist + (size_t)c * SWEEP_BINS;
+  const int b0 = 4 * threadIdx.x;
+  unsigned v[4], sum = 0;
+#pragma unroll
+  for (int j = 0; j < 4; ++j) { v[j] = hc[b0 + j]; sum += v[j]; }
+  typedef cub::BlockScan<unsigned, 1024> Scan;
+  __shared__ typename Scan::TempStorage tmp;
+  unsigned pre;
+  Scan(tmp).ExclusiveSum(sum, pre);   // (its barrier orders every thread's read of sel[c] before the one write below)
+  if (pre < kk && kk <= pre + sum) {
+    unsigned acc = pre;
+#pragma unroll
+    for (int j = 0; j < 4; ++j) {
+      if (kk <= acc + v[j]) {
+        SweepSel S = sel[c];
+        sweep_set_digit(S, (unsigned)(b0 + j), sh);
+        S.kk = kk - acc;
+        S.done = (v[j] <= SWEEP_SLACK || v[j] == S.kk) ? 1 : 0;   // small enough, or taken whole
+        sel[c] = S;
+        break;
+      }
+      acc += v[j];
+    }
+  }
+#pragma unroll
+  for (int j = 0; j < 4; ++j) hc[b0 + j] = 0;
+}
+
+// the candidates of sphere blockIdx.y: every hit whose composite is at or below the boundary bucket, at [c * cap, c * cap + count[c])
+static __global__ void __launch_bounds__(256) sweep_collect_kernel(const unsigned long long* __restrict__ keys, int n,
+                                                                   const SweepSel* __restrict__ sel, unsigned cap,
+                                                                   unsigned* __restrict__ count, unsigned long long* __restrict__ cand_rank,
+                                                                   unsigned* __restrict__ cand_slot) {
+  const int c = blockIdx.y;
+  const SweepSel S = sel[c];
+  if (S.take == 0) return;
+  const unsigned long long* kc = keys + (size_t)c * n;
+  const int lane = threadIdx.x & 31;
+  for (long long base = (long long)blockIdx.x * blockDim.x; base < n; base += (long long)gridDim.x * blockDim.x) {
+    const int s = (int)base + threadIdx.x;
+    const unsigned long long key = s < n ? kc[s] : SWEEP_MISS;
+    const unsigned long long r = sweep_rank(key), rm = r & S.mk;
+    const unsigned sm = (unsigned)s & S.ms;
+    const bool m = key != SWEEP_MISS && (rm < S.pk || (rm == S.pk && sm <= S.ps));
+    const unsigned b = __ballot_sync(0xffffffffu, m);
+    if (!b) continue;
+    unsigned at = 0;
+    if (lane == 0) at = atomicAdd(&count[c], (unsigned)__popc(b));
+    at = __shfl_sync(0xffffffffu, at, 0) + __popc(b & ((1u << lane) - 1));
+    if (m && at < cap) {
+      cand_rank[(size_t)c * cap + at] = r;
+      cand_slot[(size_t)c * cap + at] = (unsigned)s;
+    }
+  }
+}
+
+// segment c of the sort = sphere c's candidates; more than cap would mean a broken selection: flagged, never read past
+static __global__ void sweep_segments_kernel(int nq, unsigned cap, const unsigned* __restrict__ count, int* __restrict__ seg_begin,
+                                             int* __restrict__ seg_end, int* __restrict__ overflow) {
+  const int c = blockIdx.x * blockDim.x + threadIdx.x;
+  if (c >= nq) return;
+  seg_begin[c] = (int)(c * cap);
+  seg_end[c] = (int)(c * cap + (count[c] < cap ? count[c] : cap));
+  if (count[c] > cap) *overflow = 1;
+}
+
+// rows of sphere blockIdx.y: the first `take` sorted candidates (id through the pool's cold ids, delta as the sweep computed it), then
+// the sentinel rows
+static __global__ void sweep_output_kernel(int k, const SweepSel* __restrict__ sel, const unsigned* __restrict__ slot_sorted, unsigned cap,
+                                           const unsigned long long* __restrict__ keys, int n, const uint32_t* __restrict__ ids,
+                                           uint32_t* __restrict__ ids_out, double* __restrict__ delta_out) {
+  const int c = blockIdx.y;
+  const int r = blockIdx.x * blockDim.x + threadIdx.x;
+  if (r >= k) return;
+  const size_t o = (size_t)c * k + r;
+  if ((unsigned)r < sel[c].take) {
+    const unsigned s = slot_sorted[(size_t)c * cap + r];
+    ids_out[o] = ids[s];
+    delta_out[o] = __longlong_as_double((long long)keys[(size_t)c * n + s]);
+  } else {
+    ids_out[o] = 0xFFFFFFFFu;
+    delta_out[o] = -1.0;
+  }
+}
+
+}  // namespace te

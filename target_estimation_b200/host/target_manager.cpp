@@ -1146,6 +1146,94 @@ long long IntersectionSolver::queryRun(long long n, const unsigned* ids, const i
   return found;
 }
 
+long long IntersectionSolver::earliestIntersections(long long q, const double* t1, const double* origin, const double* radius, long long k,
+                                                    unsigned* ids_out, double* delta_out, long long* hits_out) {
+  if (q < 0) throw std::invalid_argument("q must be >= 0");
+  if (k < 0 || k > 65536) throw std::invalid_argument("k must be in [0, 65536]");
+  if (q > 0 && (!t1 || !origin || !radius || !hits_out)) throw std::invalid_argument("t1, origin, radius and hits_out are required");
+  if (q > 0 && k > 0 && (!ids_out || !delta_out)) throw std::invalid_argument("ids_out and delta_out are required when k > 0");
+  std::lock_guard<std::recursive_mutex> lg(target_manager_->lock());
+  if (q == 0) return 0;
+  target_manager_->flush();
+  const int G = (int)solvers_.size();
+  if (sweep_.empty()) sweep_.resize(4 * (size_t)G);
+  int n_lists = 0, only = -1;
+  for (int r = 0; r < G; ++r)
+    for (int t = 0; t < 4; ++t) {
+      te_pool* p = shardOf(r).poolOf(t, false);
+      SweepList& L = sweep_[(size_t)r * 4 + (size_t)t];
+      L.used = p && te_pool_size(p) > 0;
+      if (L.used) { ++n_lists; only = r * 4 + t; }
+    }
+  auto run = [&](int r, int t, unsigned* ids, double* delta, long long* hits) {
+    TargetManager& M = shardOf(r);
+    std::lock_guard<std::recursive_mutex> lk(M.lock());
+    ck(te_pool_earliest_intersections(M.poolOf(t, false), q, t1, origin, radius, k, ids, delta, hits));
+  };
+  if (n_lists == 1) {   // one pool holds every target: its rows are the answer
+    run(only / 4, only % 4, ids_out, delta_out, hits_out);
+  } else {
+    auto run_shard = [&](int r) {
+      for (int t = 0; t < 4; ++t) {
+        SweepList& L = sweep_[(size_t)r * 4 + (size_t)t];
+        if (!L.used) continue;
+        L.ids.resize((size_t)(q * k)); L.delta.resize((size_t)(q * k)); L.hits.resize((size_t)q);
+        run(r, t, L.ids.data(), L.delta.data(), L.hits.data());
+      }
+    };
+    // merge sphere j's sorted lists by (rank(delta), id): -0.0 ranks as 0, a non-negative double's bits order like its value
+    auto rank = [](double d) {
+      unsigned long long b;
+      std::memcpy(&b, &d, 8);
+      return b == 0x8000000000000000ull ? 0ull : b;
+    };
+    std::vector<const SweepList*> used;
+    for (const SweepList& L : sweep_)
+      if (L.used) used.push_back(&L);
+    auto merge = [&](long long j, std::vector<long long>& at) {
+      long long hits = 0;
+      for (const SweepList* L : used) hits += L->hits[(size_t)j];
+      hits_out[j] = hits;
+      at.assign(used.size(), 0);
+      for (long long row = 0; row < k; ++row) {
+        int best = -1;
+        unsigned long long best_rank = 0;
+        unsigned best_id = 0;
+        for (size_t l = 0; l < used.size(); ++l) {
+          const SweepList& L = *used[l];
+          if (at[l] >= std::min(k, L.hits[(size_t)j])) continue;
+          const size_t o = (size_t)(j * k + at[l]);
+          const unsigned long long rk = rank(L.delta[o]);
+          if (best < 0 || rk < best_rank || (rk == best_rank && L.ids[o] < best_id)) { best = (int)l; best_rank = rk; best_id = L.ids[o]; }
+        }
+        const size_t out = (size_t)(j * k + row);
+        if (best < 0) {
+          ids_out[out] = 0xFFFFFFFFu;
+          delta_out[out] = -1.0;
+        } else {
+          const size_t o = (size_t)(j * k + at[(size_t)best]++);
+          ids_out[out] = used[(size_t)best]->ids[o];
+          delta_out[out] = used[(size_t)best]->delta[o];
+        }
+      }
+    };
+    if (sharded_) {   // every shard's pools at once, then the spheres' merges spread over the shards' workers
+      sharded_->forEachShard(run_shard);
+      sharded_->forEachShard([&](int r) {
+        std::vector<long long> at;
+        for (long long j = r; j < q; j += G) merge(j, at);
+      });
+    } else {
+      run_shard(0);
+      std::vector<long long> at;
+      for (long long j = 0; j < q; ++j) merge(j, at);
+    }
+  }
+  long long total = 0;
+  for (long long j = 0; j < q; ++j) total += hits_out[j];
+  return total;
+}
+
 // ----------------------------------------------------------------------------------------------
 // utils.hpp:273-313
 // ----------------------------------------------------------------------------------------------

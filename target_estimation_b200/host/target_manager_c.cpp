@@ -217,6 +217,10 @@ long long target_isolver_query_batch(const target_isolver_c* s, long long n, con
                                      double* delta_out, double* pose7_out, unsigned char* converged_out) {
   return guard(-1LL, [&] { return S(s)->query(n, ids, stream, t1, origin, radius, pos_th, ang_th, delta_out, pose7_out, converged_out); });
 }
+long long target_isolver_earliest(const target_isolver_c* s, long long q, const double* t1, const double* origin, const double* radius, long long k,
+                                  unsigned int* ids_out, double* delta_out, long long* hits_out) {
+  return guard(-1LL, [&] { return S(s)->earliestIntersections(q, t1, origin, radius, k, ids_out, delta_out, hits_out); });
+}
 int target_isolver_last_timing(const target_isolver_c* s, double ms_out[4]) {
   return guard(-1, [&] {
     if (!ms_out) throw std::invalid_argument("ms_out is required");

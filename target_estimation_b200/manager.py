@@ -66,6 +66,7 @@ _SIG = {
     "target_isolver_get_pose": (C.c_bool, [_p, _u, _d, _d, _d, _p, _d, _p]),
     "target_isolver_query_batch": (_ll, [_p, _ll, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p]),
     "target_isolver_last_timing": (_i, [_p, _p]),
+    "target_isolver_earliest": (_ll, [_p, _ll, _p, _p, _p, _ll, _p, _p, _p]),
 }
 for _n, (_r, _a) in _SIG.items():
     _f = getattr(clib, _n)
@@ -377,6 +378,21 @@ class IntersectionSolverC:
         if found < 0:
             raise RuntimeError(clib.target_manager_last_error().decode())
         return found, delta, pose, conv
+
+    def earliest(self, t1, origin, radius, k):
+        """the k earliest sphere intercepts over every target: sphere j = (t1[j], origin[j], radius[j]); t1 and radius broadcast to
+        q = len(origin).  Returns (hits [q], ids [q][k], delta [q][k]): rows past min(k, hits[j]) are id 0xFFFFFFFF and delta -1.
+        The intercept pose of a returned target is the manager's get_estimates_batch(ids, t1 + delta)."""
+        origin = np.ascontiguousarray(origin, dtype=np.float64).reshape(-1, 3)
+        q, k = origin.shape[0], int(k)
+        t1 = np.ascontiguousarray(np.broadcast_to(t1, (q,)), dtype=np.float64)
+        radius = np.ascontiguousarray(np.broadcast_to(radius, (q,)), dtype=np.float64)
+        hits = np.zeros(q, dtype=np.int64)
+        ids = np.zeros((q, max(k, 0)), dtype=np.uint32)
+        delta = np.zeros((q, max(k, 0)))
+        if int(clib.target_isolver_earliest(self.h, q, _ptr(t1), _ptr(origin), _ptr(radius), k, _ptr(ids), _ptr(delta), _ptr(hits))) < 0:
+            raise RuntimeError(clib.target_manager_last_error().decode())
+        return hits, ids, delta
 
     def last_timing(self):
         """ms of the last query by phase: routing, moves, device, results into call order"""

@@ -297,6 +297,20 @@ class TargetPool:
     def mailbox_count(self):
         return int(lib.te_pool_mailbox_count(self._h))
 
+    # -- the k earliest sphere intercepts over every target (te_pool_earliest_intersections) ------
+    def earliest_intersections(self, t1, origin, radius, k):
+        """sphere j = (t1[j], origin[j], radius[j]); t1 and radius broadcast to q = len(origin).  Returns (hits [q], ids [q][k],
+        delta [q][k]) with the hits of each sphere by (delta, id) first and rows of id 0xFFFFFFFF / delta -1 after them."""
+        origin = _np(origin, np.float64).reshape(-1, 3)
+        q, k = origin.shape[0], int(k)
+        t1 = _np(np.broadcast_to(t1, (q,)), np.float64)
+        radius = _np(np.broadcast_to(radius, (q,)), np.float64)
+        hits = np.zeros(q, dtype=np.int64)
+        ids = np.zeros((q, max(k, 0)), dtype=np.uint32)
+        delta = np.zeros((q, max(k, 0)))
+        check(lib.te_pool_earliest_intersections(self._h, q, _ptr(t1), _ptr(origin), _ptr(radius), k, _ptr(ids), _ptr(delta), _ptr(hits)))
+        return hits, ids, delta
+
 
 class IntersectionSolver:
     """Batched IntersectionSolver: n_streams independent reference solver objects (include/te_pool.h)."""
