@@ -46,6 +46,29 @@ typedef std::vector<double> VectorXd;
 
 class TargetManager;
 
+// The k smallest (value, id) rows of q queries over every (shard, model type) pool that holds targets: what
+// IntersectionSolver::earliestIntersections and TargetManager::nearestTargets share.  Each pool selects its own rows on the device
+// (te_pool_earliest_intersections / te_pool_nearest_targets: per query, rows by (value, id), then id 0xFFFFFFFF / value -1, and
+// a count); the host merges the lists of each query by (value, id) -- a candidate's value is a non-negative double, -0.0 ranks as
+// 0 -- and sums the counts.  When one pool holds every target its rows are the answer.  The lists' buffers only grow.
+class PoolRowMerge {
+ public:
+  // one pool's rows [q][k] and counts [q]: returns < 0 on error (te_last_error())
+  typedef std::function<long long(te_pool*, unsigned* ids, double* val, long long* count)> PoolQuery;
+  // each_shard(f) runs f(r) for every r < shards.size(), possibly at once; pool calls hold the shard's lock.  Returns the total count.
+  long long run(const std::vector<TargetManager*>& shards, const std::function<void(const std::function<void(int)>&)>& each_shard,
+                long long q, long long k, const PoolQuery& query, unsigned* ids_out, double* val_out, long long* count_out);
+
+ private:
+  struct List {   // the sorted rows of one (shard, model type) pool
+    std::vector<unsigned> ids;
+    std::vector<double> val;
+    std::vector<long long> count;
+    bool used = false;
+  };
+  std::vector<List> lists_;   // [shard * 4 + model type]
+};
+
 // id -> model type, ascending ids: the host registry behind getAvailableTargets / "already exists" / "does not exist".  The
 // reference's std::map<unsigned, TargetInterface::Ptr> (target_manager.hpp:36) node-per-target layout costs a cache miss per
 // tree level: erasing the 10 k ids that expire in one tick of a million-target pool took 10 ms.  A sorted flat vector keeps the
@@ -161,6 +184,16 @@ class TargetManager {
   virtual void getEstimatesBatch(long long n, const unsigned* ids, const double* t1, double* pose7, double* twist6, double* acc6,
                                  unsigned char* found);
   virtual void flush();
+  // The k nearest targets inside a sphere at a given time, over every target of the manager (te_pool_nearest_targets on every
+  // (shard, model type) pool that holds targets; the shards of a sharded manager run at once).  Query j = (t1[j], point[j][3],
+  // radius[j]), t1 NULL = every target's current estimate.  The position of target i is pose7[0:3] of getEstimatesBatch({i}, {t1[j]})
+  // bit for bit; dist = sqrt((dx^2 + dy^2) + dz^2), every operation rounded on its own; inside = dist <= radius[j].  count_out[j] =
+  // the number of targets inside; rows 0 .. min(k, count) - 1 of ids_out[j][.] / dist_out[j][.] are those targets by (dist, id),
+  // the other rows id 0xFFFFFFFF and dist -1.  The result does not depend on the shard count or on which pool holds a target.
+  // Read-only; queued per-id calls are flushed first.  0 <= k <= 65536 (k == 0: counts only, ids_out / dist_out may be NULL); a
+  // negative or NaN radius is an error, +inf asks for the k nearest of all.  Returns the total count.
+  virtual long long nearestTargets(long long q, const double* t1 /*[q] or NULL*/, const double* point /*[q][3]*/, const double* radius,
+                                   long long k, unsigned* ids_out /*[q][k]*/, double* dist_out /*[q][k]*/, long long* count_out /*[q]*/);
   // One dense tick from host arrays, record k = the k-th target in denseIds() order (a homogeneous manager: getAvailableTargets()
   // order): no ids travel, nothing is looked up -- te_pool_tick_host: the copies, the step and the read-back of every target's
   // estimated position (est_pos_out [n][3], may be NULL: what the node broadcasts per tick, src/target_manager_ros.cpp:78-87) are
@@ -205,6 +238,7 @@ class TargetManager {
   void queue(int type, unsigned id, double dt, const double* meas, int action);
   long long updateBatchUnique(long long n, const unsigned* ids, double dt, const double* meas, const unsigned char* action);   // no id twice
   te_pool* densePool();   // the one non-empty pool of a homogeneous manager (throws otherwise)
+  PoolRowMerge nearest_rows_;
 
   int device_;
   te_pool* pools_[4] = {nullptr, nullptr, nullptr, nullptr};
@@ -314,13 +348,7 @@ class IntersectionSolver {
   std::vector<Part> part_;
   std::vector<unsigned> seen_;                        // repeat detection: seen_[stream] == gen_ within the current piece
   unsigned gen_ = 0;
-  struct SweepList {   // earliestIntersections: the sorted rows of one (shard, model type) pool (grow-only)
-    std::vector<unsigned> ids;
-    std::vector<double> delta;
-    std::vector<long long> hits;
-    bool used = false;
-  };
-  std::vector<SweepList> sweep_;                      // [shard * 4 + model type]
+  PoolRowMerge sweep_;                                // earliestIntersections
   double phase_ms_[4] = {0, 0, 0, 0};
 };
 
@@ -493,6 +521,8 @@ class ShardedTargetManager : public TargetManager {
   void getEstimatesBatch(long long n, const unsigned* ids, const double* t1, double* pose7, double* twist6, double* acc6,
                          unsigned char* found) override;
   void flush() override;
+  long long nearestTargets(long long q, const double* t1, const double* point, const double* radius, long long k, unsigned* ids_out,
+                           double* dist_out, long long* count_out) override;   // every shard at once
   // dense ticks: the records are SHARD-MAJOR (denseIds(): shard 0's targets in ascending id, then shard 1's, ...); every shard's
   // slice is copied, stepped and read back by its own worker thread on its own device
   long long updateDense(double dt, const double* meas, int meas_stride, const unsigned char* action, double* est_pos_out) override;

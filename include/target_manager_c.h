@@ -77,6 +77,16 @@ long long target_manager_get_ids(const target_manager_c* self, unsigned int* out
 int target_manager_get_state(const target_manager_c* self, unsigned int id, double* x, double* P, double* t);
 /* pending per-id calls are coalesced into one launch per tick; force them out */
 void target_manager_flush(const target_manager_c* self);
+/* The k nearest targets inside a sphere at a given time (TargetManager::nearestTargets), on every handle: plain, on a device,
+ * sharded, tick and sharded tick.  Query j = t1[j] (t1 NULL = current estimates), point[j][3], radius[j].  A target's position is
+ * pose7[0:3] of target_manager_get_estimates_batch at t1[j], bit for bit; dist = sqrt((dx^2 + dy^2) + dz^2), every operation rounded
+ * on its own; inside = dist <= radius[j].  count_out[j] = the number of targets inside; rows 0 .. min(k, count_out[j]) - 1 of
+ * ids_out[j][k] / dist_out[j][k] are those targets by (dist, id), the other rows id 0xFFFFFFFF and dist -1.  Read-only.  0 <= k <=
+ * 65536 (k == 0: counts only, ids_out / dist_out may be NULL); the arrays may be NULL only when q == 0; a negative or NaN radius is
+ * an error, +inf asks for the k nearest of all.  The pose of a returned target is target_manager_get_estimates_batch(ids, t1).
+ * Returns the total count, -1 on error. */
+long long target_manager_nearest(const target_manager_c* self, long long q, const double* t1, const double* point, const double* radius, long long k,
+                                 unsigned int* ids_out, double* dist_out, long long* count_out);
 
 /* ---- all GPUs of the box behind one handle (BASELINE.json north_star: targets shard by id, no collective on the hot path) ----
  * n_shards TargetManagers, shard r on CUDA device devices[r] (NULL = devices 0 .. n_shards-1), owner(id) = id mod n_shards.  The

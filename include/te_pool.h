@@ -248,6 +248,15 @@ int te_isolver_move_streams(te_isolver* src, te_isolver* dst, long long n, const
  * pools never intercept (zero t^4 coefficient) and run no kernel.  Synchronous.  Returns the total number of hits. */
 long long te_pool_earliest_intersections(te_pool* p, long long q, const double* t1, const double* origin /*[q][3]*/, const double* radius,
                                          long long k, uint32_t* ids_out /*[q][k]*/, double* delta_out /*[q][k]*/, long long* hits_out /*[q]*/);
+/* The k nearest targets inside a sphere, over every target of the pool (read-only).  Query j = (t1[j], point[j][3], radius[j]), host
+ * arrays; t1 NULL = every target's current estimate.  The position p_i of target i is pose7[0:3] of te_pool_read_estimates at t1[j]
+ * (t1 NULL: at none), bit for bit; dist_ij = sqrt_rn((dx^2 + dy^2) + dz^2) with d = p_i - point[j], every operation rounded on its
+ * own in that order (no FMA).  A target is inside when dist_ij <= radius[j] (the boundary counts, NaN never does).  count_out[j] =
+ * the number of targets inside; rows 0 .. min(k, count_out[j]) - 1 of ids_out[j][.] / dist_out[j][.] are those targets ordered by
+ * (dist, id), the remaining rows id 0xFFFFFFFF and dist -1.  Argument rules as te_pool_earliest_intersections; a negative or NaN
+ * radius is an error (radius = +inf: plain k nearest).  Every model type runs the kernels.  Synchronous.  Returns the total count. */
+long long te_pool_nearest_targets(te_pool* p, long long q, const double* t1 /*[q] or NULL*/, const double* point /*[q][3]*/, const double* radius,
+                                  long long k, uint32_t* ids_out /*[q][k]*/, double* dist_out /*[q][k]*/, long long* count_out /*[q]*/);
 
 /* Dense device-resident form: one query per slot (query k = slot k = solver stream k; needs n_streams >= pool size).
  * dev_t1 NULL = each target's own time; dev_delta / dev_pose7 / dev_converged may be NULL.  Asynchronous. */

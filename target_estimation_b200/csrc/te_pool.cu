@@ -382,6 +382,19 @@ void attach_mailboxes(te_pool* p, const uint32_t* ids, long long n) {
   CK(cudaStreamSynchronize(p->stream));   // the host vectors above go out of scope
 }
 
+void launch_gather_estimates(te_pool* p, const int* slots, long long n, const double* d_t1, double* pose, double* twist, double* acc,
+                             double* pose6, uint8_t* found, int rec13) {
+  Buf& b = p->buf[p->cur];
+  const int g = cdiv(n, 128);
+  switch (p->model) {
+    case te::UNIFORM_VELOCITY: te::gather_estimates_kernel<te::UNIFORM_VELOCITY><<<g, 128, 0, p->stream>>>(b.tiles, slots, n, d_t1, pose, twist, acc, pose6, found, rec13); break;
+    case te::UNIFORM_ACCELERATION: te::gather_estimates_kernel<te::UNIFORM_ACCELERATION><<<g, 128, 0, p->stream>>>(b.tiles, slots, n, d_t1, pose, twist, acc, pose6, found, rec13); break;
+    case te::ANGULAR_VELOCITIES: te::gather_estimates_kernel<te::ANGULAR_VELOCITIES><<<g, 128, 0, p->stream>>>(b.tiles, slots, n, d_t1, pose, twist, acc, pose6, found, rec13); break;
+    default: te::gather_estimates_kernel<te::ANGULAR_RATES><<<g, 128, 0, p->stream>>>(b.tiles, slots, n, d_t1, pose, twist, acc, pose6, found, rec13); break;
+  }
+  CK(cudaGetLastError());
+}
+
 }  // namespace tehost
 
 using namespace tehost;
@@ -816,19 +829,6 @@ int te_pool_read_state(te_pool* p, long long n, const uint32_t* ids, double* x, 
     CK(cudaStreamSynchronize(p->stream));
     return 0;
   });
-}
-
-static void launch_gather_estimates(te_pool* p, const int* slots, long long n, const double* d_t1, double* pose, double* twist, double* acc,
-                                    double* pose6, uint8_t* found, int rec13) {
-  Buf& b = p->buf[p->cur];
-  const int g = cdiv(n, 128);
-  switch (p->model) {
-    case te::UNIFORM_VELOCITY: te::gather_estimates_kernel<te::UNIFORM_VELOCITY><<<g, 128, 0, p->stream>>>(b.tiles, slots, n, d_t1, pose, twist, acc, pose6, found, rec13); break;
-    case te::UNIFORM_ACCELERATION: te::gather_estimates_kernel<te::UNIFORM_ACCELERATION><<<g, 128, 0, p->stream>>>(b.tiles, slots, n, d_t1, pose, twist, acc, pose6, found, rec13); break;
-    case te::ANGULAR_VELOCITIES: te::gather_estimates_kernel<te::ANGULAR_VELOCITIES><<<g, 128, 0, p->stream>>>(b.tiles, slots, n, d_t1, pose, twist, acc, pose6, found, rec13); break;
-    default: te::gather_estimates_kernel<te::ANGULAR_RATES><<<g, 128, 0, p->stream>>>(b.tiles, slots, n, d_t1, pose, twist, acc, pose6, found, rec13); break;
-  }
-  CK(cudaGetLastError());
 }
 
 int te_pool_read_estimates(te_pool* p, long long n, const uint32_t* ids, const double* t1, double* pose7, double* twist6, double* acc6,

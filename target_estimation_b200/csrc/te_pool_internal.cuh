@@ -4,7 +4,8 @@
 //   te_step.cu     step-kernel launch policy and the stepping entry points (dense / replay / host / by id / fused expiry)
 //   te_mailbox.cu  device-resident mailboxes (the node loop)
 //   te_isolver.cu  batched IntersectionSolver
-//   te_sweep.cu    the k earliest sphere intercepts over every target of a pool (te_pool_earliest_intersections)
+//   te_sweep.cu    the k earliest sphere intercepts and the k nearest targets over every target of a pool
+//                  (te_pool_earliest_intersections, te_pool_nearest_targets)
 //   te_group.cu    several pools on several devices: the NCCL all-gather of estimate records
 #pragma once
 #include <algorithm>
@@ -259,6 +260,9 @@ void init_promoted(te_pool* p, int n_add, const int* new_dst, const Buf& nb, con
 void fetch_last_id(te_pool* p);
 int compact_and_merge(te_pool* p, const te::AddData& ad, const uint32_t* d_add_ids, int n_add, uint32_t* d_erased /*or null*/);
 int* lookup_slots(te_pool* p, const uint32_t* d_ids, long long n);
+// gather_estimates_kernel on the pool's stream: query k reads slot slots[k] (slots NULL = slot k), at d_t1[k] (NULL = now)
+void launch_gather_estimates(te_pool* p, const int* slots, long long n, const double* d_t1, double* pose, double* twist, double* acc,
+                             double* pose6, uint8_t* found, int rec13);
 void fold_pending(te_pool* p);
 void demote_mailboxes(te_pool* p, const uint32_t* ids, const int* d_slots, long long n);
 void attach_mailboxes(te_pool* p, const uint32_t* ids, long long n);

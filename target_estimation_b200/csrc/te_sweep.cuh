@@ -1,14 +1,16 @@
-// te_sweep.cuh -- sm_100a kernels of te_pool_earliest_intersections (te_sweep.cu): for each of a chunk of spheres, the k targets of
-// the pool with the smallest intercept time, selected on the device without sorting the pool.
-//   keys            per sphere, isolver_kernel's delta of every slot (see sweep_broadcast_kernel) becomes a 64-bit key: the bits
-//                   of delta for a hit, ~0 otherwise; hits are counted
+// te_sweep.cuh -- sm_100a kernels of te_pool_earliest_intersections and te_pool_nearest_targets (te_sweep.cu): for each of a chunk
+// of queries, the k targets of the pool with the smallest key, selected on the device without sorting the pool.
+//   keys            per query, one 64-bit key per slot, ~0 for a slot that is no candidate; candidates are counted.  Two producers:
+//                   sweep_key_kernel (the bits of isolver_kernel's delta for a hit, see sweep_broadcast_kernel) and near_key_kernel
+//                   (the bits of the distance for a target inside the query sphere)
 //   hist / select   radix select over the 96-bit composite (rank(key), slot) in eight 12-bit digits: one histogram of the keys that
 //                   still match the selected prefix, then the digit bucket that holds the k-th; refinement stops as soon as that
 //                   bucket is small (usually after the second digit)
-//   collect         every key at or below the boundary bucket: at most k - 1 + SWEEP_SLACK candidates per sphere
-//   output          after a stable sort of the candidates by slot, then by rank (cub::DeviceSegmentedSort): rows of (id, delta)
-// A hit's key orders like its delta (a non-negative double's bits order like the value); rank() maps -0.0 to 0, so -0.0 ranks as 0
-// while the key keeps the bits that query() returns.  Slots are in ascending-id order, so (rank, slot) order is (delta, id) order.
+//   collect         every key at or below the boundary bucket: at most k - 1 + SWEEP_SLACK candidates per query
+//   output          after a stable sort of the candidates by slot, then by rank (cub::DeviceSegmentedSort): rows of (id, value)
+// A candidate's key orders like its value (a non-negative double's bits order like the value); rank() maps -0.0 to 0, so a delta of
+// -0.0 ranks as 0 while the key keeps the bits that query() returns.  Slots are in ascending-id order, so (rank, slot) order is
+// (value, id) order.
 #pragma once
 #include <cub/block/block_scan.cuh>
 
@@ -16,7 +18,7 @@
 
 namespace te {
 
-constexpr int SWEEP_MAX_CHUNK = 32;     // spheres per chunk (the y dimension of the selection kernels' grids)
+constexpr int SWEEP_MAX_CHUNK = 32;     // queries per chunk (the y dimension of the selection kernels' grids)
 constexpr int SWEEP_BINS = 4096;        // 12-bit digits
 constexpr int SWEEP_PASSES = 8;         // 96 bits = 64-bit key + 32-bit slot: (rank, slot) is unique, so 8 digits always resolve
 constexpr unsigned SWEEP_SLACK = 2048;  // a boundary bucket of at most this many keys is collected whole
@@ -82,6 +84,26 @@ static __global__ void sweep_key_kernel(int n, unsigned long long* __restrict__ 
   }
   const unsigned b = __ballot_sync(0xffffffffu, hit);
   if ((threadIdx.x & 31) == 0 && b) atomicAdd(hits, (unsigned long long)__popc(b));
+}
+
+// position (the first three doubles of gather_estimates_kernel's pose7 of every slot) -> key: the bits of the distance to the point
+// for a target inside the sphere (dist <= radius; NaN never is), SWEEP_MISS otherwise; inside targets counted.  Every operation is
+// rounded on its own, in this order, so numpy reproduces the distance bit for bit: ((dx^2 + dy^2) + dz^2), then the square root.
+// dist >= +0 always, so its bits order like its value and sweep_rank leaves them as they are.
+static __global__ void near_key_kernel(int n, const double* __restrict__ pose7, double px, double py, double pz, double radius,
+                                       unsigned long long* __restrict__ keys, unsigned long long* __restrict__ inside) {
+  const int s = blockIdx.x * blockDim.x + threadIdx.x;
+  bool in = false;
+  if (s < n) {
+    const double dx = __dsub_rn(pose7[7 * (size_t)s], px);
+    const double dy = __dsub_rn(pose7[7 * (size_t)s + 1], py);
+    const double dz = __dsub_rn(pose7[7 * (size_t)s + 2], pz);
+    const double dist = __dsqrt_rn(__dadd_rn(__dadd_rn(__dmul_rn(dx, dx), __dmul_rn(dy, dy)), __dmul_rn(dz, dz)));
+    in = dist <= radius;
+    keys[s] = in ? (unsigned long long)__double_as_longlong(dist) : SWEEP_MISS;
+  }
+  const unsigned b = __ballot_sync(0xffffffffu, in);
+  if ((threadIdx.x & 31) == 0 && b) atomicAdd(inside, (unsigned long long)__popc(b));
 }
 
 // per sphere: rows to return and the state of the selection.  Nothing to select when every hit is returned (hits <= k: the empty

@@ -11,6 +11,7 @@
 #include <stdexcept>
 #include <thread>
 
+#include "../csrc/te_nearest_args.h"
 #include "target_estimation_b200/target_manager.hpp"
 
 namespace target_estimation_b200 {
@@ -318,6 +319,22 @@ void ShardedTargetManager::getEstimatesBatch(long long n, const unsigned* ids, c
       if (found) found[k] = fo[(size_t)j];
     }
   });
+}
+
+long long ShardedTargetManager::nearestTargets(long long q, const double* t1, const double* point, const double* radius, long long k,
+                                               unsigned* ids_out, double* dist_out, long long* count_out) {
+  te::check_nearest_args(q, point, radius, k, ids_out, dist_out, count_out);
+  std::lock_guard<std::recursive_mutex> lg(target_lock_);
+  if (q == 0) return 0;
+  flush();
+  std::vector<TargetManager*> shards;
+  for (auto& s : shard_) shards.push_back(s.get());
+  return nearest_rows_.run(
+      shards, [this](const std::function<void(int)>& f) { forEachShard(f); }, q, k,
+      [&](te_pool* p, unsigned* ids, double* dist, long long* count) {
+        return te_pool_nearest_targets(p, q, t1, point, radius, k, ids, dist, count);
+      },
+      ids_out, dist_out, count_out);
 }
 
 // ---- dense ticks: shard-major records, every shard's slice on its own device at once ---------------------------------------------

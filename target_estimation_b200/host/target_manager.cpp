@@ -14,6 +14,8 @@
 #include <stdexcept>
 #include <unordered_set>
 
+#include "../csrc/te_nearest_args.h"
+
 namespace target_estimation_b200 {
 
 namespace {
@@ -1155,83 +1157,104 @@ long long IntersectionSolver::earliestIntersections(long long q, const double* t
   std::lock_guard<std::recursive_mutex> lg(target_manager_->lock());
   if (q == 0) return 0;
   target_manager_->flush();
-  const int G = (int)solvers_.size();
-  if (sweep_.empty()) sweep_.resize(4 * (size_t)G);
+  std::vector<TargetManager*> shards;
+  for (int r = 0; r < (int)solvers_.size(); ++r) shards.push_back(&shardOf(r));
+  return sweep_.run(
+      shards, [&](const std::function<void(int)>& f) { sharded_ ? sharded_->forEachShard(f) : f(0); }, q, k,
+      [&](te_pool* p, unsigned* ids, double* delta, long long* hits) {
+        return te_pool_earliest_intersections(p, q, t1, origin, radius, k, ids, delta, hits);
+      },
+      ids_out, delta_out, hits_out);
+}
+
+long long PoolRowMerge::run(const std::vector<TargetManager*>& shards, const std::function<void(const std::function<void(int)>&)>& each_shard,
+                            long long q, long long k, const PoolQuery& query, unsigned* ids_out, double* val_out, long long* count_out) {
+  const int G = (int)shards.size();
+  if (lists_.size() < 4 * (size_t)G) lists_.resize(4 * (size_t)G);
   int n_lists = 0, only = -1;
   for (int r = 0; r < G; ++r)
     for (int t = 0; t < 4; ++t) {
-      te_pool* p = shardOf(r).poolOf(t, false);
-      SweepList& L = sweep_[(size_t)r * 4 + (size_t)t];
+      te_pool* p = shards[(size_t)r]->poolOf(t, false);
+      List& L = lists_[(size_t)r * 4 + (size_t)t];
       L.used = p && te_pool_size(p) > 0;
       if (L.used) { ++n_lists; only = r * 4 + t; }
     }
-  auto run = [&](int r, int t, unsigned* ids, double* delta, long long* hits) {
-    TargetManager& M = shardOf(r);
+  auto run_pool = [&](int r, int t, unsigned* ids, double* val, long long* count) {
+    TargetManager& M = *shards[(size_t)r];
     std::lock_guard<std::recursive_mutex> lk(M.lock());
-    ck(te_pool_earliest_intersections(M.poolOf(t, false), q, t1, origin, radius, k, ids, delta, hits));
+    ck(query(M.poolOf(t, false), ids, val, count));
   };
   if (n_lists == 1) {   // one pool holds every target: its rows are the answer
-    run(only / 4, only % 4, ids_out, delta_out, hits_out);
+    run_pool(only / 4, only % 4, ids_out, val_out, count_out);
   } else {
     auto run_shard = [&](int r) {
       for (int t = 0; t < 4; ++t) {
-        SweepList& L = sweep_[(size_t)r * 4 + (size_t)t];
+        List& L = lists_[(size_t)r * 4 + (size_t)t];
         if (!L.used) continue;
-        L.ids.resize((size_t)(q * k)); L.delta.resize((size_t)(q * k)); L.hits.resize((size_t)q);
-        run(r, t, L.ids.data(), L.delta.data(), L.hits.data());
+        L.ids.resize((size_t)(q * k)); L.val.resize((size_t)(q * k)); L.count.resize((size_t)q);
+        run_pool(r, t, L.ids.data(), L.val.data(), L.count.data());
       }
     };
-    // merge sphere j's sorted lists by (rank(delta), id): -0.0 ranks as 0, a non-negative double's bits order like its value
+    // merge query j's sorted lists by (rank(value), id): -0.0 ranks as 0, a non-negative double's bits order like its value
     auto rank = [](double d) {
       unsigned long long b;
       std::memcpy(&b, &d, 8);
       return b == 0x8000000000000000ull ? 0ull : b;
     };
-    std::vector<const SweepList*> used;
-    for (const SweepList& L : sweep_)
-      if (L.used) used.push_back(&L);
+    std::vector<const List*> used;
+    for (int l = 0; l < 4 * G; ++l)
+      if (lists_[(size_t)l].used) used.push_back(&lists_[(size_t)l]);
     auto merge = [&](long long j, std::vector<long long>& at) {
-      long long hits = 0;
-      for (const SweepList* L : used) hits += L->hits[(size_t)j];
-      hits_out[j] = hits;
+      long long count = 0;
+      for (const List* L : used) count += L->count[(size_t)j];
+      count_out[j] = count;
       at.assign(used.size(), 0);
       for (long long row = 0; row < k; ++row) {
         int best = -1;
         unsigned long long best_rank = 0;
         unsigned best_id = 0;
         for (size_t l = 0; l < used.size(); ++l) {
-          const SweepList& L = *used[l];
-          if (at[l] >= std::min(k, L.hits[(size_t)j])) continue;
+          const List& L = *used[l];
+          if (at[l] >= std::min(k, L.count[(size_t)j])) continue;
           const size_t o = (size_t)(j * k + at[l]);
-          const unsigned long long rk = rank(L.delta[o]);
+          const unsigned long long rk = rank(L.val[o]);
           if (best < 0 || rk < best_rank || (rk == best_rank && L.ids[o] < best_id)) { best = (int)l; best_rank = rk; best_id = L.ids[o]; }
         }
         const size_t out = (size_t)(j * k + row);
         if (best < 0) {
           ids_out[out] = 0xFFFFFFFFu;
-          delta_out[out] = -1.0;
+          val_out[out] = -1.0;
         } else {
           const size_t o = (size_t)(j * k + at[(size_t)best]++);
           ids_out[out] = used[(size_t)best]->ids[o];
-          delta_out[out] = used[(size_t)best]->delta[o];
+          val_out[out] = used[(size_t)best]->val[o];
         }
       }
     };
-    if (sharded_) {   // every shard's pools at once, then the spheres' merges spread over the shards' workers
-      sharded_->forEachShard(run_shard);
-      sharded_->forEachShard([&](int r) {
-        std::vector<long long> at;
-        for (long long j = r; j < q; j += G) merge(j, at);
-      });
-    } else {
-      run_shard(0);
+    // every shard's pools at once, then the queries' merges spread over the shards' workers
+    each_shard(run_shard);
+    each_shard([&](int r) {
       std::vector<long long> at;
-      for (long long j = 0; j < q; ++j) merge(j, at);
-    }
+      for (long long j = r; j < q; j += G) merge(j, at);
+    });
   }
   long long total = 0;
-  for (long long j = 0; j < q; ++j) total += hits_out[j];
+  for (long long j = 0; j < q; ++j) total += count_out[j];
   return total;
+}
+
+long long TargetManager::nearestTargets(long long q, const double* t1, const double* point, const double* radius, long long k,
+                                        unsigned* ids_out, double* dist_out, long long* count_out) {
+  te::check_nearest_args(q, point, radius, k, ids_out, dist_out, count_out);
+  std::lock_guard<std::recursive_mutex> lg(target_lock_);
+  if (q == 0) return 0;
+  flushLocked();
+  return nearest_rows_.run(
+      {this}, [](const std::function<void(int)>& f) { f(0); }, q, k,
+      [&](te_pool* p, unsigned* ids, double* dist, long long* count) {
+        return te_pool_nearest_targets(p, q, t1, point, radius, k, ids, dist, count);
+      },
+      ids_out, dist_out, count_out);
 }
 
 // ----------------------------------------------------------------------------------------------

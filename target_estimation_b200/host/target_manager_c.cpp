@@ -183,6 +183,13 @@ int target_manager_get_state(const target_manager_c* self, unsigned int id, doub
 void target_manager_flush(const target_manager_c* self) {
   guard(0, [&] { M(self)->flush(); return 0; });
 }
+long long target_manager_nearest(const target_manager_c* self, long long q, const double* t1, const double* point, const double* radius, long long k,
+                                 unsigned int* ids_out, double* dist_out, long long* count_out) {
+  return guard(-1LL, [&] {
+    if (!self) throw std::invalid_argument("null manager");
+    return M(self)->nearestTargets(q, t1, point, radius, k, ids_out, dist_out, count_out);
+  });
+}
 const char* target_manager_last_error(void) { return g_err.c_str(); }
 
 // ---- IntersectionSolver -------------------------------------------------------------------------------------------

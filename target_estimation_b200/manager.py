@@ -36,6 +36,7 @@ _SIG = {
     "target_manager_get_ids": (_ll, [_p, _p, _ll]),
     "target_manager_get_state": (_i, [_p, _u, _p, _p, _p]),
     "target_manager_flush": (None, [_p]),
+    "target_manager_nearest": (_ll, [_p, _ll, _p, _p, _p, _ll, _p, _p, _p]),
     "target_manager_last_error": (C.c_char_p, []),
     "target_manager_watch": (None, [_p, _ll, _p, _ll]),
     "target_manager_log_samples": (_ll, [_p]),
@@ -214,6 +215,21 @@ class TargetManagerC:
 
     def flush(self):
         clib.target_manager_flush(self.h)
+
+    def nearest(self, t1, point, radius, k):
+        """the k nearest targets inside a sphere: query j = (t1[j], point[j], radius[j]); t1 (None = current estimates) and radius
+        broadcast to q = len(point).  Returns (count [q], ids [q][k], dist [q][k]): rows past min(k, count[j]) are id 0xFFFFFFFF and
+        dist -1.  The pose of a returned target is get_estimates_batch(ids, t1)."""
+        point = np.ascontiguousarray(point, dtype=np.float64).reshape(-1, 3)
+        q, k = point.shape[0], int(k)
+        t1 = np.ascontiguousarray(np.broadcast_to(t1, (q,)), dtype=np.float64) if t1 is not None else None
+        radius = np.ascontiguousarray(np.broadcast_to(radius, (q,)), dtype=np.float64)
+        count = np.zeros(q, dtype=np.int64)
+        ids = np.zeros((q, max(k, 0)), dtype=np.uint32)
+        dist = np.zeros((q, max(k, 0)))
+        if int(clib.target_manager_nearest(self.h, q, _ptr(t1), _ptr(point), _ptr(radius), k, _ptr(ids), _ptr(dist), _ptr(count))) < 0:
+            raise RuntimeError(clib.target_manager_last_error().decode())
+        return count, ids, dist
 
 
 class ShardedManagerC(TargetManagerC):

@@ -311,6 +311,21 @@ class TargetPool:
         check(lib.te_pool_earliest_intersections(self._h, q, _ptr(t1), _ptr(origin), _ptr(radius), k, _ptr(ids), _ptr(delta), _ptr(hits)))
         return hits, ids, delta
 
+    # -- the k nearest targets inside a sphere (te_pool_nearest_targets) ------
+    def nearest_targets(self, t1, point, radius, k):
+        """query j = (t1[j], point[j], radius[j]); t1 (None = current estimates) and radius broadcast to q = len(point).  Returns
+        (count [q], ids [q][k], dist [q][k]) with the targets inside each sphere by (dist, id) first and rows of id 0xFFFFFFFF /
+        dist -1 after them."""
+        point = _np(point, np.float64).reshape(-1, 3)
+        q, k = point.shape[0], int(k)
+        t1 = _np(np.broadcast_to(t1, (q,)), np.float64) if t1 is not None else None
+        radius = _np(np.broadcast_to(radius, (q,)), np.float64)
+        count = np.zeros(q, dtype=np.int64)
+        ids = np.zeros((q, max(k, 0)), dtype=np.uint32)
+        dist = np.zeros((q, max(k, 0)))
+        check(lib.te_pool_nearest_targets(self._h, q, _ptr(t1), _ptr(point), _ptr(radius), k, _ptr(ids), _ptr(dist), _ptr(count)))
+        return count, ids, dist
+
 
 class IntersectionSolver:
     """Batched IntersectionSolver: n_streams independent reference solver objects (include/te_pool.h)."""
