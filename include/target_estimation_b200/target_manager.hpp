@@ -178,7 +178,8 @@ class TargetManager {
                               const double* t0, const double* p0, const double* v0 = nullptr, const double* a0 = nullptr,
                               const double* p0_scale = nullptr);
   // (an id may appear more than once: the records are applied in order, as the reference's sequential update() calls would --
-  //  the batch is cut in front of every repeat and the pieces are launched one after the other)
+  //  the batch is cut in front of every repeat and the pieces are launched one after the other; meas may be NULL only when no
+  //  record is an UPDATE -- action NULL means UPDATE for every record -- else std::invalid_argument before any pool is stepped)
   virtual long long updateBatch(long long n, const unsigned* ids, double dt, const double* meas /*[n][7]*/, const unsigned char* action = nullptr);
   virtual long long eraseBatch(long long n, const unsigned* ids);
   virtual void getEstimatesBatch(long long n, const unsigned* ids, const double* t1, double* pose7, double* twist6, double* acc6,
@@ -224,6 +225,9 @@ class TargetManager {
   struct Slot { int type; };
   bool typeOf(unsigned id, int& type);
   te_pool* poolOf(int type, bool create);
+  unsigned heldTypes();   // bit t set = the pool of model type t holds targets
+  // the rows of a batch by model type of their id (one registry lookup per id; call order kept; unknown ids in no list)
+  void rowsByType(long long n, const unsigned* ids, std::vector<long long> rows[4]);
   int device() const { return device_; }
   std::recursive_mutex& lock() { return target_lock_; }
 
@@ -236,6 +240,8 @@ class TargetManager {
   void flushLocked();
   int registerClass(int type, const MatrixXd& Q, const MatrixXd& R, const MatrixXd& P0);
   void queue(int type, unsigned id, double dt, const double* meas, int action);
+  // updateBatch's arguments: meas NULL with action NULL or with an UPDATE op throws std::invalid_argument
+  static void requireMeasurements(long long n, const double* meas, const unsigned char* action);
   long long updateBatchUnique(long long n, const unsigned* ids, double dt, const double* meas, const unsigned char* action);   // no id twice
   te_pool* densePool();   // the one non-empty pool of a homogeneous manager (throws otherwise)
   PoolRowMerge nearest_rows_;
@@ -326,8 +332,8 @@ class IntersectionSolver {
     std::vector<int> stream;
     std::vector<double> t1, origin, radius, pos_th, ang_th, delta, pose;
     std::vector<unsigned char> conv;
-    int only = -1;                       // model type of the shard's targets, -1 = no target, -2 = several types (see type)
-    std::vector<signed char> type;       // several types: model type per query, -1 = unknown id
+    int only = -1;                       // model type of the shard's targets, -1 = no target, -2 = several types (see rows)
+    std::vector<long long> rows[4];      // several types: the queries of each model type (unknown ids in none)
     std::vector<std::vector<int>> moves;   // [type * G + source shard]: streams whose state comes from that shard
     long long found = 0;
   };
@@ -462,8 +468,8 @@ class TickTargetManager : public TargetManager, public TickFrontEnd {
 // the 8 GPUs of one box with no collective on the hot path ... the TargetManager API stays as the host surface in C++").
 // owner(id) = id mod G; shard r is an ordinary TargetManager on device devices[r] with its own pools and streams.  Per-id calls
 // go to the owner (their launches coalesce per shard as in TargetManager).  The batched calls route their records to the owners
-// in one host pass -- every shard's worker thread picks its own records out of the caller's arrays into page-locked staging, in
-// the caller's order, and runs the shard's batched call -- so the G devices copy and step concurrently.  Results are the
+// with one parallel stable partition on the host (routeOnHost: every shard's records in the caller's order), then every shard's
+// worker thread runs the shard's batched call -- so the G devices copy and step concurrently.  Results are the
 // reference's: an id lives in exactly one shard, its records are applied in call order.
 // The optional exchange of estimates (SURVEY.md 8(e)) is gatherEstimates(): [pose7 | twist6] records of every target, all shards,
 // gathered on every device over NCCL (te_group_*), then read back from the publishing shard's device.
@@ -545,6 +551,7 @@ class ShardedTargetManager : public TargetManager {
   // the batch and puts record k of owner r at place at[r]++ of r's staging.  Returns the records of every shard.
   std::vector<size_t> routeOnHost(long long n, const unsigned* ids, const std::function<void(int, size_t)>& reserve,
                                   const std::function<void(int, long long, long long, size_t*)>& scatter);
+  std::vector<std::vector<long long>> rowsByOwner(long long n, const unsigned* ids);   // routeOnHost: every shard's rows of the batch
   te_group* group();   // created on first use
   friend class IntersectionSolver;   // routes its queries with routeOnHost and runs them with forEachShard
   std::vector<std::unique_ptr<TargetManager>> shard_;
@@ -555,7 +562,6 @@ class ShardedTargetManager : public TargetManager {
   double gather_ms_ = -1.0;
   struct Stage {   // per shard, page-locked, grow-only
     std::vector<unsigned> ids;
-    std::vector<long long> where;
     double* meas = nullptr;
     unsigned char* action = nullptr;
     size_t cap = 0;

@@ -47,7 +47,8 @@ long long target_manager_init_batch(const target_manager_c* self, long long n, c
                                     const double* t0 /* [n] or NULL = 0 */);
 /* one tick: action[k] 2 = update(id,dt,meas[k]) / 1 = update(id,dt) / 0 = skip; action NULL = all 2.
  * Returns #applied (unknown ids are skipped like the reference's "does not exist").  An id may be named more than once:
- * its records are applied in order, like the reference's sequential update() calls (one launch per run of distinct ids). */
+ * its records are applied in order, like the reference's sequential update() calls (one launch per run of distinct ids).
+ * meas NULL with action NULL or with any action 2 is an error (-1, nothing applied). */
 long long target_manager_update_batch(const target_manager_c* self, long long n, const unsigned int* ids, double dt, const double* meas,
                                       const unsigned char* action);
 /* one dense tick from host arrays: record k belongs to the k-th id of target_manager_get_dense_ids (a plain manager: ascending ids;

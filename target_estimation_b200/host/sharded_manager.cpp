@@ -12,6 +12,7 @@
 #include <thread>
 
 #include "../csrc/te_nearest_args.h"
+#include "rows.hpp"
 #include "target_estimation_b200/target_manager.hpp"
 
 namespace target_estimation_b200 {
@@ -187,24 +188,16 @@ std::vector<unsigned int> ShardedTargetManager::getAvailableTargets() {
 long long ShardedTargetManager::initBatch(target_t type, const MatrixXd& Q, const MatrixXd& R, const MatrixXd& P0, long long n, const unsigned* ids,
                                           double dt0, const double* t0, const double* p0, const double* v0, const double* a0, const double* p0_scale) {
   if (n <= 0) return 0;
-  const unsigned G = (unsigned)shard_.size();
-  const FastMod owner_of(G);
+  const std::vector<std::vector<long long>> rows = rowsByOwner(n, ids);
   std::atomic<long long> added{0};
   forEachShard([&](int r) {
+    const std::vector<long long>& mine = rows[(size_t)r];
+    if (mine.empty()) return;
     std::vector<unsigned> s_ids;
     std::vector<double> s_t0, s_p0, s_v0, s_a0, s_sc;
-    for (long long k = 0; k < n; ++k) {
-      if (owner_of(ids[k]) != (unsigned)r) continue;
-      s_ids.push_back(ids[k]);
-      if (t0) s_t0.push_back(t0[k]);
-      if (p0) s_p0.insert(s_p0.end(), p0 + 7 * k, p0 + 7 * k + 7);
-      if (v0) s_v0.insert(s_v0.end(), v0 + 6 * k, v0 + 6 * k + 6);
-      if (a0) s_a0.insert(s_a0.end(), a0 + 6 * k, a0 + 6 * k + 6);
-      if (p0_scale) s_sc.push_back(p0_scale[k]);
-    }
-    if (s_ids.empty()) return;
-    added += shard_[(size_t)r]->initBatch(type, Q, R, P0, (long long)s_ids.size(), s_ids.data(), dt0, t0 ? s_t0.data() : nullptr, p0 ? s_p0.data() : nullptr,
-                                          v0 ? s_v0.data() : nullptr, a0 ? s_a0.data() : nullptr, p0_scale ? s_sc.data() : nullptr);
+    added += shard_[(size_t)r]->initBatch(type, Q, R, P0, (long long)mine.size(), gatherRows<1>(ids, mine, s_ids), dt0, gatherRows<1>(t0, mine, s_t0),
+                                          gatherRows<7>(p0, mine, s_p0), gatherRows<6>(v0, mine, s_v0), gatherRows<6>(a0, mine, s_a0),
+                                          gatherRows<1>(p0_scale, mine, s_sc));
   });
   return added.load();
 }
@@ -214,6 +207,7 @@ long long ShardedTargetManager::updateBatch(long long n, const unsigned* ids, do
   const unsigned G = (unsigned)shard_.size();
   const FastMod owner_of(G);
   if (G == 1) return shard_[0]->updateBatch(n, ids, dt, meas, action);
+  requireMeasurements(n, meas, action);   // before any shard steps
   const std::vector<size_t> total = routeOnHost(
       n, ids,
       [&](int r, size_t m) {   // (each worker sizes its own shard's staging: page-locking is the slow part and runs in parallel)
@@ -274,16 +268,28 @@ std::vector<size_t> ShardedTargetManager::routeOnHost(long long n, const unsigne
   return total;
 }
 
+std::vector<std::vector<long long>> ShardedTargetManager::rowsByOwner(long long n, const unsigned* ids) {
+  const FastMod owner_of((unsigned)shard_.size());
+  std::vector<std::vector<long long>> rows(shard_.size());
+  routeOnHost(
+      n, ids, [&](int r, size_t m) { rows[(size_t)r].resize(m); },
+      [&](int, long long lo, long long hi, size_t* at) {
+        for (long long k = lo; k < hi; ++k) {
+          const unsigned r = owner_of(ids[k]);
+          rows[r][at[r]++] = k;
+        }
+      });
+  return rows;
+}
+
 long long ShardedTargetManager::eraseBatch(long long n, const unsigned* ids) {
   if (n <= 0) return 0;
-  const unsigned G = (unsigned)shard_.size();
-  const FastMod owner_of(G);
+  const std::vector<std::vector<long long>> rows = rowsByOwner(n, ids);
   std::atomic<long long> erased{0};
   forEachShard([&](int r) {
+    const std::vector<long long>& mine = rows[(size_t)r];
     std::vector<unsigned> s_ids;
-    for (long long k = 0; k < n; ++k)
-      if (owner_of(ids[k]) == (unsigned)r) s_ids.push_back(ids[k]);
-    if (!s_ids.empty()) erased += shard_[(size_t)r]->eraseBatch((long long)s_ids.size(), s_ids.data());
+    if (!mine.empty()) erased += shard_[(size_t)r]->eraseBatch((long long)mine.size(), gatherRows<1>(ids, mine, s_ids));
   });
   return erased.load();
 }
@@ -291,33 +297,22 @@ long long ShardedTargetManager::eraseBatch(long long n, const unsigned* ids) {
 void ShardedTargetManager::getEstimatesBatch(long long n, const unsigned* ids, const double* t1, double* pose7, double* twist6, double* acc6,
                                              unsigned char* found) {
   if (n <= 0) return;
-  const unsigned G = (unsigned)shard_.size();
-  const FastMod owner_of(G);
-  if (G == 1) return shard_[0]->getEstimatesBatch(n, ids, t1, pose7, twist6, acc6, found);
+  if (shard_.size() == 1) return shard_[0]->getEstimatesBatch(n, ids, t1, pose7, twist6, acc6, found);
+  const std::vector<std::vector<long long>> rows = rowsByOwner(n, ids);
   forEachShard([&](int r) {
-    Stage& st = stage_[(size_t)r];
-    st.ids.clear();
-    st.where.clear();
-    std::vector<double> s_t1;
-    for (long long k = 0; k < n; ++k) {
-      if (owner_of(ids[k]) != (unsigned)r) continue;
-      st.ids.push_back(ids[k]);
-      st.where.push_back(k);
-      if (t1) s_t1.push_back(t1[k]);
-    }
-    const long long m = (long long)st.ids.size();
+    const std::vector<long long>& mine = rows[(size_t)r];
+    const size_t m = mine.size();
     if (m == 0) return;
-    std::vector<double> po(pose7 ? (size_t)m * 7 : 0), tw(twist6 ? (size_t)m * 6 : 0), ac(acc6 ? (size_t)m * 6 : 0);
-    std::vector<unsigned char> fo((size_t)m, 0);
-    shard_[(size_t)r]->getEstimatesBatch(m, st.ids.data(), t1 ? s_t1.data() : nullptr, pose7 ? po.data() : nullptr, twist6 ? tw.data() : nullptr,
-                                         acc6 ? ac.data() : nullptr, fo.data());
-    for (long long j = 0; j < m; ++j) {   // rows of different shards are disjoint: no two threads write the same output row
-      const long long k = st.where[(size_t)j];
-      if (pose7) std::memcpy(pose7 + 7 * k, &po[7 * (size_t)j], 56);
-      if (twist6) std::memcpy(twist6 + 6 * k, &tw[6 * (size_t)j], 48);
-      if (acc6) std::memcpy(acc6 + 6 * k, &ac[6 * (size_t)j], 48);
-      if (found) found[k] = fo[(size_t)j];
-    }
+    std::vector<unsigned> s_ids;
+    std::vector<double> s_t1, po(pose7 ? m * 7 : 0), tw(twist6 ? m * 6 : 0), ac(acc6 ? m * 6 : 0);
+    std::vector<unsigned char> fo(m, 0);
+    shard_[(size_t)r]->getEstimatesBatch((long long)m, gatherRows<1>(ids, mine, s_ids), gatherRows<1>(t1, mine, s_t1), pose7 ? po.data() : nullptr,
+                                         twist6 ? tw.data() : nullptr, acc6 ? ac.data() : nullptr, fo.data());
+    // rows of different shards are disjoint: no two threads write the same output row
+    scatterRows<7>(pose7, mine, po.data());
+    scatterRows<6>(twist6, mine, tw.data());
+    scatterRows<6>(acc6, mine, ac.data());
+    scatterRows<1>(found, mine, fo.data());
   });
 }
 
@@ -396,8 +391,7 @@ long long ShardedTargetManager::gatherEstimates(std::vector<unsigned>* ids, std:
   for (int type = 0; type < 4; ++type) {
     bool any = false;
     for (size_t r = 0; r < shard_.size(); ++r) {
-      pools[r] = shard_[r]->poolOf(type, false);
-      if (pools[r] && te_pool_size(pools[r]) == 0) pools[r] = nullptr;
+      pools[r] = (shard_[r]->heldTypes() >> type) & 1u ? shard_[r]->poolOf(type, false) : nullptr;
       any = any || pools[r];
     }
     if (!any) continue;

@@ -10,11 +10,13 @@
 #include <cstring>
 #include <fstream>
 #include <iostream>
+#include <numeric>
 #include <sstream>
 #include <stdexcept>
 #include <unordered_set>
 
 #include "../csrc/te_nearest_args.h"
+#include "rows.hpp"
 
 namespace target_estimation_b200 {
 
@@ -26,6 +28,8 @@ struct PoolError : std::runtime_error {
 inline void ck(long long rc) {
   if (rc < 0) throw PoolError(te_last_error());
 }
+// the model type of a TargetManager::heldTypes() mask: the one type, -1 = no target, -2 = several types
+inline int onlyType(unsigned held) { return held == 0 ? -1 : (held & (held - 1)) ? -2 : __builtin_ctz(held); }
 
 // --- minimal reader for the reference's model files (models/*.yaml: `key: scalar` and
 // `key: [v, v, ...]` lines; yaml-cpp is not available in this image) -------------------------
@@ -227,6 +231,28 @@ bool TargetManager::typeOf(unsigned id, int& type) {
   return true;
 }
 
+unsigned TargetManager::heldTypes() {
+  unsigned held = 0;
+  for (int t = 0; t < 4; ++t)
+    if (pools_[t] && te_pool_size(pools_[t]) > 0) held |= 1u << t;
+  return held;
+}
+
+void TargetManager::rowsByType(long long n, const unsigned* ids, std::vector<long long> rows[4]) {
+  for (int t = 0; t < 4; ++t) rows[t].clear();
+  for (long long k = 0; k < n; ++k) {
+    auto it = targets_.find(ids[k]);
+    if (it != targets_.end()) rows[it->second].push_back(k);
+  }
+}
+
+void TargetManager::requireMeasurements(long long n, const double* meas, const unsigned char* action) {
+  if (meas) return;
+  bool needs = !action;
+  for (long long k = 0; k < n && !needs; ++k) needs = action[k] == TE_ACT_UPDATE;
+  if (needs) throw std::invalid_argument("update ops without measurements");
+}
+
 void TargetManager::init(const unsigned int& id, const double& dt0, const double& t0, const Vector7d& p0, const Vector6d& v0,
                          const Vector6d& a0) {   // :135-142
   if (default_values_loaded_) init(default_type_, id, dt0, t0, default_Q_, default_R_, default_P_, p0, v0, a0);
@@ -309,23 +335,16 @@ long long TargetManager::initBatch(target_t type, const MatrixXd& Q, const Matri
   }
   if (keep.empty()) return 0;
   const long long na = (long long)keep.size();
-  std::vector<uint32_t> g_ids((size_t)na);
+  std::vector<uint32_t> g_ids;
   std::vector<uint16_t> g_cls((size_t)na, (uint16_t)cls);
-  std::vector<double> g_t0, g_p0((size_t)na * 7), g_v0, g_a0, g_sc;
-  auto gather = [&](const double* src, int w, std::vector<double>& dst) -> const double* {
-    if (!src) return nullptr;
-    dst.resize((size_t)na * w);
-    for (long long k = 0; k < na; ++k) std::memcpy(&dst[(size_t)k * w], src + (size_t)keep[k] * w, sizeof(double) * w);
-    return dst.data();
-  };
-  for (long long k = 0; k < na; ++k) g_ids[k] = ids[keep[k]];
+  std::vector<double> g_t0, g_p0, g_v0, g_a0, g_sc;
   const bool all = na == n;
-  const double* s_p0 = all ? p0 : gather(p0, 7, g_p0);
-  const double* s_t0 = all ? t0 : gather(t0, 1, g_t0);
-  const double* s_v0 = all ? v0 : gather(v0, 6, g_v0);
-  const double* s_a0 = all ? a0 : gather(a0, 6, g_a0);
-  const double* s_sc = all ? p0_scale : gather(p0_scale, 1, g_sc);
-  long long added = te_pool_add_batch(poolOf((int)type, true), na, g_ids.data(), g_cls.data(), s_t0, s_p0, s_v0, s_a0, s_sc);
+  const double* s_p0 = all ? p0 : gatherRows<7>(p0, keep, g_p0);
+  const double* s_t0 = all ? t0 : gatherRows<1>(t0, keep, g_t0);
+  const double* s_v0 = all ? v0 : gatherRows<6>(v0, keep, g_v0);
+  const double* s_a0 = all ? a0 : gatherRows<6>(a0, keep, g_a0);
+  const double* s_sc = all ? p0_scale : gatherRows<1>(p0_scale, keep, g_sc);
+  long long added = te_pool_add_batch(poolOf((int)type, true), na, gatherRows<1>(ids, keep, g_ids), g_cls.data(), s_t0, s_p0, s_v0, s_a0, s_sc);
   ck(added);
   targets_.insert(fresh.begin(), fresh.end());
   return added;
@@ -397,6 +416,7 @@ void TargetManager::update(const double& dt) {   // :220-225
 long long TargetManager::updateBatch(long long n, const unsigned* ids, double dt, const double* meas, const unsigned char* action) {
   std::lock_guard<std::recursive_mutex> lg(target_lock_);
   if (n <= 0) return 0;
+  requireMeasurements(n, meas, action);
   flushLocked();
   // te_pool_step_ids applies one op per id per launch.  A batch that names an id again stands for the reference's sequential
   // update() calls, which apply every record in order: cut the batch in front of each repeat and launch the pieces one after
@@ -408,11 +428,9 @@ long long TargetManager::updateBatch(long long n, const unsigned* ids, double dt
     // ids in arbitrary order (a /tf message lists its targets as they come): a homogeneous manager hands the batch over as it is --
     // the device finds a repeated id while it looks the ids up, before anything is stepped (te_pool_step_ids returns -2) -- and
     // only then the batch is cut on the host (a hash set of four million ids costs 50 x the tick it guards)
-    int n_pools = 0, only = -1;
-    for (int t = 0; t < 4; ++t)
-      if (pools_[t] && te_pool_size(pools_[t]) > 0) { ++n_pools; only = t; }
-    if (n_pools == 0) return 0;
-    if (n_pools == 1) {
+    const int only = onlyType(heldTypes());
+    if (only == -1) return 0;
+    if (only >= 0) {
       const long long rc = te_pool_step_ids(pools_[only], n, ids, nullptr, dt, meas, action);
       if (rc != -2) {
         ck(rc);
@@ -436,32 +454,24 @@ long long TargetManager::updateBatch(long long n, const unsigned* ids, double dt
 
 long long TargetManager::updateBatchUnique(long long n, const unsigned* ids, double dt, const double* meas, const unsigned char* action) {
   if (n <= 0) return 0;
-  int n_pools = 0, only = -1;
-  for (int t = 0; t < 4; ++t)
-    if (pools_[t] && te_pool_size(pools_[t]) > 0) { ++n_pools; only = t; }
-  if (n_pools == 0) return 0;
-  if (n_pools == 1) {   // homogeneous manager: the batch goes to the device as it is
+  const int only = onlyType(heldTypes());
+  if (only == -1) return 0;
+  if (only >= 0) {   // homogeneous manager: the batch goes to the device as it is
     long long rc = te_pool_step_ids(pools_[only], n, ids, nullptr, dt, meas, action);
     ck(rc);
     return rc;
   }
   // mixed manager: split the batch by model type on the host
-  Pending split[4];
-  for (long long k = 0; k < n; ++k) {
-    auto it = targets_.find(ids[k]);
-    if (it == targets_.end()) continue;
-    Pending& q = split[it->second];
-    q.ids.push_back(ids[k]);
-    q.action.push_back(action ? action[k] : (uint8_t)TE_ACT_UPDATE);
-    const size_t o = q.meas.size();
-    q.meas.resize(o + 7, 0.0);
-    if (meas) std::memcpy(&q.meas[o], meas + 7 * (size_t)k, 7 * sizeof(double));
-  }
+  std::vector<long long> rows[4];
+  rowsByType(n, ids, rows);
+  std::vector<uint32_t> s_ids;
+  std::vector<double> s_meas;
+  std::vector<uint8_t> s_act;
   long long applied = 0;
   for (int t = 0; t < 4; ++t) {
-    if (split[t].ids.empty()) continue;
-    long long rc = te_pool_step_ids(pools_[t], (long long)split[t].ids.size(), split[t].ids.data(), nullptr, dt, split[t].meas.data(),
-                                    split[t].action.data());
+    if (rows[t].empty()) continue;
+    long long rc = te_pool_step_ids(pools_[t], (long long)rows[t].size(), gatherRows<1>(ids, rows[t], s_ids), nullptr, dt,
+                                    gatherRows<7>(meas, rows[t], s_meas), gatherRows<1>(action, rows[t], s_act));
     ck(rc);
     applied += rc;
   }
@@ -469,10 +479,8 @@ long long TargetManager::updateBatchUnique(long long n, const unsigned* ids, dou
 }
 
 te_pool* TargetManager::densePool() {
-  int n_pools = 0, only = -1;
-  for (int t = 0; t < 4; ++t)
-    if (pools_[t] && te_pool_size(pools_[t]) > 0) { ++n_pools; only = t; }
-  if (n_pools != 1) throw std::invalid_argument("a dense tick needs a manager whose targets share one model type");
+  const int only = onlyType(heldTypes());
+  if (only < 0) throw std::invalid_argument("a dense tick needs a manager whose targets share one model type");
   return pools_[only];
 }
 
@@ -524,12 +532,12 @@ bool TargetManager::erase(const unsigned int& id) {   // :227-241
 long long TargetManager::eraseBatch(long long n, const unsigned* ids) {
   std::lock_guard<std::recursive_mutex> lg(target_lock_);
   flushLocked();
+  std::vector<long long> rows[4];
+  rowsByType(n, ids, rows);
   std::vector<uint32_t> per[4], found;
-  for (long long k = 0; k < n; ++k) {
-    auto it = targets_.find(ids[k]);
-    if (it == targets_.end()) continue;
-    per[it->second].push_back(ids[k]);
-    found.push_back(ids[k]);
+  for (int t = 0; t < 4; ++t) {
+    gatherRows<1>(ids, rows[t], per[t]);
+    found.insert(found.end(), per[t].begin(), per[t].end());
   }
   std::sort(found.begin(), found.end());
   targets_.eraseSorted(found.data(), found.size());
@@ -555,38 +563,27 @@ void TargetManager::getEstimatesBatch(long long n, const unsigned* ids, const do
   if (n <= 0) return;
   flushLocked();
   if (found) std::memset(found, 0, (size_t)n);
-  int n_pools = 0, only = -1;
-  for (int t = 0; t < 4; ++t)
-    if (pools_[t] && te_pool_size(pools_[t]) > 0) { ++n_pools; only = t; }
-  if (n_pools == 0) return;
-  if (n_pools == 1) {
+  const int only = onlyType(heldTypes());
+  if (only == -1) return;
+  if (only >= 0) {
     ck(te_pool_read_estimates(pools_[only], n, ids, t1, pose7, twist6, acc6, nullptr, found));
     return;
   }
+  std::vector<long long> rows[4];
+  rowsByType(n, ids, rows);
+  std::vector<uint32_t> s_ids;
+  std::vector<double> s_t1, po, tw, ac;
+  std::vector<uint8_t> fo;
   for (int t = 0; t < 4; ++t) {
-    if (!pools_[t]) continue;
-    std::vector<uint32_t> sub;
-    std::vector<long long> where;
-    std::vector<double> st1;
-    for (long long k = 0; k < n; ++k) {
-      auto it = targets_.find(ids[k]);
-      if (it == targets_.end() || it->second != t) continue;
-      sub.push_back(ids[k]);
-      where.push_back(k);
-      if (t1) st1.push_back(t1[k]);
-    }
-    if (sub.empty()) continue;
-    const long long m = (long long)sub.size();
-    std::vector<double> po((size_t)m * 7), tw((size_t)m * 6), ac((size_t)m * 6);
-    std::vector<uint8_t> fo((size_t)m);
-    ck(te_pool_read_estimates(pools_[t], m, sub.data(), t1 ? st1.data() : nullptr, po.data(), tw.data(), ac.data(), nullptr, fo.data()));
-    for (long long j = 0; j < m; ++j) {
-      const long long k = where[j];
-      if (pose7) std::memcpy(pose7 + 7 * k, &po[7 * j], 56);
-      if (twist6) std::memcpy(twist6 + 6 * k, &tw[6 * j], 48);
-      if (acc6) std::memcpy(acc6 + 6 * k, &ac[6 * j], 48);
-      if (found) found[k] = fo[j];
-    }
+    const size_t m = rows[t].size();
+    if (m == 0) continue;
+    po.resize(m * 7); tw.resize(m * 6); ac.resize(m * 6); fo.resize(m);
+    ck(te_pool_read_estimates(pools_[t], (long long)m, gatherRows<1>(ids, rows[t], s_ids), gatherRows<1>(t1, rows[t], s_t1), po.data(),
+                              tw.data(), ac.data(), nullptr, fo.data()));
+    scatterRows<7>(pose7, rows[t], po.data());
+    scatterRows<6>(twist6, rows[t], tw.data());
+    scatterRows<6>(acc6, rows[t], ac.data());
+    scatterRows<1>(found, rows[t], fo.data());
   }
 }
 
@@ -653,15 +650,12 @@ void TargetManager::log() {   // :119-123: every target publishes measurement / 
   log_n_.resize((base + 1) * m, 0);
   double t_sample = std::nan("");
   // one batched read-back per pool that holds watched ids
+  std::vector<long long> rows[4];
+  rowsByType((long long)m, log_ids_.data(), rows);
+  std::vector<uint32_t> sub;
   for (int type = 0; type < 4; ++type) {
-    if (!pools_[type]) continue;
-    std::vector<uint32_t> sub;
-    std::vector<size_t> where;
-    for (size_t j = 0; j < m; ++j) {
-      auto it = targets_.find(log_ids_[j]);
-      if (it != targets_.end() && it->second == type) { sub.push_back(log_ids_[j]); where.push_back(j); }
-    }
-    if (sub.empty()) continue;
+    if (rows[type].empty()) continue;
+    gatherRows<1>(log_ids_.data(), rows[type], sub);
     int N = 0, M = 0;
     te_model_dims(type, &N, &M);
     const long long k = (long long)sub.size();
@@ -669,7 +663,7 @@ void TargetManager::log() {   // :119-123: every target publishes measurement / 
     ck(te_pool_read_state(pools_[type], k, sub.data(), nullptr, P.data(), t.data(), nullptr, nullptr, mp.data()));
     ck(te_pool_read_estimates(pools_[type], k, sub.data(), nullptr, nullptr, tw.data(), ac.data(), pi.data(), nullptr));
     for (long long q = 0; q < k; ++q) {
-      const size_t j = where[(size_t)q];
+      const size_t j = (size_t)rows[type][(size_t)q];
       double* row = &log_rows_[(base * m + j) * 26];
       row[0] = t[(size_t)q];
       std::memcpy(row + 1, &mp[(size_t)q * 7], 7 * sizeof(double));
@@ -970,24 +964,13 @@ long long IntersectionSolver::query(long long n, const unsigned* ids, const int*
 }
 
 // the model type(s) of shard r's targets: one pool in use -> every query goes to it (the kernel finds unknown ids itself); several
-// -> a host lookup per query
+// -> the queries split by model type on the host
 void IntersectionSolver::classify(int r, long long m, const unsigned* ids) {
   Part& P = part_[(size_t)r];
   TargetManager& M = shardOf(r);
   std::lock_guard<std::recursive_mutex> lg(M.lock());
-  int n_pools = 0;
-  P.only = -1;
-  for (int t = 0; t < 4; ++t) {
-    te_pool* p = M.poolOf(t, false);
-    if (p && te_pool_size(p) > 0) { ++n_pools; P.only = t; }
-  }
-  if (n_pools <= 1) return;
-  P.only = -2;
-  P.type.resize((size_t)m);
-  for (long long j = 0; j < m; ++j) {
-    int ty;
-    P.type[(size_t)j] = M.typeOf(ids[j], ty) ? (signed char)ty : (signed char)-1;
-  }
+  P.only = onlyType(M.heldTypes());
+  if (P.only == -2) M.rowsByType(m, ids, P.rows);
 }
 
 // the streams shard r queries whose state lives on another shard, grouped by (model type, source); home_ then names r.  (A stream
@@ -996,13 +979,16 @@ void IntersectionSolver::collectMoves(int r, long long m, const int* stream) {
   Part& P = part_[(size_t)r];
   const int G = (int)part_.size();
   for (auto& v : P.moves) v.clear();
-  for (long long j = 0; j < m; ++j) {
-    const int t = P.only >= 0 ? P.only : (P.only == -2 ? P.type[(size_t)j] : -1);
-    if (t < 0) continue;
+  auto visit = [&](int t, long long j) {
     int& h = home_[(size_t)t * (size_t)n_streams_ + (size_t)stream[j]];
     if (h >= 0 && h != r) P.moves[(size_t)t * G + (size_t)h].push_back(stream[j]);
     h = r;
-  }
+  };
+  if (P.only >= 0)
+    for (long long j = 0; j < m; ++j) visit(P.only, j);
+  else if (P.only == -2)
+    for (int t = 0; t < 4; ++t)
+      for (long long j : P.rows[t]) visit(t, j);
 }
 
 long long IntersectionSolver::queryShard(int r, long long m, const unsigned* ids, const int* stream, const double* t1, const double* origin,
@@ -1023,42 +1009,29 @@ long long IntersectionSolver::queryShard(int r, long long m, const unsigned* ids
     if (conv) conv[j] = 0;
   }
   if (P.only == -1) return 0;
+  std::vector<int> by_row;   // stream NULL = the query's row
+  if (pose7 && !stream) {
+    by_row.resize((size_t)m);
+    std::iota(by_row.begin(), by_row.end(), 0);
+    stream = by_row.data();
+  }
   long long found = 0;
-  std::vector<long long> rows;
   std::vector<unsigned> s_ids;
   std::vector<int> s_stream;
-  std::vector<double> s_t1, s_origin, s_radius, s_pth, s_ath, s_delta, s_pose;
-  std::vector<unsigned char> s_conv;
+  std::vector<double> s_t1, s_origin, s_radius, s_pth, s_ath, s_delta((size_t)m), s_pose(pose7 ? 7 * (size_t)m : 0);
+  std::vector<unsigned char> s_conv(pose7 ? (size_t)m : 0);
   for (int t = 0; t < 4; ++t) {   // one sub-batch per model type
-    rows.clear();
-    for (long long j = 0; j < m; ++j)
-      if (P.type[(size_t)j] == t) rows.push_back(j);
-    const long long q = (long long)rows.size();
-    if (q == 0) continue;
-    s_ids.resize((size_t)q); s_stream.resize((size_t)q); s_t1.resize((size_t)q); s_origin.resize(3 * (size_t)q); s_radius.resize((size_t)q);
-    s_pth.resize(pos_th ? (size_t)q : 0); s_ath.resize(ang_th ? (size_t)q : 0);
-    s_delta.resize((size_t)q); s_pose.resize(pose7 ? 7 * (size_t)q : 0); s_conv.resize((size_t)q);
-    for (long long i = 0; i < q; ++i) {
-      const long long j = rows[(size_t)i];
-      s_ids[(size_t)i] = ids[j];
-      s_stream[(size_t)i] = stream ? stream[j] : (int)j;
-      s_t1[(size_t)i] = t1[j];
-      std::memcpy(&s_origin[3 * (size_t)i], origin + 3 * j, 24);
-      s_radius[(size_t)i] = radius[j];
-      if (pos_th) s_pth[(size_t)i] = pos_th[j];
-      if (ang_th) s_ath[(size_t)i] = ang_th[j];
-    }
-    const long long rc = te_isolver_query(solverFor(r, t), q, s_ids.data(), pose7 ? s_stream.data() : nullptr, s_t1.data(), s_origin.data(), s_radius.data(),
-                                          pos_th ? s_pth.data() : nullptr, ang_th ? s_ath.data() : nullptr, s_delta.data(),
-                                          pose7 ? s_pose.data() : nullptr, s_conv.data());
+    const std::vector<long long>& rows = P.rows[t];
+    if (rows.empty()) continue;
+    const long long rc = te_isolver_query(solverFor(r, t), (long long)rows.size(), gatherRows<1>(ids, rows, s_ids), gatherRows<1>(stream, rows, s_stream),
+                                          gatherRows<1>(t1, rows, s_t1), gatherRows<3>(origin, rows, s_origin), gatherRows<1>(radius, rows, s_radius),
+                                          gatherRows<1>(pos_th, rows, s_pth), gatherRows<1>(ang_th, rows, s_ath), s_delta.data(),
+                                          pose7 ? s_pose.data() : nullptr, pose7 ? s_conv.data() : nullptr);
     ck(rc);
     found += rc;
-    for (long long i = 0; i < q; ++i) {
-      const long long j = rows[(size_t)i];
-      if (delta) delta[j] = s_delta[(size_t)i];
-      if (pose7) std::memcpy(pose7 + 7 * j, &s_pose[7 * (size_t)i], 56);
-      if (conv) conv[j] = pose7 ? s_conv[(size_t)i] : 0;
-    }
+    scatterRows<1>(delta, rows, s_delta.data());
+    scatterRows<7>(pose7, rows, s_pose.data());
+    scatterRows<1>(pose7 ? conv : nullptr, rows, s_conv.data());
   }
   return found;
 }
@@ -1135,14 +1108,12 @@ long long IntersectionSolver::queryRun(long long n, const unsigned* ids, const i
   t0 = clk::now();
   long long found = 0;
   for (const Part& P : part_) found += P.found;
+  if (converged && !with_pose) std::memset(converged, 0, (size_t)n);
   sharded_->forEachShard([&](int r) {
     const Part& P = part_[(size_t)r];
-    for (size_t j = 0; j < total[(size_t)r]; ++j) {
-      const long long k = P.where[j];
-      if (delta) delta[k] = P.delta[j];
-      if (pose7) std::memcpy(pose7 + 7 * k, &P.pose[7 * j], 56);
-      if (converged) converged[k] = with_pose ? P.conv[j] : 0;
-    }
+    scatterRows<1>(delta, P.where, P.delta.data());
+    scatterRows<7>(pose7, P.where, P.pose.data());
+    scatterRows<1>(with_pose ? converged : nullptr, P.where, P.conv.data());
   });
   phase_ms_[3] += ms_since(t0);
   return found;
@@ -1172,13 +1143,14 @@ long long PoolRowMerge::run(const std::vector<TargetManager*>& shards, const std
   const int G = (int)shards.size();
   if (lists_.size() < 4 * (size_t)G) lists_.resize(4 * (size_t)G);
   int n_lists = 0, only = -1;
-  for (int r = 0; r < G; ++r)
+  for (int r = 0; r < G; ++r) {
+    const unsigned held = shards[(size_t)r]->heldTypes();
     for (int t = 0; t < 4; ++t) {
-      te_pool* p = shards[(size_t)r]->poolOf(t, false);
       List& L = lists_[(size_t)r * 4 + (size_t)t];
-      L.used = p && te_pool_size(p) > 0;
+      L.used = (held >> t) & 1u;
       if (L.used) { ++n_lists; only = r * 4 + t; }
     }
+  }
   auto run_pool = [&](int r, int t, unsigned* ids, double* val, long long* count) {
     TargetManager& M = *shards[(size_t)r];
     std::lock_guard<std::recursive_mutex> lk(M.lock());
