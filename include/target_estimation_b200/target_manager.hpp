@@ -47,10 +47,11 @@ typedef std::vector<double> VectorXd;
 class TargetManager;
 
 // The k smallest (value, id) rows of q queries over every (shard, model type) pool that holds targets: what
-// IntersectionSolver::earliestIntersections and TargetManager::nearestTargets share.  Each pool selects its own rows on the device
-// (te_pool_earliest_intersections / te_pool_nearest_targets: per query, rows by (value, id), then id 0xFFFFFFFF / value -1, and
-// a count); the host merges the lists of each query by (value, id) -- a candidate's value is a non-negative double, -0.0 ranks as
-// 0 -- and sums the counts.  When one pool holds every target its rows are the answer.  The lists' buffers only grow.
+// IntersectionSolver::earliestIntersections, TargetManager::nearestTargets and TargetManager::gatedTargets share.  Each pool selects
+// its own rows on the device (te_pool_earliest_intersections / te_pool_nearest_targets / te_pool_gated_targets: per query, rows by
+// (value, id), then id 0xFFFFFFFF / value -1, and a count); the host merges the lists of each query by (value, id) -- a candidate's
+// value is a non-negative double, -0.0 ranks as 0 -- and sums the counts.  When one pool holds every target its rows are the
+// answer.  The lists' buffers only grow.
 class PoolRowMerge {
  public:
   // one pool's rows [q][k] and counts [q]: returns < 0 on error (te_last_error())
@@ -195,6 +196,28 @@ class TargetManager {
   // negative or NaN radius is an error, +inf asks for the k nearest of all.  Returns the total count.
   virtual long long nearestTargets(long long q, const double* t1 /*[q] or NULL*/, const double* point /*[q][3]*/, const double* radius,
                                    long long k, unsigned* ids_out /*[q][k]*/, double* dist_out /*[q][k]*/, long long* count_out /*[q]*/);
+  // Gating: the k targets with the smallest Mahalanobis distance to a measured position, over every target of the manager
+  // (te_pool_gated_targets on every (shard, model type) pool that holds targets; the shards of a sharded manager run at once).  Query
+  // j = (t1[j], z[j][3], gate[j]); for target i with state x, covariance P, time t and model class (Q, R):
+  //  1. p = pose7[0:3] of getEstimatesBatch({i}, {t1[j]}) bit for bit (the position nearestTargets uses); t1 NULL: the current estimate.
+  //  2. C (3 x 3): P, Q, R are read through their upper triangle ((r, c) with r > c from (c, r)).  t1 NULL: C(a,b) = P(a,b), no
+  //     predict, no Q.  t1 given: the position block of A(tau) P A(tau)^T + Q, tau = t1[j] - t, h = (0.5*tau)*tau, every operation
+  //     rounded on its own: with the position-derivative offsets o = UV (0, 3), UA (0, 3, 6), AR (0, 6, 12), AV (0, 6) and
+  //     m[u][v] = P(o_u + a, o_v + b), rows r[v] = (m[0][v] + tau*m[1][v]) + h*m[2][v], then c = (r[0] + tau*r[1]) + h*r[2] (h terms
+  //     only with three offsets), C(a,b) = c + Q(a,b).
+  //  3. S = C + R[0:3,0:3].
+  //  4. d = p - z[j]; L00 = sqrt(S00), L10 = S10/L00, L20 = S20/L00, L11 = sqrt(S11 - L10*L10), L21 = (S21 - L20*L10)/L11,
+  //     L22 = sqrt((S22 - L20*L20) - L21*L21); w0 = d0/L00, w1 = (d1 - L10*w0)/L11, w2 = ((d2 - L20*w0) - L21*w1)/L22;
+  //     d^2 = (w0*w0 + w1*w1) + w2*w2.  A target whose factor does not exist (a radicand <= 0 or NaN) is never a candidate.
+  //  5. inside = d^2 <= gate[j]; count_out[j] = the number of targets inside; rows 0 .. min(k, count) - 1 of ids_out[j][.] /
+  //     d2_out[j][.] are those targets by (d^2, id), the other rows id 0xFFFFFFFF and d^2 -1.
+  //  6. The result does not depend on the shard count or on which pool holds a target.  Read-only; queued per-id calls are flushed
+  //     first.  Returns the total count.
+  //  7. 0 <= k <= 65536 (k == 0: counts only, ids_out / d2_out may be NULL); a negative or NaN gate is an error, +inf asks for the k
+  //     smallest distances over every target whose S has a factor.
+  // Position only, for every model: for UV / UA the filter's full innovation, for AR / AV the exact position marginal of the 6-D one.
+  virtual long long gatedTargets(long long q, const double* t1 /*[q] or NULL*/, const double* z /*[q][3]*/, const double* gate /*[q]*/,
+                                 long long k, unsigned* ids_out /*[q][k]*/, double* d2_out /*[q][k]*/, long long* count_out /*[q]*/);
   // One dense tick from host arrays, record k = the k-th target in denseIds() order (a homogeneous manager: getAvailableTargets()
   // order): no ids travel, nothing is looked up -- te_pool_tick_host: the copies, the step and the read-back of every target's
   // estimated position (est_pos_out [n][3], may be NULL: what the node broadcasts per tick, src/target_manager_ros.cpp:78-87) are
@@ -245,6 +268,7 @@ class TargetManager {
   long long updateBatchUnique(long long n, const unsigned* ids, double dt, const double* meas, const unsigned char* action);   // no id twice
   te_pool* densePool();   // the one non-empty pool of a homogeneous manager (throws otherwise)
   PoolRowMerge nearest_rows_;
+  PoolRowMerge gated_rows_;
 
   int device_;
   te_pool* pools_[4] = {nullptr, nullptr, nullptr, nullptr};
@@ -529,6 +553,8 @@ class ShardedTargetManager : public TargetManager {
   void flush() override;
   long long nearestTargets(long long q, const double* t1, const double* point, const double* radius, long long k, unsigned* ids_out,
                            double* dist_out, long long* count_out) override;   // every shard at once
+  long long gatedTargets(long long q, const double* t1, const double* z, const double* gate, long long k, unsigned* ids_out,
+                         double* d2_out, long long* count_out) override;   // every shard at once
   // dense ticks: the records are SHARD-MAJOR (denseIds(): shard 0's targets in ascending id, then shard 1's, ...); every shard's
   // slice is copied, stepped and read back by its own worker thread on its own device
   long long updateDense(double dt, const double* meas, int meas_stride, const unsigned char* action, double* est_pos_out) override;

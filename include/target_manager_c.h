@@ -88,6 +88,18 @@ void target_manager_flush(const target_manager_c* self);
  * Returns the total count, -1 on error. */
 long long target_manager_nearest(const target_manager_c* self, long long q, const double* t1, const double* point, const double* radius, long long k,
                                  unsigned int* ids_out, double* dist_out, long long* count_out);
+/* Gating: the k targets with the smallest Mahalanobis distance to a measured position (TargetManager::gatedTargets, whose comment
+ * states the contract operation by operation), on every handle: plain, on a device, sharded, tick and sharded tick.  Query j = t1[j]
+ * (t1 NULL = current estimates and covariances), z[j][3], gate[j].  A target's position p is pose7[0:3] of
+ * target_manager_get_estimates_batch at t1[j], bit for bit; its position covariance C is the position block of P (t1 NULL) or of the
+ * predict step A(tau) P A(tau)^T + Q to t1[j]; S = C + R[0:3,0:3]; d^2 = (p - z)^T S^-1 (p - z) through the Cholesky factor of S,
+ * every operation rounded on its own; inside = d^2 <= gate[j], and a target whose S has no factor is never inside.  count_out[j] =
+ * the number of targets inside; rows 0 .. min(k, count_out[j]) - 1 of ids_out[j][k] / d2_out[j][k] are those targets by (d^2, id),
+ * the other rows id 0xFFFFFFFF and d^2 -1.  Read-only.  0 <= k <= 65536 (k == 0: counts only, ids_out / d2_out may be NULL); the
+ * arrays may be NULL only when q == 0; a negative or NaN gate is an error, +inf asks for the k smallest distances of all.  The pose
+ * of a returned target is target_manager_get_estimates_batch(ids, t1).  Returns the total count, -1 on error. */
+long long target_manager_gated(const target_manager_c* self, long long q, const double* t1, const double* z, const double* gate, long long k,
+                               unsigned int* ids_out, double* d2_out, long long* count_out);
 
 /* ---- all GPUs of the box behind one handle (BASELINE.json north_star: targets shard by id, no collective on the hot path) ----
  * n_shards TargetManagers, shard r on CUDA device devices[r] (NULL = devices 0 .. n_shards-1), owner(id) = id mod n_shards.  The

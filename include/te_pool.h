@@ -257,6 +257,36 @@ long long te_pool_earliest_intersections(te_pool* p, long long q, const double* 
  * radius is an error (radius = +inf: plain k nearest).  Every model type runs the kernels.  Synchronous.  Returns the total count. */
 long long te_pool_nearest_targets(te_pool* p, long long q, const double* t1 /*[q] or NULL*/, const double* point /*[q][3]*/, const double* radius,
                                   long long k, uint32_t* ids_out /*[q][k]*/, double* dist_out /*[q][k]*/, long long* count_out /*[q]*/);
+/* Gating: the k targets with the smallest Mahalanobis distance to a measured position, over every target of the pool (read-only).
+ * Query j = (t1[j], z[j][3], gate[j]), host arrays.  For query j and target i, with state x, covariance P, time t, model class
+ * (Q, R) and state layout of kinematic block size B:
+ *  1. Position: p = pose7[0:3] of te_pool_read_estimates at t1[j], bit for bit (what te_pool_nearest_targets uses); t1 NULL: the
+ *     current estimate.
+ *  2. Position covariance C (3 x 3).  P, Q and R are always read through their upper triangle: entry (r, c) with r > c is taken
+ *     from (c, r) (what the packed kernels keep current).
+ *     t1 NULL: C(a,b) = P(a,b); no predict step, no Q.
+ *     t1 given: C = the position block of the predict step A(tau) P A(tau)^T + Q with tau = t1[j] - t and h = (0.5*tau)*tau, in
+ *     the operation order of predict_kinematic, every operation rounded on its own (no contraction).  Position-derivative offsets
+ *     o: UV (0, 3), UA (0, 3, 6), AR (0, 6, 12), AV (0, 6) -- the position rows of AV's EKF Jacobian are [I 0 tau*I 0], and the
+ *     position block of F P F^T depends only on those rows.  m[u][v] = P(o_u + a, o_v + b); rows first:
+ *     r[v] = (m[0][v] + tau*m[1][v]) + h*m[2][v]; then columns: c = (r[0] + tau*r[1]) + h*r[2] (the h terms only with three
+ *     offsets); C(a,b) = c + Q(a,b).
+ *  3. Innovation covariance: S = C + R[0:3,0:3], the position rows and columns of the class's M x M R.
+ *  4. Distance: d = p - z[j], rounded per component.  Cholesky factor, in this order: L00 = sqrt(S00); L10 = S10/L00;
+ *     L20 = S20/L00; L11 = sqrt(S11 - L10*L10); L21 = (S21 - L20*L10)/L11; L22 = sqrt((S22 - L20*L20) - L21*L21).  Forward
+ *     solve: w0 = d0/L00; w1 = (d1 - L10*w0)/L11; w2 = ((d2 - L20*w0) - L21*w1)/L22.  d^2 = (w0*w0 + w1*w1) + w2*w2.  A target
+ *     whose factor does not exist (any radicand <= 0 or NaN) is never a candidate.
+ *  5. Selection: a target is inside when d^2 <= gate[j] (the boundary counts).  count_out[j] = the number of targets inside; rows
+ *     0 .. min(k, count) - 1 of ids_out[j][.] / d2_out[j][.] hold those targets ordered by (d^2, id); the remaining rows hold id
+ *     0xFFFFFFFF and d^2 -1.
+ *  6. The query is read-only.  Returns the total count.
+ *  7. Argument rules as te_pool_nearest_targets with gate in place of radius: 0 <= k <= 65536 (k == 0: counts only, ids_out /
+ *     d2_out may then be NULL); a negative or NaN gate is an error, +inf asks for the k smallest distances over every target whose
+ *     S has a factor.
+ * Gating is on position only, for every model: for UV / UA that is the filter's full innovation, for AR / AV the exact position
+ * marginal of the 6-D innovation.  Synchronous. */
+long long te_pool_gated_targets(te_pool* p, long long q, const double* t1 /*[q] or NULL*/, const double* z /*[q][3]*/, const double* gate,
+                                long long k, uint32_t* ids_out /*[q][k]*/, double* d2_out /*[q][k]*/, long long* count_out /*[q]*/);
 
 /* Dense device-resident form: one query per slot (query k = slot k = solver stream k; needs n_streams >= pool size).
  * dev_t1 NULL = each target's own time; dev_delta / dev_pose7 / dev_converged may be NULL.  Asynchronous. */

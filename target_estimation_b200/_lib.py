@@ -79,6 +79,7 @@ SIGNATURES = {
     "te_isolver_query_dense": (_i, [_p, _p, _p, _p, _d, _d, _p, _p, _p]),
     "te_pool_earliest_intersections": (_ll, [_p, _ll, _p, _p, _p, _ll, _p, _p, _p]),
     "te_pool_nearest_targets": (_ll, [_p, _ll, _p, _p, _p, _ll, _p, _p, _p]),
+    "te_pool_gated_targets": (_ll, [_p, _ll, _p, _p, _p, _ll, _p, _p, _p]),
     "te_isolver_move_streams": (_i, [_p, _p, _ll, _p]),
     "te_pool_tick_host_async": (_i, [_p, _d, _p, _i, _p, _i, _p]),
     "te_pool_tick_host_wait": (_i, [_p, _i]),

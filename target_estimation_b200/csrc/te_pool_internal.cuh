@@ -4,8 +4,8 @@
 //   te_step.cu     step-kernel launch policy and the stepping entry points (dense / replay / host / by id / fused expiry)
 //   te_mailbox.cu  device-resident mailboxes (the node loop)
 //   te_isolver.cu  batched IntersectionSolver
-//   te_sweep.cu    the k earliest sphere intercepts and the k nearest targets over every target of a pool
-//                  (te_pool_earliest_intersections, te_pool_nearest_targets)
+//   te_sweep.cu    the k earliest sphere intercepts, the k nearest targets and the k gated targets over every target of a pool
+//                  (te_pool_earliest_intersections, te_pool_nearest_targets, te_pool_gated_targets)
 //   te_group.cu    several pools on several devices: the NCCL all-gather of estimate records
 #pragma once
 #include <algorithm>

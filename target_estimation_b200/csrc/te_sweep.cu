@@ -1,9 +1,10 @@
-// te_sweep.cu -- te_pool_earliest_intersections and te_pool_nearest_targets of include/te_pool.h: the k earliest sphere intercepts
-// and the k nearest targets inside a sphere, over every target of a pool, selected on the device (kernels in te_sweep.cuh).  Both
-// produce one key per (query, slot) and share the selection below.  Only q x k rows and q counts cross PCIe.
+// te_sweep.cu -- te_pool_earliest_intersections, te_pool_nearest_targets and te_pool_gated_targets of include/te_pool.h: the k
+// earliest sphere intercepts, the k nearest targets inside a sphere and the k targets of smallest Mahalanobis distance inside a gate,
+// over every target of a pool, selected on the device (kernels in te_sweep.cuh).  All three produce one key per (query, slot) and
+// share the selection below.  Only q x k rows and q counts cross PCIe.
 #include <cub/device/device_segmented_sort.cuh>
 
-#include "te_nearest_args.h"
+#include "te_query_args.h"
 #include "te_pool_internal.cuh"
 #include "te_sweep.cuh"
 
@@ -110,6 +111,21 @@ unsigned long long bits_of(double v) {
   std::memcpy(&b, &v, 8);
   return b;
 }
+
+// gate_prep_kernel of the pool's model over every slot: t1 NULL = no predict
+template <int TYPE>
+void launch_gate_prep_t(te_pool* p, int n, const double* t1, double* chol) {
+  const Buf& b = p->buf[p->cur];
+  te::gate_prep_kernel<TYPE><<<cdiv(n, 256), 256, 0, p->stream>>>(n, b.tiles, b.cold.cls, p->dQ, p->dR, t1 ? 1 : 0, t1 ? *t1 : 0.0, chol);
+}
+void launch_gate_prep(te_pool* p, int n, const double* t1, double* chol) {
+  switch (p->model) {
+    case te::UNIFORM_VELOCITY: launch_gate_prep_t<te::UNIFORM_VELOCITY>(p, n, t1, chol); break;
+    case te::UNIFORM_ACCELERATION: launch_gate_prep_t<te::UNIFORM_ACCELERATION>(p, n, t1, chol); break;
+    case te::ANGULAR_VELOCITIES: launch_gate_prep_t<te::ANGULAR_VELOCITIES>(p, n, t1, chol); break;
+    default: launch_gate_prep_t<te::ANGULAR_RATES>(p, n, t1, chol); break;
+  }
+}
 }  // namespace
 
 extern "C" long long te_pool_earliest_intersections(te_pool* p, long long q, const double* t1, const double* origin, const double* radius,
@@ -148,7 +164,7 @@ extern "C" long long te_pool_earliest_intersections(te_pool* p, long long q, con
 extern "C" long long te_pool_nearest_targets(te_pool* p, long long q, const double* t1, const double* point, const double* radius, long long k,
                                              uint32_t* ids_out, double* dist_out, long long* count_out) {
   return guarded_ll(p, [&]() -> long long {
-    te::check_nearest_args(q, point, radius, k, ids_out, dist_out, count_out);
+    te::check_query_args(te::NEAREST_ARGS, q, point, radius, k, ids_out, dist_out, count_out);
     if (q == 0) return 0;
     const long long n = p->n;
     if (n == 0) return no_rows(q, k, ids_out, dist_out, count_out);
@@ -169,6 +185,37 @@ extern "C" long long te_pool_nearest_targets(te_pool* p, long long q, const doub
           gathered_t1 = t1 ? bits_of(t1[j]) : 0;
         }
         te::near_key_kernel<<<cdiv(n, 256), 256, 0, p->stream>>>((int)n, pose7, point[3 * j], point[3 * j + 1], point[3 * j + 2], radius[j],
+                                                                 keys + (size_t)c * n, inside + c);
+      }
+    });
+  });
+}
+
+extern "C" long long te_pool_gated_targets(te_pool* p, long long q, const double* t1, const double* z, const double* gate, long long k,
+                                           uint32_t* ids_out, double* d2_out, long long* count_out) {
+  return guarded_ll(p, [&]() -> long long {
+    te::check_query_args(te::GATE_ARGS, q, z, gate, k, ids_out, d2_out, count_out);
+    if (q == 0) return 0;
+    const long long n = p->n;
+    if (n == 0) return no_rows(q, k, ids_out, d2_out, count_out);
+    // positions as te_pool_nearest_targets gathers them; consecutive queries at the same t1 (every query when t1 is NULL) share one
+    // gather and one factor of S per slot
+    double* pose7 = p->arena.get_n<double>((size_t)n * 7);
+    double* chol = p->arena.get_n<double>((size_t)n * 6);
+    double* b_t1 = t1 ? p->arena.get_n<double>((size_t)n) : nullptr;
+    bool prepared = false;
+    unsigned long long prepared_t1 = 0;
+    return select_rows(p, q, k, ids_out, d2_out, count_out, [&](long long j0, int nq, unsigned long long* keys, unsigned long long* inside) {
+      for (int c = 0; c < nq; ++c) {
+        const long long j = j0 + c;
+        if (!prepared || (t1 && bits_of(t1[j]) != prepared_t1)) {
+          if (t1) te::fill_dt_kernel<<<cdiv(n, 256), 256, 0, p->stream>>>(b_t1, (int)n, t1[j]);
+          launch_gather_estimates(p, nullptr, n, b_t1, pose7, nullptr, nullptr, nullptr, nullptr, 0);
+          launch_gate_prep(p, (int)n, t1 ? t1 + j : nullptr, chol);
+          prepared = true;
+          prepared_t1 = t1 ? bits_of(t1[j]) : 0;
+        }
+        te::gate_key_kernel<<<cdiv(n, 256), 256, 0, p->stream>>>((int)n, pose7, chol, z[3 * j], z[3 * j + 1], z[3 * j + 2], gate[j],
                                                                  keys + (size_t)c * n, inside + c);
       }
     });

@@ -1,8 +1,9 @@
-// te_sweep.cuh -- sm_100a kernels of te_pool_earliest_intersections and te_pool_nearest_targets (te_sweep.cu): for each of a chunk
-// of queries, the k targets of the pool with the smallest key, selected on the device without sorting the pool.
-//   keys            per query, one 64-bit key per slot, ~0 for a slot that is no candidate; candidates are counted.  Two producers:
-//                   sweep_key_kernel (the bits of isolver_kernel's delta for a hit, see sweep_broadcast_kernel) and near_key_kernel
-//                   (the bits of the distance for a target inside the query sphere)
+// te_sweep.cuh -- sm_100a kernels of te_pool_earliest_intersections, te_pool_nearest_targets and te_pool_gated_targets (te_sweep.cu):
+// for each of a chunk of queries, the k targets of the pool with the smallest key, selected on the device without sorting the pool.
+//   keys            per query, one 64-bit key per slot, ~0 for a slot that is no candidate; candidates are counted.  Three producers:
+//                   sweep_key_kernel (the bits of isolver_kernel's delta for a hit, see sweep_broadcast_kernel), near_key_kernel
+//                   (the bits of the distance for a target inside the query sphere) and gate_key_kernel (the bits of the Mahalanobis
+//                   d^2 for a target inside the gate)
 //   hist / select   radix select over the 96-bit composite (rank(key), slot) in eight 12-bit digits: one histogram of the keys that
 //                   still match the selected prefix, then the digit bucket that holds the k-th; refinement stops as soon as that
 //                   bucket is small (usually after the second digit)
@@ -101,6 +102,105 @@ static __global__ void near_key_kernel(int n, const double* __restrict__ pose7, 
     const double dist = __dsqrt_rn(__dadd_rn(__dadd_rn(__dmul_rn(dx, dx), __dmul_rn(dy, dy)), __dmul_rn(dz, dz)));
     in = dist <= radius;
     keys[s] = in ? (unsigned long long)__double_as_longlong(dist) : SWEEP_MISS;
+  }
+  const unsigned b = __ballot_sync(0xffffffffu, in);
+  if ((threadIdx.x & 31) == 0 && b) atomicAdd(inside, (unsigned long long)__popc(b));
+}
+
+// The gating query (te_pool_gated_targets) splits its work in two: gate_prep_kernel, once per run of queries at the same t1, turns
+// every slot's covariance into the Cholesky factor of its position innovation covariance S; gate_key_kernel, once per query, turns
+// the slot's position (pose7 of gather_estimates_kernel) and that factor into the Mahalanobis d^2.  Every operation is rounded on
+// its own (__dadd_rn / __dmul_rn / __ddiv_rn / __dsqrt_rn) in the order of the contract in include/te_pool.h, so numpy reproduces
+// every bit; left to ptxas, the multiplies and adds would be contracted into FMAs according to the surrounding code.
+
+// upper-triangle read of a symmetric matrix: entry (r, c) with r > c comes from (c, r), which is what the packed kernels keep current
+__device__ __forceinline__ int gate_upper(int r, int c, int n) { return r <= c ? r * n + c : c * n + r; }
+
+// per slot: the six entries L00, L10, L20, L11, L21, L22 of the factor of S = C + R[0:3, 0:3] into chol[6 * slot], L00 = NaN when
+// the factor does not exist (a radicand <= 0 or NaN), which makes every d^2 of the slot NaN.  use_t1 == 0: C = P[0:3, 0:3].
+// use_t1 != 0: C = the position block of A(tau) P A(tau)^T + Q with tau = t1 - t, evaluated like predict_kinematic (rows, then
+// columns) over the position-derivative offsets: (0, 3) UV, (0, 3, 6) UA, (0, 6, 12) AR, (0, 6) AV -- the position rows of
+// predict_av's Jacobian are [I 0 tau*I 0], so the position block of F P F^T depends on those rows only.  One thread per slot: the
+// 32 lanes of a warp read one tile, each field of it one 256 B segment.
+template <int TYPE>
+__global__ void __launch_bounds__(256) gate_prep_kernel(int n, const double* __restrict__ tiles, const uint16_t* __restrict__ cls,
+                                                        const double* __restrict__ Qtab, const double* __restrict__ Rtab, int use_t1,
+                                                        double t1, double* __restrict__ chol) {
+  using MT = Model<TYPE>;
+  using LY = Layout<TYPE>;
+  constexpr int N = MT::N, M = MT::M;
+  constexpr int NO = (TYPE == UNIFORM_VELOCITY || TYPE == ANGULAR_VELOCITIES) ? 2 : 3;   // offsets
+  constexpr int OS = (TYPE == UNIFORM_VELOCITY || TYPE == UNIFORM_ACCELERATION) ? 3 : 6;  // offset stride
+  const int s = blockIdx.x * blockDim.x + threadIdx.x;
+  if (s >= n) return;
+  const double* rec = tiles + (size_t)(s / TILE) * LY::TILE_DOUBLES + (s % TILE);
+  const int c = (int)cls[s];
+  const double* Q = Qtab + (size_t)c * N * N;
+  const double* R = Rtab + (size_t)c * M * M;
+  double tau = 0.0, h = 0.0;
+  if (use_t1) {
+    tau = __dsub_rn(t1, rec[LY::F_T * TILE]);
+    h = __dmul_rn(__dmul_rn(0.5, tau), tau);
+  }
+  auto P = [&](int r, int cc) { return rec[(LY::F_P + gate_upper(r, cc, N)) * TILE]; };
+  double S[3][3];   // the lower triangle (a >= b) is what the factor reads
+#pragma unroll
+  for (int a = 0; a < 3; ++a)
+#pragma unroll
+    for (int b = 0; b <= a; ++b) {
+      double C;
+      if (!use_t1) {
+        C = P(a, b);
+      } else {
+        double r[NO];
+#pragma unroll
+        for (int v = 0; v < NO; ++v) {
+          r[v] = __dadd_rn(P(a, v * OS + b), __dmul_rn(tau, P(OS + a, v * OS + b)));
+          if constexpr (NO == 3) r[v] = __dadd_rn(r[v], __dmul_rn(h, P(2 * OS + a, v * OS + b)));
+        }
+        C = __dadd_rn(r[0], __dmul_rn(tau, r[1]));
+        if constexpr (NO == 3) C = __dadd_rn(C, __dmul_rn(h, r[NO - 1]));
+        C = __dadd_rn(C, __ldg(&Q[gate_upper(a, b, N)]));
+      }
+      S[a][b] = __dadd_rn(C, __ldg(&R[gate_upper(a, b, M)]));
+    }
+  const double l00 = __dsqrt_rn(S[0][0]);
+  const double l10 = __ddiv_rn(S[1][0], l00);
+  const double l20 = __ddiv_rn(S[2][0], l00);
+  const double rad1 = __dsub_rn(S[1][1], __dmul_rn(l10, l10));
+  const double l11 = __dsqrt_rn(rad1);
+  const double l21 = __ddiv_rn(__dsub_rn(S[2][1], __dmul_rn(l20, l10)), l11);
+  const double rad2 = __dsub_rn(__dsub_rn(S[2][2], __dmul_rn(l20, l20)), __dmul_rn(l21, l21));
+  const double l22 = __dsqrt_rn(rad2);
+  const bool ok = S[0][0] > 0.0 && rad1 > 0.0 && rad2 > 0.0;   // false for NaN too
+  double* o = chol + 6 * (size_t)s;
+  o[0] = ok ? l00 : __longlong_as_double(0x7ff8000000000000ll);
+  o[1] = l10;
+  o[2] = l20;
+  o[3] = l11;
+  o[4] = l21;
+  o[5] = l22;
+}
+
+// position (pose7 as in near_key_kernel) and factor -> key: the bits of d^2 = (w0^2 + w1^2) + w2^2, w = L^-1 (p - z) by forward
+// substitution, for a target inside the gate (d^2 <= gate; NaN -- no factor -- never is), SWEEP_MISS otherwise; inside targets
+// counted.  d^2 >= +0 always, so its bits order like its value.
+static __global__ void gate_key_kernel(int n, const double* __restrict__ pose7, const double* __restrict__ chol, double zx, double zy,
+                                       double zz, double gate, unsigned long long* __restrict__ keys,
+                                       unsigned long long* __restrict__ inside) {
+  const int s = blockIdx.x * blockDim.x + threadIdx.x;
+  bool in = false;
+  if (s < n) {
+    const double* L = chol + 6 * (size_t)s;
+    const double d0 = __dsub_rn(pose7[7 * (size_t)s], zx);
+    const double d1 = __dsub_rn(pose7[7 * (size_t)s + 1], zy);
+    const double d2 = __dsub_rn(pose7[7 * (size_t)s + 2], zz);
+    const double w0 = __ddiv_rn(d0, L[0]);
+    const double w1 = __ddiv_rn(__dsub_rn(d1, __dmul_rn(L[1], w0)), L[3]);
+    const double w2 = __ddiv_rn(__dsub_rn(__dsub_rn(d2, __dmul_rn(L[2], w0)), __dmul_rn(L[4], w1)), L[5]);
+    const double m2 = __dadd_rn(__dadd_rn(__dmul_rn(w0, w0), __dmul_rn(w1, w1)), __dmul_rn(w2, w2));
+    in = m2 <= gate;
+    keys[s] = in ? (unsigned long long)__double_as_longlong(m2) : SWEEP_MISS;
   }
   const unsigned b = __ballot_sync(0xffffffffu, in);
   if ((threadIdx.x & 31) == 0 && b) atomicAdd(inside, (unsigned long long)__popc(b));

@@ -11,7 +11,7 @@
 #include <stdexcept>
 #include <thread>
 
-#include "../csrc/te_nearest_args.h"
+#include "../csrc/te_query_args.h"
 #include "rows.hpp"
 #include "target_estimation_b200/target_manager.hpp"
 
@@ -318,7 +318,7 @@ void ShardedTargetManager::getEstimatesBatch(long long n, const unsigned* ids, c
 
 long long ShardedTargetManager::nearestTargets(long long q, const double* t1, const double* point, const double* radius, long long k,
                                                unsigned* ids_out, double* dist_out, long long* count_out) {
-  te::check_nearest_args(q, point, radius, k, ids_out, dist_out, count_out);
+  te::check_query_args(te::NEAREST_ARGS, q, point, radius, k, ids_out, dist_out, count_out);
   std::lock_guard<std::recursive_mutex> lg(target_lock_);
   if (q == 0) return 0;
   flush();
@@ -330,6 +330,20 @@ long long ShardedTargetManager::nearestTargets(long long q, const double* t1, co
         return te_pool_nearest_targets(p, q, t1, point, radius, k, ids, dist, count);
       },
       ids_out, dist_out, count_out);
+}
+
+long long ShardedTargetManager::gatedTargets(long long q, const double* t1, const double* z, const double* gate, long long k,
+                                             unsigned* ids_out, double* d2_out, long long* count_out) {
+  te::check_query_args(te::GATE_ARGS, q, z, gate, k, ids_out, d2_out, count_out);
+  std::lock_guard<std::recursive_mutex> lg(target_lock_);
+  if (q == 0) return 0;
+  flush();
+  std::vector<TargetManager*> shards;
+  for (auto& s : shard_) shards.push_back(s.get());
+  return gated_rows_.run(
+      shards, [this](const std::function<void(int)>& f) { forEachShard(f); }, q, k,
+      [&](te_pool* p, unsigned* ids, double* d2, long long* count) { return te_pool_gated_targets(p, q, t1, z, gate, k, ids, d2, count); },
+      ids_out, d2_out, count_out);
 }
 
 // ---- dense ticks: shard-major records, every shard's slice on its own device at once ---------------------------------------------

@@ -15,7 +15,7 @@
 #include <stdexcept>
 #include <unordered_set>
 
-#include "../csrc/te_nearest_args.h"
+#include "../csrc/te_query_args.h"
 #include "rows.hpp"
 
 namespace target_estimation_b200 {
@@ -1217,7 +1217,7 @@ long long PoolRowMerge::run(const std::vector<TargetManager*>& shards, const std
 
 long long TargetManager::nearestTargets(long long q, const double* t1, const double* point, const double* radius, long long k,
                                         unsigned* ids_out, double* dist_out, long long* count_out) {
-  te::check_nearest_args(q, point, radius, k, ids_out, dist_out, count_out);
+  te::check_query_args(te::NEAREST_ARGS, q, point, radius, k, ids_out, dist_out, count_out);
   std::lock_guard<std::recursive_mutex> lg(target_lock_);
   if (q == 0) return 0;
   flushLocked();
@@ -1227,6 +1227,18 @@ long long TargetManager::nearestTargets(long long q, const double* t1, const dou
         return te_pool_nearest_targets(p, q, t1, point, radius, k, ids, dist, count);
       },
       ids_out, dist_out, count_out);
+}
+
+long long TargetManager::gatedTargets(long long q, const double* t1, const double* z, const double* gate, long long k, unsigned* ids_out,
+                                      double* d2_out, long long* count_out) {
+  te::check_query_args(te::GATE_ARGS, q, z, gate, k, ids_out, d2_out, count_out);
+  std::lock_guard<std::recursive_mutex> lg(target_lock_);
+  if (q == 0) return 0;
+  flushLocked();
+  return gated_rows_.run(
+      {this}, [](const std::function<void(int)>& f) { f(0); }, q, k,
+      [&](te_pool* p, unsigned* ids, double* d2, long long* count) { return te_pool_gated_targets(p, q, t1, z, gate, k, ids, d2, count); },
+      ids_out, d2_out, count_out);
 }
 
 // ----------------------------------------------------------------------------------------------

@@ -190,6 +190,13 @@ long long target_manager_nearest(const target_manager_c* self, long long q, cons
     return M(self)->nearestTargets(q, t1, point, radius, k, ids_out, dist_out, count_out);
   });
 }
+long long target_manager_gated(const target_manager_c* self, long long q, const double* t1, const double* z, const double* gate, long long k,
+                               unsigned int* ids_out, double* d2_out, long long* count_out) {
+  return guard(-1LL, [&] {
+    if (!self) throw std::invalid_argument("null manager");
+    return M(self)->gatedTargets(q, t1, z, gate, k, ids_out, d2_out, count_out);
+  });
+}
 const char* target_manager_last_error(void) { return g_err.c_str(); }
 
 // ---- IntersectionSolver -------------------------------------------------------------------------------------------

@@ -37,6 +37,7 @@ _SIG = {
     "target_manager_get_state": (_i, [_p, _u, _p, _p, _p]),
     "target_manager_flush": (None, [_p]),
     "target_manager_nearest": (_ll, [_p, _ll, _p, _p, _p, _ll, _p, _p, _p]),
+    "target_manager_gated": (_ll, [_p, _ll, _p, _p, _p, _ll, _p, _p, _p]),
     "target_manager_last_error": (C.c_char_p, []),
     "target_manager_watch": (None, [_p, _ll, _p, _ll]),
     "target_manager_log_samples": (_ll, [_p]),
@@ -230,6 +231,21 @@ class TargetManagerC:
         if int(clib.target_manager_nearest(self.h, q, _ptr(t1), _ptr(point), _ptr(radius), k, _ptr(ids), _ptr(dist), _ptr(count))) < 0:
             raise RuntimeError(clib.target_manager_last_error().decode())
         return count, ids, dist
+
+    def gated(self, t1, z, gate, k):
+        """gating: the k targets of smallest Mahalanobis d^2 to a measured position, query j = (t1[j], z[j], gate[j]); t1 (None =
+        current estimates and covariances) and gate broadcast to q = len(z).  Returns (count [q], ids [q][k], d2 [q][k]): rows past
+        min(k, count[j]) are id 0xFFFFFFFF and d2 -1.  The pose of a returned target is get_estimates_batch(ids, t1)."""
+        z = np.ascontiguousarray(z, dtype=np.float64).reshape(-1, 3)
+        q, k = z.shape[0], int(k)
+        t1 = np.ascontiguousarray(np.broadcast_to(t1, (q,)), dtype=np.float64) if t1 is not None else None
+        gate = np.ascontiguousarray(np.broadcast_to(gate, (q,)), dtype=np.float64)
+        count = np.zeros(q, dtype=np.int64)
+        ids = np.zeros((q, max(k, 0)), dtype=np.uint32)
+        d2 = np.zeros((q, max(k, 0)))
+        if int(clib.target_manager_gated(self.h, q, _ptr(t1), _ptr(z), _ptr(gate), k, _ptr(ids), _ptr(d2), _ptr(count))) < 0:
+            raise RuntimeError(clib.target_manager_last_error().decode())
+        return count, ids, d2
 
 
 class ShardedManagerC(TargetManagerC):

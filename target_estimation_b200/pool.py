@@ -326,6 +326,21 @@ class TargetPool:
         check(lib.te_pool_nearest_targets(self._h, q, _ptr(t1), _ptr(point), _ptr(radius), k, _ptr(ids), _ptr(dist), _ptr(count)))
         return count, ids, dist
 
+    # -- gating: the k smallest Mahalanobis distances to a measured position (te_pool_gated_targets) --
+    def gated_targets(self, t1, z, gate, k):
+        """query j = (t1[j], z[j], gate[j]); t1 (None = current estimates and covariances) and gate broadcast to q = len(z).  Returns
+        (count [q], ids [q][k], d2 [q][k]) with the targets inside each gate by (d2, id) first and rows of id 0xFFFFFFFF / d2 -1 after
+        them."""
+        z = _np(z, np.float64).reshape(-1, 3)
+        q, k = z.shape[0], int(k)
+        t1 = _np(np.broadcast_to(t1, (q,)), np.float64) if t1 is not None else None
+        gate = _np(np.broadcast_to(gate, (q,)), np.float64)
+        count = np.zeros(q, dtype=np.int64)
+        ids = np.zeros((q, max(k, 0)), dtype=np.uint32)
+        d2 = np.zeros((q, max(k, 0)))
+        check(lib.te_pool_gated_targets(self._h, q, _ptr(t1), _ptr(z), _ptr(gate), k, _ptr(ids), _ptr(d2), _ptr(count)))
+        return count, ids, d2
+
 
 class IntersectionSolver:
     """Batched IntersectionSolver: n_streams independent reference solver objects (include/te_pool.h)."""
