@@ -80,7 +80,9 @@ __global__ void __launch_bounds__(WARPS * 32, 1) kf_step_av_direct_kernel(const 
 // launch (te_pool_step_dense_ticks): the target stays in registers for all its ticks.
 // MULTI: the replay / live instantiation (n_ticks > 1 or a tick gate); the single-tick instantiation carries none of its code (its
 // registers cost the dense tick a spill).
-template <int TYPE, int WARPS, int MIN_CTAS, bool MULTI = false>
+// AXIS: the axis-blocked step (te_kin_sym.cuh) of a packed pool in which no class couples the axes: UA moves 29 of its 56 packed
+// fields, UV 17 of 29.
+template <int TYPE, int WARPS, int MIN_CTAS, bool MULTI = false, bool AXIS = false>
 __global__ void __launch_bounds__(WARPS * 32, MIN_CTAS) kf_step_kin_direct_kernel(const StepArgs a) {
   using MT = Model<TYPE>;
   using LY = Layout<TYPE>;
@@ -119,7 +121,7 @@ __global__ void __launch_bounds__(WARPS * 32, MIN_CTAS) kf_step_kin_direct_kerne
     if (MULTI) {
       if (!valid) continue;
       // a lane whose actions are all ACT_NONE still goes through load / store: cheaper than a second pass to find out
-      KinSym<TYPE> ks;
+      KinSym<TYPE, AXIS> ks;
       ks.load(in);
       if (a.tick_gate) {
         // live launch: the target stays in registers while its ticks arrive one by one -- a tick costs neither a launch nor a
@@ -272,10 +274,10 @@ __global__ void __launch_bounds__(WARPS * 32, MIN_CTAS) kf_step_kin_direct_kerne
 #pragma unroll
         for (int k = 0; k < 3; ++k) meas[k] = __ldg(mp + k);
       }
-      KinSym<TYPE> ks;
+      KinSym<TYPE, AXIS> ks;
       ks.load(in);
       ks.tick(act, dt, meas, Q, R);
-      ks.store(out, a.packed != 0);
+      ks.store(out, a.packed != 0, AXIS && a.dst_tiles);
       if (a.pos_out) {
 #pragma unroll
         for (int k = 0; k < 3; ++k) a.pos_out[(size_t)slot * 3 + k] = ks.x[k];

@@ -10,12 +10,20 @@
 //       reference's order; the mirrored position (c, r) is the transposed macro matrix and is not computed
 //   update  (src/kalman.cpp:90-95) with C = [I3 0]:  S = P'[0:3,0:3] + R = L L^T,  Z = L^-1 P'[0:3,:],
 //       x += Z^T L^-1 (y - x'[0:3]),  P = P' - Z^T Z   ( = (I - K C) P' with K = P'[:,0:3] S^-1 )
+//
+// AXIS: the axis-blocked form, for pools in which no registered class couples the x / y / z axes (te_pool::all_axis).  Index
+// i = a * 3 + r of the state belongs to axis r = i % 3; every covariance entry (i, j) with i % 3 != j % 3 is then exactly +-0 in
+// HBM on every tick (DESIGN.md section 2), so the lane loads and stores only x, the in-axis entries of the upper triangle (3 NB x
+// NB blocks: UV 9 of 21, UA 18 of 45), t and n_meas.  tick() runs the same operations in the same order, minus the terms that
+// are structurally zero: the off-diagonal blocks of the predict, the off-diagonal entries of S and L (S is diagonal), and every
+// term of u, Z, x and P that carries one of them.  Each dropped term is a +-0 product added to a value, so the kept results
+// are bit for bit those of the full form (tests/test_gpu_axis_blocks.py).
 #pragma once
 #include "te_av_sym.cuh"
 
 namespace te {
 
-template <int TYPE>
+template <int TYPE, bool AXIS = false>
 struct KinSym {
   using MT = Model<TYPE>;
   using LY = Layout<TYPE>;
@@ -25,6 +33,8 @@ struct KinSym {
   SymP<N> P;
   double t;
   long long nm;
+  // does entry (i, j) carry information?  (the blocked form never touches the others)
+  static __device__ __forceinline__ constexpr bool kept(int i, int j) { return !AXIS || i % B == j % B; }
 
   __device__ __forceinline__ void load(const double* in) {
 #pragma unroll
@@ -35,7 +45,7 @@ struct KinSym {
     for (int i = 0; i < N; ++i)
 #pragma unroll
       for (int j = 0; j < N; ++j)
-        if (i <= j) P(i, j) = in[(LY::F_P + i * N + j) * TILE];
+        if (i <= j && kept(i, j)) P(i, j) = in[(LY::F_P + i * N + j) * TILE];
   }
 
   // one TargetManager::update(id, dt[, meas]) of this lane's target
@@ -55,7 +65,7 @@ struct KinSym {
     for (int r = 0; r < B; ++r) {
 #pragma unroll
       for (int c = 0; c < B; ++c) {
-        if (r <= c) {
+        if (r <= c && (!AXIS || r == c)) {   // block (r, c) couples axis r with axis c
           double m[NB][NB];
 #pragma unroll
           for (int a = 0; a < NB; ++a)
@@ -94,39 +104,47 @@ struct KinSym {
       for (int i = 0; i < M; ++i)
 #pragma unroll
         for (int j = 0; j < M; ++j)
-          if (j <= i) ch.at(i, j) = P(j, i) + __ldg(&R[i * M + j]);
-      ch.factor();
+          if (j <= i && kept(i, j)) ch.at(i, j) = P(j, i) + __ldg(&R[i * M + j]);
+      if (AXIS) {   // S diagonal: factor()'s d of column k is S_kk, its inverse square root the only operation left
+#pragma unroll
+        for (int k = 0; k < M; ++k) ch.L[k][k] = rsqrt(ch.L[k][k]);
+      } else {
+        ch.factor();
+      }
       double u[M];   // L^-1 (y - x'[0:3])
 #pragma unroll
       for (int k = 0; k < M; ++k) {
         double s = meas[k] - x[k];
 #pragma unroll
         for (int m = 0; m < M; ++m)
-          if (m < k) s -= ch.L[k][m] * u[m];
+          if (m < k && !AXIS) s -= ch.L[k][m] * u[m];
         u[k] = s * ch.L[k][k];
       }
-      double Z[M][N];   // L^-1 P'[0:3,:] (forward substitution; the diagonal of ch holds 1 / L_kk)
+      double Z[M][N];   // L^-1 P'[0:3,:] (forward substitution; the diagonal of ch holds 1 / L_kk); blocked: row k = axis(j) only
 #pragma unroll
       for (int j = 0; j < N; ++j) {
 #pragma unroll
         for (int k = 0; k < M; ++k) {
+          if (!kept(k, j)) continue;
           double s = P(k, j);
 #pragma unroll
           for (int m = 0; m < M; ++m)
-            if (m < k) s -= ch.L[k][m] * Z[m][j];
+            if (m < k && !AXIS) s -= ch.L[k][m] * Z[m][j];
           Z[k][j] = s * ch.L[k][k];
         }
 #pragma unroll
-        for (int k = 0; k < M; ++k) x[j] += Z[k][j] * u[k];
+        for (int k = 0; k < M; ++k)
+          if (kept(k, j)) x[j] += Z[k][j] * u[k];
       }
 #pragma unroll
       for (int i = 0; i < N; ++i)
 #pragma unroll
         for (int j = 0; j < N; ++j)
-          if (i <= j) {
+          if (i <= j && kept(i, j)) {
             double s = P(i, j);
 #pragma unroll
-            for (int k = 0; k < M; ++k) s -= Z[k][i] * Z[k][j];
+            for (int k = 0; k < M; ++k)
+              if (kept(k, i)) s -= Z[k][i] * Z[k][j];
             P(i, j) = s;
           }
       nm += 1;      // updateMeasurement (src/target_interface.cpp:142-146)
@@ -134,14 +152,21 @@ struct KinSym {
     t = t + dt;     // updateTime (:148-152)
   }
 
-  // packed: only the upper triangle is written (the pool mirrors it on demand, te_pool.cu ensure_full)
-  __device__ __forceinline__ void store(double* out, bool packed) const {
+  // packed: only the upper triangle is written (the pool mirrors it on demand, te_pool.cu ensure_full).  The blocked form is
+  // always packed and writes the in-axis entries only -- into the lane's own slot, whose cross-axis entries are already +-0.  A
+  // compacting tick writes into another target's old slot: cross_zeros then clears the cross-axis entries of the upper triangle,
+  // which the slot's previous owner may have left non-zero (a NaN from a non-finite p0_scale).
+  __device__ __forceinline__ void store(double* out, bool packed, bool cross_zeros = false) const {
 #pragma unroll
     for (int i = 0; i < N; ++i) out[(LY::F_X + i) * TILE] = x[i];
 #pragma unroll
     for (int i = 0; i < N; ++i)
 #pragma unroll
       for (int j = 0; j < N; ++j) {
+        if (!kept(i, j)) {
+          if (i <= j && cross_zeros) out[(LY::F_P + i * N + j) * TILE] = 0.0;
+          continue;
+        }
         const double v = i <= j ? P.v[i * N - (i * (i - 1)) / 2 + (j - i)] : P.v[j * N - (j * (j - 1)) / 2 + (i - j)];
         if (i <= j || !packed) out[(LY::F_P + i * N + j) * TILE] = v;
       }

@@ -606,6 +606,14 @@ int te_pool_register_class(te_pool* p, const double* Q, const double* R, const d
       return true;
     };
     if (!sym(Q, p->N) || !sym(R, p->M) || !sym(P0, p->N)) p->all_sym = false;
+    auto decoupled = [](const double* A, int n, int axes) {   // entry (i, j) belongs to axes i % axes and j % axes
+      for (int i = 0; i < n; ++i)
+        for (int j = 0; j < n; ++j)
+          if (i % axes != j % axes && A[i * n + j] != 0.0) return false;
+      return true;
+    };
+    const bool kin = p->model == te::UNIFORM_VELOCITY || p->model == te::UNIFORM_ACCELERATION;
+    if (!kin || !decoupled(Q, p->N, 3) || !decoupled(P0, p->N, 3) || !decoupled(R, p->M, p->M)) p->all_axis = false;
     {
       // T = L^-1, R = L L^T (plain FP64 Cholesky, then forward substitution against the identity); zeros if R has no factor
       const int m = p->M;

@@ -133,6 +133,10 @@ struct te_pool {
   int variant = 0;
   int grid_cap = 0;      // test hook (te_pool_set_grid_cap): upper bound on the CTAs of a step launch, 0 = none
   bool all_sym = true;   // every registered class has bitwise-symmetric Q, R, P0 (symmetric-covariance kernels are legal)
+  // UV / UA: no registered class couples the x / y / z axes (Q, P0 zero between axes, R diagonal), so every cross-axis covariance
+  // entry in HBM stays +-0 and the packed direct kernels move the per-axis blocks only (te_kin_sym.cuh AXIS).  Always false for
+  // AV / AR.  Like all_sym, it only ever goes from true to false.
+  bool all_axis = true;
   // The direct symmetric kernels maintain the UPPER triangle of every covariance only ("packed": 36 of UA's 92 fields are
   // neither read nor written per step).  lower_stale = the lower triangles in HBM are out of date; whoever needs the full
   // matrix (a full-matrix kernel, a state read-back) mirrors it first / on the fly.

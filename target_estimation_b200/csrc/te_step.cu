@@ -47,14 +47,13 @@ void launch_split_t(te_pool* p, const te::StepArgs& a, int n_work_hint) { launch
 
 bool uses_direct(const te_pool* p);
 void ensure_full(te_pool* p);
-template <int TYPE, int WARPS, int CTAS> void launch_kin_direct(te_pool* p, const te::StepArgs& a, int n_work_hint);
+void launch_kin(te_pool* p, const te::StepArgs& a, int n_work_hint);
 void launch_step_multi(te_pool* p, const te::StepArgs& a_in, int n_work_hint) {
   te::StepArgs a = a_in;
   if (uses_direct(p) && p->model != te::ANGULAR_VELOCITIES) {   // UV / UA: the direct kernel keeps the target in registers for all ticks
     a.packed = (p->all_sym && p->variant != 12) ? 1 : 0;
     if (a.packed) p->lower_stale = true;
-    if (p->model == te::UNIFORM_VELOCITY) launch_kin_direct<te::UNIFORM_VELOCITY, 4, 3>(p, a, n_work_hint);
-    else launch_kin_direct<te::UNIFORM_ACCELERATION, 8, 1>(p, a, n_work_hint);
+    launch_kin(p, a, n_work_hint);
     return;
   }
   ensure_full(p);
@@ -108,10 +107,10 @@ void launch_av_stream(te_pool* p, const te::StepArgs& a, int n_work_hint) {
   else launch_av_stream_k<QC, false>(p, a, n_work_hint);
 }
 
-template <int TYPE, int WARPS, int CTAS>
+template <int TYPE, int WARPS, int CTAS, bool AXIS>
 void launch_kin_direct_k(te_pool* p, const te::StepArgs& a, int n_work_hint) {
   const bool multi = a.n_ticks > 1 || a.tick_gate != nullptr;   // replay / live launches: an instantiation of their own
-  auto kern = multi ? te::kf_step_kin_direct_kernel<TYPE, WARPS, CTAS, true> : te::kf_step_kin_direct_kernel<TYPE, WARPS, CTAS, false>;
+  auto kern = multi ? te::kf_step_kin_direct_kernel<TYPE, WARPS, CTAS, true, AXIS> : te::kf_step_kin_direct_kernel<TYPE, WARPS, CTAS, false, AXIS>;
   int grid = capped(p, std::min(p->n_sm * CTAS, std::max(1, cdiv(n_work_hint, WARPS))));
   // programmatic stream serialization: see the kernel's griddepcontrol.wait
   cudaLaunchConfig_t cfg{};
@@ -132,11 +131,40 @@ void launch_kin_direct_k(te_pool* p, const te::StepArgs& a, int n_work_hint) {
 }
 // small pools (fewer tiles than the SMs have scheduler partitions) spread over more, smaller CTAs: one warp per partition has
 // the FP64 pipe to itself, which is what bounds a tick of a few hundred tiles
-template <int TYPE, int WARPS, int CTAS>
+template <int TYPE, int WARPS, int CTAS, bool AXIS>
 void launch_kin_direct(te_pool* p, const te::StepArgs& a, int n_work_hint) {
-  if (n_work_hint <= 2 * p->n_sm) launch_kin_direct_k<TYPE, 2, 1>(p, a, n_work_hint);
-  else if (n_work_hint <= 4 * p->n_sm) launch_kin_direct_k<TYPE, 4, 1>(p, a, n_work_hint);
-  else launch_kin_direct_k<TYPE, WARPS, CTAS>(p, a, n_work_hint);
+  if (n_work_hint <= 2 * p->n_sm) launch_kin_direct_k<TYPE, 2, 1, AXIS>(p, a, n_work_hint);
+  else if (n_work_hint <= 4 * p->n_sm) launch_kin_direct_k<TYPE, 4, 1, AXIS>(p, a, n_work_hint);
+  else launch_kin_direct_k<TYPE, WARPS, CTAS, AXIS>(p, a, n_work_hint);
+}
+// The axis-blocked form at its large-pool shape.  TE_AXIS_SHAPE ("WARPSxCTAS", read per call) is the tuning knob with which
+// tools/bench_axis_blocks.py measures the other shapes against it.
+template <int TYPE, int WARPS, int CTAS>
+void launch_kin_axis(te_pool* p, const te::StepArgs& a, int n_work_hint) {
+  const char* shape = std::getenv("TE_AXIS_SHAPE");
+  if (shape && n_work_hint > 4 * p->n_sm) {
+    if (!std::strcmp(shape, "8x1")) return launch_kin_direct_k<TYPE, 8, 1, true>(p, a, n_work_hint);
+    if (!std::strcmp(shape, "8x2")) return launch_kin_direct_k<TYPE, 8, 2, true>(p, a, n_work_hint);
+    if (!std::strcmp(shape, "4x3")) return launch_kin_direct_k<TYPE, 4, 3, true>(p, a, n_work_hint);
+    if (!std::strcmp(shape, "4x4")) return launch_kin_direct_k<TYPE, 4, 4, true>(p, a, n_work_hint);
+  }
+  launch_kin_direct<TYPE, WARPS, CTAS, true>(p, a, n_work_hint);
+}
+// UV / UA on the direct kernels (variants 0 / 12 / 13): the axis-blocked form when the pool is packed and no class couples the axes
+void launch_kin(te_pool* p, const te::StepArgs& a, int n_work_hint) {
+  const bool axis = a.packed && p->all_axis;
+  if (p->model == te::UNIFORM_VELOCITY) {
+    // measured, packed, 4 Mi targets: <4,3> (12 warps per SM) 1.17e10, <4,4> 1.11e10, <8,1> 1.09e10 steps/s.  Axis-blocked (80 registers
+    // against 128; tools/bench_axis_blocks.py, B200 at 1000 W, ms per tick in two runs): <8,2> 0.2285 / 0.2321, <4,4> 0.2299 / 0.2318,
+    // <4,3> 0.2349 / 0.2339, <8,1> 0.2823 / 0.2786
+    if (axis) launch_kin_axis<te::UNIFORM_VELOCITY, 8, 2>(p, a, n_work_hint);
+    else launch_kin_direct<te::UNIFORM_VELOCITY, 4, 3, false>(p, a, n_work_hint);
+  } else {
+    // axis-blocked (126 registers against 234), 4 Mi targets, ms per tick in two runs: <4,3> 0.3720 / 0.3728, <8,2> 0.3778 / 0.3785,
+    // <4,4> 0.3797 / 0.3798, <8,1> 0.3822 / 0.3806
+    if (axis) launch_kin_axis<te::UNIFORM_ACCELERATION, 4, 3>(p, a, n_work_hint);
+    else launch_kin_direct<te::UNIFORM_ACCELERATION, 8, 1, false>(p, a, n_work_hint);
+  }
 }
 
 // does the current variant run a direct symmetric-covariance kernel (te_direct.cuh)?
@@ -164,13 +192,14 @@ void ensure_full(te_pool* p) {
 // Stage bytes of the staged kernel: UV 13056, UA 25344, AV 43008, AR 90624.
 // Kernel per model and variant.  Variants are what the tests switch between, not tuning shapes:
 //   0   default, while every class is bitwise symmetric (packed: upper triangle only): UV / UA direct symmetric-covariance kernels
-//       (te_direct.cuh); AV dense ticks (in place and compacting) the TMA-streamed kernel (te_av_stream.cuh), AV sparse ticks and pools
-//       with a class whose R has no Cholesky factor the direct kernel; AR the warp-specialised row-split kernel on the full matrix
-//       (te_split.cuh).  A pool with an asymmetric class runs the full-matrix kernels (10).
+//       (te_direct.cuh), in their axis-blocked form (per-axis covariance blocks only) while no class couples the axes; AV dense
+//       ticks (in place and compacting) the TMA-streamed kernel (te_av_stream.cuh), AV sparse ticks and pools with a class whose R
+//       has no Cholesky factor the direct kernel; AR the warp-specialised row-split kernel on the full matrix (te_split.cuh).  A
+//       pool with an asymmetric class runs the full-matrix kernels (10).
 //   1   the TMA-staged one-warp-per-tile kernel on the full matrix (te_kernels.cuh; also what replay launches of AV / AR run)
 //   10  forced full-matrix kernels (UV / UA staged, AV row-split): what a pool with an asymmetric class runs
 //   11  AR row-split kernel moving the upper triangle only (44 % fewer bytes, not faster: DESIGN.md section 7)
-//   12  UV / UA / AV direct kernels writing both halves of the covariance
+//   12  UV / UA / AV direct kernels writing both halves of the covariance (never the axis-blocked form)
 //   13  as 0, but AV dense ticks on the direct kernel too
 // Shape experiments of round 1 (warps x stages sweeps, the AR / AV two-lanes-per-target kernels, thread-per-target AR) were
 // measured, lost, and are gone from the tree: DESIGN.md section 7 keeps their numbers.
@@ -182,11 +211,8 @@ void launch_step(te_pool* p, const te::StepArgs& a_in, int n_work_hint) {
     if (a.packed) p->lower_stale = true;
     switch (p->model) {
       case te::UNIFORM_VELOCITY:
-        // measured, packed, 4 Mi targets: <4,3> (12 warps per SM) 1.17e10, <4,4> 1.11e10, <8,1> 1.09e10 steps/s
-        launch_kin_direct<te::UNIFORM_VELOCITY, 4, 3>(p, a, n_work_hint);
-        return;
       case te::UNIFORM_ACCELERATION:
-        launch_kin_direct<te::UNIFORM_ACCELERATION, 8, 1>(p, a, n_work_hint);
+        launch_kin(p, a, n_work_hint);
         return;
       default:
         if (av_stream_serves(p, a)) {
