@@ -218,6 +218,25 @@ class TargetManager {
   // Position only, for every model: for UV / UA the filter's full innovation, for AR / AV the exact position marginal of the 6-D one.
   virtual long long gatedTargets(long long q, const double* t1 /*[q] or NULL*/, const double* z /*[q][3]*/, const double* gate /*[q]*/,
                                  long long k, unsigned* ids_out /*[q][k]*/, double* d2_out /*[q][k]*/, long long* count_out /*[q]*/);
+  // Association of one frame of unlabelled position detections (contract of te_pool_associate in include/te_pool.h, INTEGRATION.md
+  // section 12): all q detections are stamped t1, detection j is the pose record det[j][0:7] and is gated on det[j][0:3].
+  //  1. Target i is a candidate for j when t_i <= t1 (NaN never) and d^2 <= gate, d^2 bit for bit gatedTargets' for (t1, det[j][0:3]);
+  //     count_out[j] (may be NULL) = the number of candidates; j's candidate list = its first min(K, count) by (d^2, id) -- when every
+  //     target has t <= t1, gatedTargets(k = K)'s rows.
+  //  2. Greedy on sorted edges: the edges of all candidate lists in ascending (d^2, id, j) order, each taken when neither end is
+  //     taken yet.  id_out[j] / d2_out[j] = the assigned target and its d^2, 0xFFFFFFFF / -1 without one.  A detection whose K
+  //     candidates all go to better edges stays unassigned.
+  //  3. apply = 1: every assigned target i gets update(i, t1 - t_i, det[j]) (dt rounded once, bit for bit te_pool_step_ids with that
+  //     dt); nothing else changes.  apply = 0: read-only.  Queued per-id calls are flushed first in both modes.  On a tick handle the
+  //     update is a by-hand update, as updateBatch's.
+  //  4. The result does not depend on the shard count, on which (shard, model type) pool holds a target, or on slot order.
+  //  5. std::invalid_argument, nothing applied: t1 not finite; gate negative, NaN or +inf; K outside [1, 32]; q < 0; det, id_out or
+  //     d2_out NULL while q > 0.
+  // One pool holding every target runs te_pool_associate; otherwise every pool's te_pool_gated_candidates (the shards at once) are
+  // merged by (d^2, id) as gatedTargets merges, te_assign_greedy runs on the first pool's device, and the assigned records go to
+  // their pools' te_pool_update_at.  Returns the number of assigned detections.
+  virtual long long associate(double t1, long long q, const double* det /*[q][7]*/, double gate, int K, int apply, unsigned* id_out /*[q]*/,
+                              double* d2_out /*[q]*/, long long* count_out /*[q] or NULL*/);
   // One dense tick from host arrays, record k = the k-th target in denseIds() order (a homogeneous manager: getAvailableTargets()
   // order): no ids travel, nothing is looked up -- te_pool_tick_host: the copies, the step and the read-back of every target's
   // estimated position (est_pos_out [n][3], may be NULL: what the node broadcasts per tick, src/target_manager_ros.cpp:78-87) are
@@ -267,8 +286,15 @@ class TargetManager {
   static void requireMeasurements(long long n, const double* meas, const unsigned char* action);
   long long updateBatchUnique(long long n, const unsigned* ids, double dt, const double* meas, const unsigned char* action);   // no id twice
   te_pool* densePool();   // the one non-empty pool of a homogeneous manager (throws otherwise)
+  // associate() over the pools of `shards` (each_shard as in PoolRowMerge::run); update(n, ids, det) applies the assigned records
+  long long associateOver(const std::vector<TargetManager*>& shards, const std::function<void(const std::function<void(int)>&)>& each_shard,
+                          double t1, long long q, const double* det, double gate, int K, int apply, unsigned* id_out, double* d2_out,
+                          long long* count_out, const std::function<void(long long, const unsigned*, const double*)>& update);
+  void updateAt(double t1, long long n, const unsigned* ids, const double* det);   // te_pool_update_at of every model type's rows
+  friend class ShardedTargetManager;
   PoolRowMerge nearest_rows_;
   PoolRowMerge gated_rows_;
+  PoolRowMerge assoc_rows_;
 
   int device_;
   te_pool* pools_[4] = {nullptr, nullptr, nullptr, nullptr};
@@ -555,6 +581,8 @@ class ShardedTargetManager : public TargetManager {
                            double* dist_out, long long* count_out) override;   // every shard at once
   long long gatedTargets(long long q, const double* t1, const double* z, const double* gate, long long k, unsigned* ids_out,
                          double* d2_out, long long* count_out) override;   // every shard at once
+  long long associate(double t1, long long q, const double* det, double gate, int K, int apply, unsigned* id_out, double* d2_out,
+                      long long* count_out) override;   // candidates of every shard at once, updates routed by owner
   // dense ticks: the records are SHARD-MAJOR (denseIds(): shard 0's targets in ascending id, then shard 1's, ...); every shard's
   // slice is copied, stepped and read back by its own worker thread on its own device
   long long updateDense(double dt, const double* meas, int meas_stride, const unsigned char* action, double* est_pos_out) override;

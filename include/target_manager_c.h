@@ -100,6 +100,13 @@ long long target_manager_nearest(const target_manager_c* self, long long q, cons
  * of a returned target is target_manager_get_estimates_batch(ids, t1).  Returns the total count, -1 on error. */
 long long target_manager_gated(const target_manager_c* self, long long q, const double* t1, const double* z, const double* gate, long long k,
                                unsigned int* ids_out, double* d2_out, long long* count_out);
+/* Association of one frame: TargetManager::associate (contract of te_pool_associate in te_pool.h, INTEGRATION.md section 12).  The q
+ * detections det[q][7] are stamped t1 and gated on their positions; each is assigned at most one target, greedily by (d^2, id, j)
+ * over every detection's K best candidates (1 <= K <= 32); apply = 1 updates every assigned target with its detection at t1.
+ * id_out / d2_out [q] = the assigned target and its d^2 (0xFFFFFFFF / -1: none), count_out [q] (may be NULL) = the candidates.
+ * Returns the number of assigned detections, -1 on error (nothing applied). */
+long long target_manager_associate(const target_manager_c* self, double t1, long long q, const double* det, double gate, int K, int apply,
+                                   unsigned int* id_out, double* d2_out, long long* count_out);
 
 /* ---- all GPUs of the box behind one handle (BASELINE.json north_star: targets shard by id, no collective on the hot path) ----
  * n_shards TargetManagers, shard r on CUDA device devices[r] (NULL = devices 0 .. n_shards-1), owner(id) = id mod n_shards.  The

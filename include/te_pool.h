@@ -288,6 +288,45 @@ long long te_pool_nearest_targets(te_pool* p, long long q, const double* t1 /*[q
 long long te_pool_gated_targets(te_pool* p, long long q, const double* t1 /*[q] or NULL*/, const double* z /*[q][3]*/, const double* gate,
                                 long long k, uint32_t* ids_out /*[q][k]*/, double* d2_out /*[q][k]*/, long long* count_out /*[q]*/);
 
+/* ---- association: one frame of unlabelled position detections (INTEGRATION.md section 12, DESIGN.md section 4.10) ---------- */
+/* All q detections are stamped t1; detection j is a pose record det[j][0:7] (the record te_pool_step_ids takes) and is gated on its
+ * position z_j = det[j][0:3] only.
+ *  1. Candidates: target i is a candidate for detection j when t_i <= t1 (a NaN time never is: the update needs dt >= 0) and
+ *     d2_ij <= gate, d2_ij being bit for bit te_pool_gated_targets' d^2 for the query (t1, z_j) (its steps 1-4).  count_out[j] = the
+ *     number of candidates (count_out may be NULL).  The candidate list of j = its first min(K, count) candidates by (d^2, id): when
+ *     every target has t <= t1, exactly te_pool_gated_targets(t1, z_j, gate, k = K)'s rows and count.
+ *  2. Assignment, greedy on sorted edges: the edges (j, i, d^2) of all candidate lists, visited in ascending (d^2, id, j) order; an
+ *     edge is taken when neither its detection nor its target is taken yet.  id_out[j] / d2_out[j] = the assigned target and its d^2,
+ *     0xFFFFFFFF / -1 for a detection without one.  K bounds the work: a detection whose K candidates all go to better edges stays
+ *     unassigned even when it has further candidates.
+ *  3. apply = 1: every assigned target i gets update(i, t1 - t_i, det[j]) -- dt rounded once, the result bit for bit that of
+ *     te_pool_step_ids with that per-row dt and measurement (t, n_meas and measured_pose change as there); other targets are not
+ *     touched.  apply = 0: read-only.
+ *  4. Argument errors (nothing applied): t1 not finite; gate negative, NaN or +inf (+inf has no spatial bound: te_pool_gated_targets
+ *     serves it); K outside [1, 32]; q < 0; det, id_out or d2_out NULL while q > 0.
+ * The candidates come from a grid index over every target's gate box (no q x size sweep), the matching runs on the device, and only
+ * the detections go up and q ids, d^2 and counts come back.  Synchronous.  Returns the number of assigned detections. */
+long long te_pool_associate(te_pool* p, double t1, long long q, const double* det /*[q][7]*/, double gate, int K, int apply,
+                            uint32_t* id_out /*[q]*/, double* d2_out /*[q]*/, long long* count_out /*[q] or NULL*/);
+/* Step 1 alone, read-only: the candidate lists of q positions z[q][3] over the pool, rows ids_out[j][.] / d2_out[j][.] by (d^2, id)
+ * and rows of id 0xFFFFFFFF / d^2 -1 after them (the rows several pools' lists are merged from, as gatedTargets merges).  Argument
+ * rules of te_pool_associate with z for det and ids_out for id_out.  Returns the total count. */
+long long te_pool_gated_candidates(te_pool* p, double t1, long long q, const double* z /*[q][3]*/, double gate, int K,
+                                   uint32_t* ids_out /*[q][K]*/, double* d2_out /*[q][K]*/, long long* count_out /*[q] or NULL*/);
+/* Step 2 alone over host rows, on p's device and stream (p's targets are not read): detection j's rows ids[j][.] / d2[j][.] hold its
+ * candidates by (d^2, id) with d^2 >= 0, then rows of d^2 -1 (any other layout is an error).  id_out / d2_out as te_pool_associate.
+ * 1 <= K <= 32.  Returns the number of assigned detections. */
+long long te_assign_greedy(te_pool* p, long long q, int K, const uint32_t* ids /*[q][K]*/, const double* d2 /*[q][K]*/, uint32_t* id_out /*[q]*/,
+                           double* d2_out /*[q]*/);
+/* Step 3 alone: op k = update(ids[k], t1 - t, meas[k]) with dt = t1 - t of the target computed on the device (rounded once), then
+ * the path of te_pool_step_ids (same scatter, duplicate check -- -2, nothing applied -- and step launch).  Unknown ids are skipped;
+ * a target with t > t1 (or a NaN t) is an error and nothing is applied.  t1 must be finite.  Returns #applied. */
+long long te_pool_update_at(te_pool* p, long long n, const uint32_t* ids, double t1, const double* meas /*[n][7]*/);
+/* What the pool's last te_pool_associate / te_pool_gated_candidates / te_assign_greedy call saw: out[0] = grid levels that held a
+ * target, out[1] = targets on the list every detection checks directly (a non-finite gate box), out[2] = candidates over all
+ * detections, out[3] = matching rounds (0 for te_pool_gated_candidates). */
+int te_pool_assoc_stats(te_pool* p, long long* out /*[4]*/);
+
 /* Dense device-resident form: one query per slot (query k = slot k = solver stream k; needs n_streams >= pool size).
  * dev_t1 NULL = each target's own time; dev_delta / dev_pose7 / dev_converged may be NULL.  Asynchronous. */
 int te_isolver_query_dense(te_isolver* s, const double* dev_t1, const double* dev_origin /*[size][3]*/, const double* dev_radius,

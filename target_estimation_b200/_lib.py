@@ -80,6 +80,11 @@ SIGNATURES = {
     "te_pool_earliest_intersections": (_ll, [_p, _ll, _p, _p, _p, _ll, _p, _p, _p]),
     "te_pool_nearest_targets": (_ll, [_p, _ll, _p, _p, _p, _ll, _p, _p, _p]),
     "te_pool_gated_targets": (_ll, [_p, _ll, _p, _p, _p, _ll, _p, _p, _p]),
+    "te_pool_associate": (_ll, [_p, _d, _ll, _p, _d, _i, _i, _p, _p, _p]),
+    "te_pool_gated_candidates": (_ll, [_p, _d, _ll, _p, _d, _i, _p, _p, _p]),
+    "te_assign_greedy": (_ll, [_p, _ll, _i, _p, _p, _p, _p]),
+    "te_pool_update_at": (_ll, [_p, _ll, _p, _d, _p]),
+    "te_pool_assoc_stats": (_i, [_p, _p]),
     "te_isolver_move_streams": (_i, [_p, _p, _ll, _p]),
     "te_pool_tick_host_async": (_i, [_p, _d, _p, _i, _p, _i, _p]),
     "te_pool_tick_host_wait": (_i, [_p, _i]),

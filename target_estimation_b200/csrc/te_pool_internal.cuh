@@ -6,6 +6,8 @@
 //   te_isolver.cu  batched IntersectionSolver
 //   te_sweep.cu    the k earliest sphere intercepts, the k nearest targets and the k gated targets over every target of a pool
 //                  (te_pool_earliest_intersections, te_pool_nearest_targets, te_pool_gated_targets)
+//   te_assoc.cu    association of unlabelled detections: grid-indexed gate candidates, device greedy matching, update at t1
+//                  (te_pool_associate, te_pool_gated_candidates, te_assign_greedy, te_pool_update_at)
 //   te_group.cu    several pools on several devices: the NCCL all-gather of estimate records
 #pragma once
 #include <algorithm>
@@ -142,6 +144,7 @@ struct te_pool {
   // matrix (a full-matrix kernel, a state read-back) mirrors it first / on the fly.
   bool lower_stale = false;
   long long n = 0;   // live targets
+  long long assoc_stats[4] = {0, 0, 0, 0};   // te_pool_assoc_stats: of the last association call
   tehost::Buf buf[2];
   int cur = 0;
   // per-slot work arrays (capacity wcap slots)
@@ -270,6 +273,9 @@ void launch_gather_estimates(te_pool* p, const int* slots, long long n, const do
 void fold_pending(te_pool* p);
 void demote_mailboxes(te_pool* p, const uint32_t* ids, const int* d_slots, long long n);
 void attach_mailboxes(te_pool* p, const uint32_t* ids, long long n);
+// ---- te_sweep.cu ----
+// gate_prep_kernel of the pool's model over every slot: the factor of S into chol[6 * slot]; t1 NULL = no predict
+void launch_gate_prep(te_pool* p, int n, const double* t1, double* chol);
 // ---- te_mailbox.cu ----
 void prefetch_start(te_pool* p);   // put the registered message's copies into the copy stream's queue (no-op if none / started)
 // ---- te_step.cu ----
@@ -279,6 +285,10 @@ void launch_step(te_pool* p, const te::StepArgs& a_in, int n_work_hint);
 void launch_step_multi(te_pool* p, const te::StepArgs& a_in, int n_work_hint);
 te::StepArgs base_args(te_pool* p);
 void check_meas_stride(te_pool* p, int stride);
+// te_pool_step_ids over device arrays (d_dt NULL = dt_scalar, d_meas NULL only without UPDATE ops, d_act NULL = UPDATE): the scatter,
+// the duplicate check (-2, nothing applied) and the step launch.  Returns #applied.
+long long step_ops(te_pool* p, long long n, const uint32_t* d_ids, const double* d_dt, double dt_scalar, const double* d_meas,
+                   const uint8_t* d_act);
 
 template <class T> T* to_dev(te_pool* p, const T* host, size_t n) {
   if (!host || !n) return nullptr;

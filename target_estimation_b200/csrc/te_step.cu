@@ -642,14 +642,58 @@ int te_pool_tick_host_wait(te_pool* p, int lag) {
   });
 }
 
+}  // extern "C"
+
+namespace tehost {
+long long step_ops(te_pool* p, long long n, const uint32_t* d_ids, const double* d_dt, double dt_scalar, const double* d_meas,
+                   const uint8_t* d_act) {
+  ensure_work(p, (size_t)p->n);
+  Buf& b = p->buf[p->cur];
+  CK(cudaMemsetAsync(p->d_counters, 0, 3 * sizeof(int), p->stream));
+  CK(cudaMemsetAsync(p->alive, 0, (size_t)p->n * sizeof(int), p->stream));   // per-slot claim counts of this call (alive[] is scratch between compactions)
+  te::scatter_ops_kernel<<<cdiv(n, 256), 256, 0, p->stream>>>(b.cold.ids, (int)p->n, n, d_ids, d_dt, dt_scalar, d_meas, d_act, p->action,
+                                                               p->dt_slot, b.cold.meas, p->tile_flag, p->tile_list, p->d_counters, p->alive);
+  CK(cudaGetLastError());
+  if (n > 1) {   // a repeated id?  (checked before anything is stepped)
+    int dups = 0;
+    CK(cudaMemcpyAsync(&dups, p->d_counters + 2, sizeof(int), cudaMemcpyDeviceToHost, p->stream));
+    CK(cudaStreamSynchronize(p->stream));
+    if (dups > 0) {
+      CK(cudaMemsetAsync(p->action, 0, (size_t)p->n, p->stream));
+      CK(cudaMemsetAsync(p->tile_flag, 0, (size_t)cdiv(p->n, te::TILE) + 4, p->stream));
+      CK(cudaStreamSynchronize(p->stream));
+      last_error() = "an id appears more than once in the batch: nothing applied";
+      return -2;
+    }
+  }
+  te::StepArgs a = base_args(p);
+  a.tile_list = p->tile_list;
+  a.d_nwork = p->d_counters;
+  a.dt = dt_scalar;
+  a.dt_slot = p->dt_slot;
+  a.meas = b.cold.meas;
+  a.meas_stride = 7;
+  a.meas_tma = 1;
+  a.action = p->action;
+  a.default_action = TE_ACT_NONE;
+  a.clear_action = 1;
+  a.tile_flag = p->tile_flag;
+  launch_step(p, a, (int)std::min<long long>(n, a.n_tiles));
+  int applied = 0;
+  CK(cudaMemcpyAsync(&applied, p->d_counters + 1, sizeof(int), cudaMemcpyDeviceToHost, p->stream));
+  CK(cudaStreamSynchronize(p->stream));
+  return applied;
+}
+}  // namespace tehost
+
+extern "C" {
+
 long long te_pool_step_ids(te_pool* p, long long n, const uint32_t* ids, const double* dt, double dt_scalar, const double* meas,
                            const uint8_t* action) {
   return guarded_ll(p, [&]() -> long long {
     if (n <= 0 || p->n == 0) return 0;
     if (!ids) throw std::invalid_argument("null ids");
     if (!dt && !(dt_scalar >= 0.0)) throw std::invalid_argument("dt must be >= 0");
-    ensure_work(p, (size_t)p->n);
-    Buf& b = p->buf[p->cur];
     uint32_t* d_ids = to_dev(p, ids, n);
     double* d_dt = to_dev(p, dt, n);
     double* d_meas = to_dev(p, meas, n * 7);
@@ -659,40 +703,7 @@ long long te_pool_step_ids(te_pool* p, long long n, const uint32_t* ids, const d
       if (action) for (long long k = 0; k < n && !needs; ++k) needs = action[k] == TE_ACT_UPDATE;
       if (needs) throw std::invalid_argument("update ops without measurements");
     }
-    CK(cudaMemsetAsync(p->d_counters, 0, 3 * sizeof(int), p->stream));
-    CK(cudaMemsetAsync(p->alive, 0, (size_t)p->n * sizeof(int), p->stream));   // per-slot claim counts of this call (alive[] is scratch between compactions)
-    te::scatter_ops_kernel<<<cdiv(n, 256), 256, 0, p->stream>>>(b.cold.ids, (int)p->n, n, d_ids, d_dt, dt_scalar, d_meas, d_act, p->action,
-                                                                 p->dt_slot, b.cold.meas, p->tile_flag, p->tile_list, p->d_counters, p->alive);
-    CK(cudaGetLastError());
-    if (n > 1) {   // a repeated id?  (checked before anything is stepped)
-      int dups = 0;
-      CK(cudaMemcpyAsync(&dups, p->d_counters + 2, sizeof(int), cudaMemcpyDeviceToHost, p->stream));
-      CK(cudaStreamSynchronize(p->stream));
-      if (dups > 0) {
-        CK(cudaMemsetAsync(p->action, 0, (size_t)p->n, p->stream));
-        CK(cudaMemsetAsync(p->tile_flag, 0, (size_t)cdiv(p->n, te::TILE) + 4, p->stream));
-        CK(cudaStreamSynchronize(p->stream));
-        last_error() = "an id appears more than once in the batch: nothing applied";
-        return -2;
-      }
-    }
-    te::StepArgs a = base_args(p);
-    a.tile_list = p->tile_list;
-    a.d_nwork = p->d_counters;
-    a.dt = dt_scalar;
-    a.dt_slot = p->dt_slot;
-    a.meas = b.cold.meas;
-    a.meas_stride = 7;
-    a.meas_tma = 1;
-    a.action = p->action;
-    a.default_action = TE_ACT_NONE;
-    a.clear_action = 1;
-    a.tile_flag = p->tile_flag;
-    launch_step(p, a, (int)std::min<long long>(n, a.n_tiles));
-    int applied = 0;
-    CK(cudaMemcpyAsync(&applied, p->d_counters + 1, sizeof(int), cudaMemcpyDeviceToHost, p->stream));
-    CK(cudaStreamSynchronize(p->stream));
-    return applied;
+    return step_ops(p, n, d_ids, d_dt, dt_scalar, d_meas, d_act);
   });
 }
 

@@ -112,6 +112,9 @@ unsigned long long bits_of(double v) {
   return b;
 }
 
+}  // namespace
+
+namespace tehost {
 // gate_prep_kernel of the pool's model over every slot: t1 NULL = no predict
 template <int TYPE>
 void launch_gate_prep_t(te_pool* p, int n, const double* t1, double* chol) {
@@ -126,7 +129,7 @@ void launch_gate_prep(te_pool* p, int n, const double* t1, double* chol) {
     default: launch_gate_prep_t<te::ANGULAR_RATES>(p, n, t1, chol); break;
   }
 }
-}  // namespace
+}  // namespace tehost
 
 extern "C" long long te_pool_earliest_intersections(te_pool* p, long long q, const double* t1, const double* origin, const double* radius,
                                                     long long k, uint32_t* ids_out, double* delta_out, long long* hits_out) {

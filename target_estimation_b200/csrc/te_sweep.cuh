@@ -182,23 +182,30 @@ __global__ void __launch_bounds__(256) gate_prep_kernel(int n, const double* __r
   o[5] = l22;
 }
 
-// position (pose7 as in near_key_kernel) and factor -> key: the bits of d^2 = (w0^2 + w1^2) + w2^2, w = L^-1 (p - z) by forward
-// substitution, for a target inside the gate (d^2 <= gate; NaN -- no factor -- never is), SWEEP_MISS otherwise; inside targets
-// counted.  d^2 >= +0 always, so its bits order like its value.
+// d^2 = (w0^2 + w1^2) + w2^2 of slot s for the measured position z, w = L^-1 (p - z) by forward substitution over the slot's position
+// (pose7 as in near_key_kernel) and factor (gate_prep_kernel): steps 4 and 5 of the gating contract in include/te_pool.h, in one
+// place for gate_key_kernel and the association's candidate search (te_assoc.cuh).  NaN when the slot has no factor.
+__device__ __forceinline__ double gate_d2(const double* __restrict__ pose7, const double* __restrict__ chol, size_t s, double zx, double zy,
+                                          double zz) {
+  const double* L = chol + 6 * s;
+  const double d0 = __dsub_rn(pose7[7 * s], zx);
+  const double d1 = __dsub_rn(pose7[7 * s + 1], zy);
+  const double d2 = __dsub_rn(pose7[7 * s + 2], zz);
+  const double w0 = __ddiv_rn(d0, L[0]);
+  const double w1 = __ddiv_rn(__dsub_rn(d1, __dmul_rn(L[1], w0)), L[3]);
+  const double w2 = __ddiv_rn(__dsub_rn(__dsub_rn(d2, __dmul_rn(L[2], w0)), __dmul_rn(L[4], w1)), L[5]);
+  return __dadd_rn(__dadd_rn(__dmul_rn(w0, w0), __dmul_rn(w1, w1)), __dmul_rn(w2, w2));
+}
+
+// position and factor -> key: the bits of d^2 (gate_d2) for a target inside the gate (d^2 <= gate; NaN -- no factor -- never is),
+// SWEEP_MISS otherwise; inside targets counted.  d^2 >= +0 always, so its bits order like its value.
 static __global__ void gate_key_kernel(int n, const double* __restrict__ pose7, const double* __restrict__ chol, double zx, double zy,
                                        double zz, double gate, unsigned long long* __restrict__ keys,
                                        unsigned long long* __restrict__ inside) {
   const int s = blockIdx.x * blockDim.x + threadIdx.x;
   bool in = false;
   if (s < n) {
-    const double* L = chol + 6 * (size_t)s;
-    const double d0 = __dsub_rn(pose7[7 * (size_t)s], zx);
-    const double d1 = __dsub_rn(pose7[7 * (size_t)s + 1], zy);
-    const double d2 = __dsub_rn(pose7[7 * (size_t)s + 2], zz);
-    const double w0 = __ddiv_rn(d0, L[0]);
-    const double w1 = __ddiv_rn(__dsub_rn(d1, __dmul_rn(L[1], w0)), L[3]);
-    const double w2 = __ddiv_rn(__dsub_rn(__dsub_rn(d2, __dmul_rn(L[2], w0)), __dmul_rn(L[4], w1)), L[5]);
-    const double m2 = __dadd_rn(__dadd_rn(__dmul_rn(w0, w0), __dmul_rn(w1, w1)), __dmul_rn(w2, w2));
+    const double m2 = gate_d2(pose7, chol, (size_t)s, zx, zy, zz);
     in = m2 <= gate;
     keys[s] = in ? (unsigned long long)__double_as_longlong(m2) : SWEEP_MISS;
   }

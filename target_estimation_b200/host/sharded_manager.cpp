@@ -346,6 +346,28 @@ long long ShardedTargetManager::gatedTargets(long long q, const double* t1, cons
       ids_out, d2_out, count_out);
 }
 
+long long ShardedTargetManager::associate(double t1, long long q, const double* det, double gate, int K, int apply, unsigned* id_out,
+                                          double* d2_out, long long* count_out) {
+  te::check_assoc_args(te::ASSOC_ARGS, t1, q, det, gate, K, id_out, d2_out);
+  std::lock_guard<std::recursive_mutex> lg(target_lock_);
+  if (q == 0) return 0;
+  flush();
+  std::vector<TargetManager*> shards;
+  for (auto& s : shard_) shards.push_back(s.get());
+  return associateOver(
+      shards, [this](const std::function<void(int)>& f) { forEachShard(f); }, t1, q, det, gate, K, apply, id_out, d2_out, count_out,
+      [&](long long n, const unsigned* ids, const double* rec) {
+        const std::vector<std::vector<long long>> rows = rowsByOwner(n, ids);
+        forEachShard([&](int r) {
+          const std::vector<long long>& mine = rows[(size_t)r];
+          if (mine.empty()) return;
+          std::vector<unsigned> s_ids;
+          std::vector<double> s_rec;
+          shard_[(size_t)r]->updateAt(t1, (long long)mine.size(), gatherRows<1>(ids, mine, s_ids), gatherRows<7>(rec, mine, s_rec));
+        });
+      });
+}
+
 // ---- dense ticks: shard-major records, every shard's slice on its own device at once ---------------------------------------------
 std::vector<unsigned int> ShardedTargetManager::denseIds() {
   std::vector<unsigned int> all;

@@ -1241,6 +1241,84 @@ long long TargetManager::gatedTargets(long long q, const double* t1, const doubl
       ids_out, d2_out, count_out);
 }
 
+long long TargetManager::associate(double t1, long long q, const double* det, double gate, int K, int apply, unsigned* id_out, double* d2_out,
+                                   long long* count_out) {
+  te::check_assoc_args(te::ASSOC_ARGS, t1, q, det, gate, K, id_out, d2_out);
+  std::lock_guard<std::recursive_mutex> lg(target_lock_);
+  if (q == 0) return 0;
+  flushLocked();
+  return associateOver(
+      {this}, [](const std::function<void(int)>& f) { f(0); }, t1, q, det, gate, K, apply, id_out, d2_out, count_out,
+      [&](long long n, const unsigned* ids, const double* rec) { updateAt(t1, n, ids, rec); });
+}
+
+long long TargetManager::associateOver(const std::vector<TargetManager*>& shards, const std::function<void(const std::function<void(int)>&)>& each_shard,
+                                       double t1, long long q, const double* det, double gate, int K, int apply, unsigned* id_out, double* d2_out,
+                                       long long* count_out, const std::function<void(long long, const unsigned*, const double*)>& update) {
+  int n_pools = 0, first = -1;   // first = shard * 4 + type of the first pool that holds targets
+  for (int r = 0; r < (int)shards.size(); ++r) {
+    const unsigned held = shards[(size_t)r]->heldTypes();
+    for (int t = 0; t < 4; ++t)
+      if ((held >> t) & 1u) {
+        ++n_pools;
+        if (first < 0) first = r * 4 + t;
+      }
+  }
+  auto on_first = [&](const std::function<long long(te_pool*)>& f) {
+    TargetManager& M = *shards[(size_t)(first / 4)];
+    std::lock_guard<std::recursive_mutex> lk(M.lock());
+    const long long rc = f(M.poolOf(first % 4, false));
+    ck(rc);
+    return rc;
+  };
+  if (n_pools == 0) {
+    std::fill(id_out, id_out + q, 0xFFFFFFFFu);
+    std::fill(d2_out, d2_out + q, -1.0);
+    if (count_out) std::fill(count_out, count_out + q, 0LL);
+    return 0;
+  }
+  if (n_pools == 1)   // one pool holds every target: the whole frame on its device
+    return on_first([&](te_pool* p) { return te_pool_associate(p, t1, q, det, gate, K, apply, id_out, d2_out, count_out); });
+  // every pool's candidate lists, merged by (d^2, id) as gatedTargets merges them; the matching on the first pool's device
+  std::vector<double> z((size_t)q * 3);
+  for (long long j = 0; j < q; ++j) std::memcpy(&z[(size_t)j * 3], det + 7 * (size_t)j, 24);
+  std::vector<unsigned> rows_id((size_t)(q * K));
+  std::vector<double> rows_d2((size_t)(q * K));
+  std::vector<long long> count((size_t)q);
+  assoc_rows_.run(
+      shards, each_shard, q, K,
+      [&](te_pool* p, unsigned* ids, double* d2, long long* cnt) { return te_pool_gated_candidates(p, t1, q, z.data(), gate, K, ids, d2, cnt); },
+      rows_id.data(), rows_d2.data(), count.data());
+  const long long assigned =
+      on_first([&](te_pool* p) { return te_assign_greedy(p, q, K, rows_id.data(), rows_d2.data(), id_out, d2_out); });
+  if (count_out) std::copy(count.begin(), count.end(), count_out);
+  if (apply && assigned > 0) {
+    std::vector<unsigned> ids;
+    std::vector<double> rec;
+    ids.reserve((size_t)assigned);
+    rec.reserve((size_t)assigned * 7);
+    for (long long j = 0; j < q; ++j)
+      if (d2_out[j] >= 0.0) {
+        ids.push_back(id_out[j]);
+        rec.insert(rec.end(), det + 7 * (size_t)j, det + 7 * (size_t)j + 7);
+      }
+    update((long long)ids.size(), ids.data(), rec.data());
+  }
+  return assigned;
+}
+
+void TargetManager::updateAt(double t1, long long n, const unsigned* ids, const double* det) {
+  std::lock_guard<std::recursive_mutex> lg(target_lock_);
+  std::vector<long long> rows[4];
+  rowsByType(n, ids, rows);
+  for (int t = 0; t < 4; ++t) {
+    if (rows[t].empty()) continue;
+    std::vector<unsigned> t_ids;
+    std::vector<double> t_det;
+    ck(te_pool_update_at(poolOf(t, false), (long long)rows[t].size(), gatherRows<1>(ids, rows[t], t_ids), t1, gatherRows<7>(det, rows[t], t_det)));
+  }
+}
+
 // ----------------------------------------------------------------------------------------------
 // utils.hpp:273-313
 // ----------------------------------------------------------------------------------------------

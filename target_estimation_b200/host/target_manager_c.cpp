@@ -197,6 +197,13 @@ long long target_manager_gated(const target_manager_c* self, long long q, const 
     return M(self)->gatedTargets(q, t1, z, gate, k, ids_out, d2_out, count_out);
   });
 }
+long long target_manager_associate(const target_manager_c* self, double t1, long long q, const double* det, double gate, int K, int apply,
+                                   unsigned int* id_out, double* d2_out, long long* count_out) {
+  return guard(-1LL, [&] {
+    if (!self) throw std::invalid_argument("null manager");
+    return M(self)->associate(t1, q, det, gate, K, apply, id_out, d2_out, count_out);
+  });
+}
 const char* target_manager_last_error(void) { return g_err.c_str(); }
 
 // ---- IntersectionSolver -------------------------------------------------------------------------------------------

@@ -38,6 +38,7 @@ _SIG = {
     "target_manager_flush": (None, [_p]),
     "target_manager_nearest": (_ll, [_p, _ll, _p, _p, _p, _ll, _p, _p, _p]),
     "target_manager_gated": (_ll, [_p, _ll, _p, _p, _p, _ll, _p, _p, _p]),
+    "target_manager_associate": (_ll, [_p, _d, _ll, _p, _d, _i, _i, _p, _p, _p]),
     "target_manager_last_error": (C.c_char_p, []),
     "target_manager_watch": (None, [_p, _ll, _p, _ll]),
     "target_manager_log_samples": (_ll, [_p]),
@@ -246,6 +247,21 @@ class TargetManagerC:
         if int(clib.target_manager_gated(self.h, q, _ptr(t1), _ptr(z), _ptr(gate), k, _ptr(ids), _ptr(d2), _ptr(count))) < 0:
             raise RuntimeError(clib.target_manager_last_error().decode())
         return count, ids, d2
+
+    def associate(self, t1, det, gate, K, apply=False):
+        """one frame of unlabelled detections det [q][7] (pose records stamped t1, gated on det[:, 0:3]): each detection is assigned at
+        most one target, greedily by (d2, id, j) over its K best candidates; apply=True updates every assigned target with its
+        detection at t1.  Returns (id [q], d2 [q], count [q]): id 0xFFFFFFFF / d2 -1 for an unassigned detection, count = its
+        candidates."""
+        det = np.ascontiguousarray(det, dtype=np.float64).reshape(-1, 7)
+        q = det.shape[0]
+        ids = np.zeros(q, dtype=np.uint32)
+        d2 = np.zeros(q)
+        count = np.zeros(q, dtype=np.int64)
+        if int(clib.target_manager_associate(self.h, float(t1), q, _ptr(det), float(gate), int(K), 1 if apply else 0, _ptr(ids), _ptr(d2),
+                                             _ptr(count))) < 0:
+            raise RuntimeError(clib.target_manager_last_error().decode())
+        return ids, d2, count
 
 
 class ShardedManagerC(TargetManagerC):

@@ -341,6 +341,52 @@ class TargetPool:
         check(lib.te_pool_gated_targets(self._h, q, _ptr(t1), _ptr(z), _ptr(gate), k, _ptr(ids), _ptr(d2), _ptr(count)))
         return count, ids, d2
 
+    # -- association of one frame of unlabelled detections (te_pool_associate and its three steps) --
+    def associate(self, t1, det, gate, K, apply=False):
+        """det [q][7] pose records stamped t1, gated on det[:, 0:3]; greedy assignment over each detection's K best candidates,
+        apply=True updates the assigned targets at t1.  Returns (id [q], d2 [q], count [q]) (id 0xFFFFFFFF / d2 -1: unassigned)."""
+        det = _np(det, np.float64).reshape(-1, 7)
+        q = det.shape[0]
+        ids = np.zeros(q, dtype=np.uint32)
+        d2 = np.zeros(q)
+        count = np.zeros(q, dtype=np.int64)
+        check(lib.te_pool_associate(self._h, float(t1), q, _ptr(det), float(gate), int(K), 1 if apply else 0, _ptr(ids), _ptr(d2), _ptr(count)))
+        return ids, d2, count
+
+    def gated_candidates(self, t1, z, gate, K):
+        """the candidate lists of positions z [q][3] at t1: (count [q], ids [q][K], d2 [q][K]) as gated_targets' with k = K, over
+        the targets with t <= t1"""
+        z = _np(z, np.float64).reshape(-1, 3)
+        q, K = z.shape[0], int(K)
+        count = np.zeros(q, dtype=np.int64)
+        ids = np.zeros((q, max(K, 0)), dtype=np.uint32)
+        d2 = np.zeros((q, max(K, 0)))
+        check(lib.te_pool_gated_candidates(self._h, float(t1), q, _ptr(z), float(gate), K, _ptr(ids), _ptr(d2), _ptr(count)))
+        return count, ids, d2
+
+    def assign_greedy(self, ids, d2):
+        """greedy assignment over candidate rows ids / d2 [q][K] (each row by (d2, id), then d2 -1), on this pool's device.  Returns
+        (id [q], d2 [q])."""
+        ids = _np(ids, np.uint32)
+        d2 = _np(d2, np.float64)
+        q, K = ids.shape
+        id_out = np.zeros(q, dtype=np.uint32)
+        d2_out = np.zeros(q)
+        check(lib.te_assign_greedy(self._h, q, K, _ptr(ids), _ptr(d2), _ptr(id_out), _ptr(d2_out)))
+        return id_out, d2_out
+
+    def update_at(self, ids, t1, meas):
+        """update(id, t1 - t, meas[k]) for every id (dt from each target's own t, on the device).  Returns #applied."""
+        ids = _np(ids, np.uint32)
+        meas = _np(meas, np.float64, (ids.size, 7))
+        return check(lib.te_pool_update_at(self._h, ids.size, _ptr(ids), float(t1), _ptr(meas)))
+
+    def assoc_stats(self):
+        """of the last association call: {levels, everywhere, candidates, rounds}"""
+        out = np.zeros(4, dtype=np.int64)
+        check(lib.te_pool_assoc_stats(self._h, _ptr(out)))
+        return dict(zip(("levels", "everywhere", "candidates", "rounds"), (int(v) for v in out)))
+
 
 class IntersectionSolver:
     """Batched IntersectionSolver: n_streams independent reference solver objects (include/te_pool.h)."""
